@@ -61,7 +61,39 @@ def parse():
     p.add_argument('--no-cpu-baseline', action='store_true')
     p.add_argument('--single-stream', action='store_true', help='run the mini-batches back to back on one stream (A/B of the two-stream overlap)')
     p.add_argument('--no-graph', action='store_true', help='launch kernels eagerly instead of replaying the captured step graph')
-    return p.parse_args()
+    p.add_argument('--dump-outputs', metavar='DIR', default=None,
+                   help='after the timed steps, write what the last timed step computed as DIR/<name>.npy (rank 0; float32 / '
+                        'float64, at most 64 MB in all: larger outputs are cut to a fixed seeded sample of rows), so that two '
+                        'builds can be compared output for output on identical inputs')
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error('--steps must be at least 1')
+    if args.dump_outputs is not None and args.impl == 'reference':
+        p.error('--dump-outputs records the CUDA path; the reference arm runs a scaled-down sample of the workload')
+    return args
+
+
+DUMP_LIMIT = 64 * 10 ** 6          # bytes of all .npy files together
+NPY_HEADER = 128
+
+
+def dump_outputs(out_dir, arrays):
+    """Write ``arrays`` (name -> tensor / array) as ``out_dir/<name>.npy``: float64 stays float64, integers become float64
+    (exact), everything else float32.  When the files would exceed DUMP_LIMIT bytes in all, each array keeps the same
+    fraction of its leading axis, chosen by a fixed seed, so that arrays with the same leading axis keep the same rows."""
+    arrays = {k: (v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)) for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float64 if v.dtype == np.float64 or v.dtype.kind in 'iub' else np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    budget = DUMP_LIMIT - NPY_HEADER * len(arrays)
+    if total > budget:
+        frac = budget / total
+        for k, v in arrays.items():
+            if v.ndim and v.shape[0] > 1:
+                keep = max(1, int(v.shape[0] * frac))
+                arrays[k] = v[np.sort(np.random.RandomState(0).choice(v.shape[0], keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), v)
 
 
 def peaks():
@@ -196,7 +228,7 @@ def bench_forward64(args, model, sa, dev, world, rank, local, dist):
     with torch.no_grad():
         pl = model.make_plan(Batch.from_data_list(dl), graphs=dl)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
-    out = {}
+    out, last = {}, {}
     sampler = ClockSampler(local)
     sampler.start()
     for tag, t in (('t1.0', 1.0), ('t0.05', 0.05)):
@@ -206,14 +238,16 @@ def bench_forward64(args, model, sa, dev, world, rank, local, dist):
                 model.run_plan(pl, ct)
             torch.cuda.synchronize()
             ms = []
-            for _ in range(max(args.steps, 3)):
+            for _ in range(args.steps):
                 flush.fill_(0)
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 e0.record()
-                model.run_plan(pl, ct)
+                scores = model.run_plan(pl, ct)
                 e1.record()
                 torch.cuda.synchronize()
                 ms.append(e0.elapsed_time(e1))
+            if args.dump_outputs is not None:
+                last.update({f'{tag}_{k}': v.cpu() for k, v in zip(('tr', 'rot', 'tor', 'sc_tor'), scores)})
             model.profile = []
             model.run_plan(pl, ct)
             torch.cuda.synchronize()
@@ -228,13 +262,15 @@ def bench_forward64(args, model, sa, dev, world, rank, local, dist):
         peak_tf, hbm, peak_src = peaks()
         print(json.dumps({
             'metric': 'score-model graph-forwards/sec (batch 64 forward microbench)', 'value': out['t1.0']['graph_forwards_per_s'], 'unit': 'graph-forwards/s',
-            'n_gpus': world, 'steps': max(args.steps, 3), 'warmup': max(args.warmup, 3), 'ms_per_step': out['t1.0']['ms_per_forward'], 'higher_is_better': True,
+            'n_gpus': world, 'steps': args.steps, 'warmup': max(args.warmup, 3), 'ms_per_step': out['t1.0']['ms_per_forward'], 'higher_is_better': True,
             'scaling': 'weak', 'vs_baseline': None, 'dtype': args.mode, 'data': 'synthetic',
             'config': {'workload': 'forward64: 64 x 3dpf pocket graph (BASELINE.json configs[2]), README big model, resident batch, t = 1.0 (value) and t = 0.05',
                        'conv_mode': args.mode, 'l2': '256 MiB flush before every timed forward'},
             'clocks': sampler.summary(), 'detail': out,
             'roofline': {'bound': 'tensor', 'achieved': out['t1.0']['conv_tflops'], 'peak': peak_tf, 'unit': 'TFLOP/s', 'frac': out['t1.0']['conv_tflops'] / peak_tf,
                          'traffic': None, 'peak_source': peak_src}}))
+        if args.dump_outputs is not None:
+            dump_outputs(args.dump_outputs, last)
     if world > 1:
         dist.destroy_process_group()
 
@@ -275,21 +311,22 @@ def bench_set(args, model, conf, sa, ca, dev, world, rank, local, dist):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0 = time.time()
     e0.record()
-    res, best, ok = one_pass(rows)
+    for _ in range(args.steps):
+        res, best, ok = one_pass(rows)
     e1.record()
     torch.cuda.synchronize()
-    wall = time.time() - t0
+    wall = (time.time() - t0) / args.steps
     if world > 1:
         dist.barrier()
     sampler.stop_flag = True
-    ms = _reduce_max(e0.elapsed_time(e1), dev, world, dist)
+    ms = _reduce_max(e0.elapsed_time(e1) / args.steps, dev, world, dist)
     wall = _reduce_max(wall, dev, world, dist)
     poses = n * spc
     if rank == 0:
         order = torch.argsort(best, descending=True)
         print(json.dumps({
             'metric': 'docked poses/sec (20-step reverse diffusion)', 'value': poses / (ms / 1000.0), 'unit': 'poses/s', 'n_gpus': world,
-            'steps': 1, 'warmup': max(1, min(args.warmup, 2)), 'ms_per_step': ms, 'higher_is_better': True, 'scaling': 'strong',
+            'steps': args.steps, 'warmup': max(1, min(args.warmup, 2)), 'ms_per_step': ms, 'higher_is_better': True, 'scaling': 'strong',
             'vs_baseline': None, 'dtype': args.mode, 'data': 'synthetic',
             'config': {'workload': (f'screen: one synthetic pocket (139 residues, 7 flexible) x {n} procedural ligands (PDBBind size law) x {spc} samples, '
                                     f'{args.inference_steps} steps + confidence, ligands split over the ranks, 2 ligands per sampler call (BASELINE.json configs[4]; it names 10000 ligands)'
@@ -301,6 +338,14 @@ def bench_set(args, model, conf, sa, ca, dev, world, rank, local, dist):
             'clocks': sampler.summary(), 'wall_s': wall, 'succeeded_on_rank0': ok,
             'top3': [(int(i), round(float(best[i]), 4)) for i in order[:3]],
             'e2e': {'value': poses / (wall * 1000.0 / 1000.0), 'unit': 'poses/s', 'h2d_bytes_per_step': int(model.static_h2d_bytes), 'd2h_bytes_per_step': None}}))
+        if args.dump_outputs is not None:
+            # per complex of rank 0's shard, in complex order: samples ranked by confidence, positions in the input frame
+            done = [r for r in res if r is not None]
+            dump_outputs(args.dump_outputs, {
+                'best_confidence': best,
+                'confidence': np.concatenate([r['confidence'] for r in done]),
+                'ligand_pos': np.concatenate([r['ligand_pos'].reshape(-1, 3) for r in done]),
+                'atom_pos': np.concatenate([r['atom_pos'].reshape(-1, 3) for r in done])})
     if world > 1:
         dist.destroy_process_group()
 
@@ -358,16 +403,17 @@ def main():
         torch.cuda.synchronize()
 
     def gather_rank(poses, confidence):
-        """The single collective of the path: all-gather final poses + confidences, rank by confidence."""
+        """The single collective of the path: all-gather final poses + confidences, rank by confidence
+        -> (all poses, all confidences, ranking)."""
         from diffdock_pocket_b200.parallel import gather_and_rank
-        return gather_and_rank(poses, confidence)[2]
+        return gather_and_rank(poses, confidence)
 
     # ---- e2e pass through the public API (host graphs in, host poses out) --------------------------------
     def e2e_step(dl):
         torch.manual_seed(7)
         out, c = ps.sampling(dl, model, args.inference_steps, sch, sch, sch, sch, dev, t2s, sa, concurrent_batches=not args.single_stream, **kw)
         poses = torch.stack([o['ligand'].pos for o in out]).to(dev)
-        return gather_rank(poses, c.reshape(-1).to(dev)).cpu()
+        return gather_rank(poses, c.reshape(-1).to(dev))[2].cpu()
 
     # ---- resident pass: plans + pose states (+ captured step graphs) built once, inputs already in HBM ----------
     chunks = [list(range(i, min(i + args.batch_size, args.samples))) for i in range(0, args.samples, args.batch_size)]
@@ -440,12 +486,16 @@ def main():
         torch.cuda.profiler.start()
     ev0.record()
     for _ in range(args.steps):
-        resident_step()
+        last = resident_step()
         flush.fill_(0)                           # L2 flush between timed iterations (256 MiB > 126 MB L2)
     ev1.record()
     barrier()
     if args.profile_range:
         torch.cuda.profiler.stop()
+    if rank == 0 and args.dump_outputs is not None:
+        # ligand poses and confidences of every rank (the gathered result), side-chain atoms of this rank's samples
+        dump_outputs(args.dump_outputs, {'ligand_pos': last[0], 'confidence': last[1], 'rank_order': last[2],
+                                         'atom_pos': torch.cat([pl.atom_pos for pl in plans]).reshape(N, -1, 3)})
     ms = ev0.elapsed_time(ev1) / args.steps
     launches = launches_per_step
     sampler.stop_flag = True

@@ -174,11 +174,21 @@ def make_async(R):
 
 
 # ------------------------------------------------------------------------------------------------- conv backward
+ROW_STRIDE = {'ea': 8, 'w1': 8}
+
+
+def sums(g):
+    g = g.astype(np.float64)
+    return np.array([g.sum(), np.abs(g).sum(), (g * g).sum()])
+
+
 def make_conv_grads(R):
     """Gradients of the reference's own ``TensorProductConvLayer`` (models/score_model.py:84-125 over models/layers.py /
     the FCTP restatement) by PyTorch autograd, as ``loss.backward()`` computes them in utils/training.py:147-191: with
     respect to the node features, edge attributes, edge harmonics and both Linears of the edge MLP.  The [weight_numel,
-    hidden] gradient of the second Linear is stored as a strided sample plus its sums (7 MB per case otherwise)."""
+    hidden] gradient of the second Linear is stored as a strided sample plus its sums (7 MB per case otherwise); those of
+    the edge attributes and of the first Linear as every ROW_STRIDE-th row plus their sums and shape (the file stays below
+    1 MB)."""
     d = {}
     for case, (in_ir, out_ir, nf, faster, sh_ir) in refpin.CONV_CASES.items():
         conv = R.score_model.TensorProductConvLayer(in_ir, sh_ir, out_ir, nf, residual=False, batch_norm=True, faster=faster)
@@ -192,8 +202,11 @@ def make_conv_grads(R):
             g = g.detach().numpy()
             if name == 'w2':
                 d[f'grad_{case}_w2_sample'] = g.reshape(-1)[::97].copy()
-                d[f'grad_{case}_w2_sums'] = np.array([g.astype(np.float64).sum(), np.abs(g).astype(np.float64).sum(),
-                                                      (g.astype(np.float64) ** 2).sum()])
+                d[f'grad_{case}_w2_sums'] = sums(g)
+            elif name in ROW_STRIDE:
+                key = f'grad_{case}_{name}'
+                d[key] = g[::ROW_STRIDE[name]].copy()
+                d[key + '_stride'], d[key + '_shape'], d[key + '_sums'] = np.array(ROW_STRIDE[name]), np.array(g.shape), sums(g)
             else:
                 d[f'grad_{case}_{name}'] = g
     save('ref_conv_grads.npz', d)
@@ -208,18 +221,19 @@ def run_forward(R, rm, b):
     return out, cap
 
 
-def pack_forward(d, tag, out, cap, atom_stride=5, rec_stride=2):
+def pack_forward(d, tag, out, cap, atom_stride=50, rec_stride=8, lig_stride=2):
+    """Per-layer features as every n-th row (strides stored with them) so that each fixture file stays below 1 MB."""
     for k, v in zip(('tr', 'rot', 'tor', 'sc'), out):
         d[f'{tag}_{k}'] = v.numpy()
     for nm in ('ll', 'lr', 'la', 'aa'):
         d[f'{tag}_{nm}'] = cap.rec[nm].numpy().astype(np.int32)
     for l, (lig, atom, rec) in enumerate(cap.layers()):
-        d[f'{tag}_lig_L{l}'] = lig.numpy()
+        d[f'{tag}_lig_L{l}'] = lig[::lig_stride].numpy()
         if atom is not None:
             d[f'{tag}_atom_L{l}'] = atom[::atom_stride].numpy()
         if rec is not None:
             d[f'{tag}_rec_L{l}'] = rec[::rec_stride].numpy()
-    d[f'{tag}_strides'] = np.array([atom_stride, rec_stride])
+    d[f'{tag}_strides'] = np.array([atom_stride, rec_stride, lig_stride])
 
 
 def make_forward(R):
@@ -261,7 +275,7 @@ def make_forward(R):
         d[f'{name}_lig_pos'] = torch.stack([x['ligand'].pos for x in dl]).numpy()
         d[f'{name}_atom_pos'] = torch.stack([x['atom'].pos for x in dl]).numpy()
         out, cap = run_forward(R, rm, ref_batch(R, dl, 0.35, sa))
-        pack_forward(d, name, out, cap, atom_stride=1, rec_stride=1)
+        pack_forward(d, name, out, cap, atom_stride=2, rec_stride=1, lig_stride=1)
         with torch.no_grad():
             d[f'{name}_confidence'] = rc(ref_batch(R, dl, 0.0, ca)).numpy()
     g = inputs.synthetic_complex(21, n_lig=3, n_res=30, flexible_residues=0)     # rigid ligand, nothing flexible

@@ -74,11 +74,11 @@ def _check(z, tag, pl, out, mode):
     tol = TOL[mode]
     for nm in ('ll', 'lr', 'la', 'aa'):                                            # graphs bit-exact with the reference run
         assert np.array_equal(pl.es[nm].edge_index().cpu().numpy().astype(np.int32), z[f'{tag}_{nm}']), nm
-    sa_, sr_ = int(z[f'{tag}_strides'][0]), int(z[f'{tag}_strides'][1])
+    sa_, sr_, sl_ = (int(s) for s in z[f'{tag}_strides'])             # rows stored: every sa_-th atom, sr_-th residue, sl_-th ligand atom
     worst = 0.0
     for l, (gl, ga, gr) in enumerate(pl.last_layers):
         want = z[f'{tag}_lig_L{l}']
-        e, ec = T.rel_err(gl[:, :want.shape[1]], want), T.rel_err_cols(gl[:, :want.shape[1]], want)
+        e, ec = T.rel_err(gl[::sl_, :want.shape[1]], want), T.rel_err_cols(gl[::sl_, :want.shape[1]], want)
         assert e < tol and ec < 4 * tol, (mode, 'lig', l, e, ec)
         worst = max(worst, e)
         if f'{tag}_atom_L{l}' in z:

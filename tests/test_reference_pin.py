@@ -189,9 +189,9 @@ def _check_forward(z, tag, om, out, strides=(1, 1)):
     dbg = om._debug
     for nm in ('ll', 'lr', 'la', 'aa'):
         assert np.array_equal(dbg[nm].numpy().astype(np.int32), z[f'{tag}_{nm}']), nm
-    sa_, sr_ = int(z[f'{tag}_strides'][0]), int(z[f'{tag}_strides'][1])
+    sa_, sr_, sl_ = (int(s) for s in z[f'{tag}_strides'])             # rows stored: every sa_-th atom, sr_-th residue, sl_-th ligand atom
     for l, (lig, atom, rec) in enumerate(dbg['layers']):
-        assert T.rel_err(lig, z[f'{tag}_lig_L{l}']) < 1e-5 and T.rel_err_cols(lig, z[f'{tag}_lig_L{l}']) < 1e-4, l
+        assert T.rel_err(lig[::sl_], z[f'{tag}_lig_L{l}']) < 1e-5 and T.rel_err_cols(lig[::sl_], z[f'{tag}_lig_L{l}']) < 1e-4, l
         if f'{tag}_atom_L{l}' in z:
             assert T.rel_err(atom[::sa_], z[f'{tag}_atom_L{l}']) < 1e-5, l
         if f'{tag}_rec_L{l}' in z:
@@ -400,17 +400,28 @@ def _conv_grads(conv, case):
     return dict(zip(('x', 'ea', 'sh', 'w1', 'b1', 'w2', 'b2'), [g.detach().cpu().numpy() for g in gs]))
 
 
+def _sums(g):
+    g = g.astype(np.float64)
+    return np.array([g.sum(), np.abs(g).sum(), (g * g).sum()])
+
+
 def check_conv_grads(got, case, rtol):
-    """Compare a dict of gradients with tests/golden/ref_conv_grads.npz (autograd through the reference's own layer)."""
+    """Compare a dict of gradients with tests/golden/ref_conv_grads.npz (autograd through the reference's own layer).
+    Gradients the fixture holds as a row sample (``_stride``, ``_shape``, ``_sums``) are compared on those rows and, over
+    the whole array, by their absolute and squared sums."""
     z = _z('ref_conv_grads.npz')
     for name in ('x', 'ea', 'sh', 'w1', 'b1', 'b2'):
-        want = z[f'grad_{case}_{name}']
-        assert got[name].shape == want.shape
-        assert T.rel_err(got[name], want) < rtol, (case, name, T.rel_err(got[name], want))
+        key, g = f'grad_{case}_{name}', got[name]
+        want = z[key]
+        if key + '_stride' in z:
+            assert g.shape == tuple(z[key + '_shape'])
+            np.testing.assert_allclose(_sums(g)[1:], z[key + '_sums'][1:], rtol=10 * rtol)
+            g = g[::int(z[key + '_stride'])]
+        assert g.shape == want.shape
+        assert T.rel_err(g, want) < rtol, (case, name, T.rel_err(g, want))
     w2 = got['w2']
     assert T.rel_err(w2.reshape(-1)[::97], z[f'grad_{case}_w2_sample']) < rtol
-    sums = np.array([w2.astype(np.float64).sum(), np.abs(w2).astype(np.float64).sum(), (w2.astype(np.float64) ** 2).sum()])
-    np.testing.assert_allclose(sums[1:], z[f'grad_{case}_w2_sums'][1:], rtol=10 * rtol)
+    np.testing.assert_allclose(_sums(w2)[1:], z[f'grad_{case}_w2_sums'][1:], rtol=10 * rtol)
 
 
 @pytest.mark.parametrize('case', list(refpin.CONV_CASES))

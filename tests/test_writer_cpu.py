@@ -1,5 +1,6 @@
 """Ranked-pose writer (SURVEY.md 8(f)-2; inference.py:198-240, process_mols.py:726-733, utils/visualise.py:62-132): text-level
-SDF / PDB output, checked by reading the files back.  Uses the reference's example complex when /root/reference is present."""
+SDF / PDB output, checked by reading the files back.  Input: the 3dpf holo ligand (with hydrogens) and its pocket, written
+from tests/golden/3dpf_holo.npz by ``scripts/make_fixtures.py pocket``."""
 import os
 
 import numpy as np
@@ -7,11 +8,9 @@ import pytest
 
 from diffdock_pocket_b200 import inputs, writer
 
-EX = '/root/reference/example_data'
-needs_example = pytest.mark.skipif(not os.path.exists(os.path.join(EX, '3dpf_ligand.sdf')), reason='reference example_data not present')
+EX = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', '3dpf_pocket')
 
 
-@needs_example
 def test_ranked_sdf_and_flexible_protein_pdb_round_trip(tmp_path):
     g = inputs.load_example_3dpf(EX, apo=False, flexible='auto')
     center = g.original_center.numpy()
