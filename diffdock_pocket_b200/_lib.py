@@ -102,6 +102,14 @@ _SIGS = {
     'ddp_pose_update': (i32, [C.POINTER(Pose), C.POINTER(StepCoef), vp]),
     'ddp_pose_max_ligand_atoms': (i32, []),
     'ddp_pose_update_dev': (i32, [C.POINTER(Pose), vp, vp]),
+    # deterministic mode (fixed-point accumulation, DDP_ACC_FIXED_SHIFT)
+    'ddp_fixed_to_float': (i32, [vp, C.c_int64, vp, vp]),
+    'ddp_tpconv_fp32_fixed': (i32, [C.POINTER(TpConv), C.POINTER(TpEdges), vp, vp, vp]),
+    'ddp_tpconv_umma_fixed': (i32, [C.POINTER(TpConv), vp, i32, C.POINTER(TpEdges), vp, vp, vp]),
+    'ddp_tpconv_umma_group_fixed': (i32, [vp, vp, i32, vp, vp, i32, vp, vp]),
+    'ddp_tp_backward_fixed': (i32, [C.POINTER(TpConv), i32, vp, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, vp]),
+    'ddp_node_update_fixed': (i32, [vp, i32, i32, C.POINTER(Update), i32, i32, i32, vp, i32, vp]),
+    'ddp_node_update_multi_fixed': (i32, [C.POINTER(NodeUpdateJob), i32, vp]),
 }
 EXPORTS = sorted(_SIGS)
 _LIB = None
@@ -182,3 +190,51 @@ def ptr(t):
 
 def stream_ptr():
     return torch.cuda.current_stream().cuda_stream
+
+
+# ------------------------------------------------------------------------------------------ deterministic mode
+FIXED_SHIFT = 32                  # DDP_ACC_FIXED_SHIFT (include/ddp_b200.h)
+STATUS_FIXED_RANGE = 1            # DDP_STATUS_FIXED_RANGE
+
+
+def deterministic():
+    """The accumulation mode callers get: fixed point (bitwise reproducible) under
+    ``torch.use_deterministic_algorithms(True)`` (also with ``warn_only=True``), fp32 atomics otherwise."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def sum_dtype(det):
+    return torch.int64 if det else torch.float32
+
+
+_STATUS = {}
+
+
+def _cuda_device(device):
+    device = torch.device(device)
+    return torch.device('cuda', torch.cuda.current_device()) if device.index is None else device
+
+
+def status_word(device):
+    """The sticky device status word of the fixed-point kernels on ``device`` (one int32 per device, allocated once, so
+    recorded launch sequences and captured graphs may hold its address)."""
+    device = _cuda_device(device)
+    w = _STATUS.get(device)
+    if w is None:
+        w = _STATUS[device] = torch.zeros(1, dtype=torch.int32, device=device)
+    return w
+
+
+def check_status(device, value=None):
+    """Read (and clear) the status word after a synchronisation: raises RuntimeError if a fixed-point accumulation saw a
+    non-finite partial sum or one outside the representable range since the last check.  ``value``: the word's content
+    already copied to the host with the results (otherwise it is read here).  The word is cleared before the exception,
+    so the next call on the same device starts clean."""
+    w = _STATUS.get(_cuda_device(device))
+    if w is None:
+        return
+    v = int(w.item()) if value is None else int(value)
+    if v:
+        w.zero_()
+        raise RuntimeError('deterministic accumulation: a partial sum was not finite or outside the fixed-point range '
+                           f'(|v| < 2^{63 - FIXED_SHIFT}); status word 0x{v:x}')

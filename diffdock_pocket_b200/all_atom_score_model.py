@@ -402,6 +402,10 @@ class TensorProductScoreModel(nn.Module):
         f32 = dict(dtype=torch.float32, device=dev)
         pl = Plan()
         pl.device = dev
+        # accumulation mode, fixed for the plan's lifetime: int64 fixed-point sums under torch.use_deterministic_algorithms
+        pl.deterministic = _lib.deterministic()
+        sum_t = dict(dtype=_lib.sum_dtype(pl.deterministic), device=dev)
+        pl.status = _lib.status_word(dev) if pl.deterministic else None
         lig, rec, atom = data['ligand'], data['receptor'], data['atom']
         B = int(data.num_graphs) if hasattr(data, 'num_graphs') or 'num_graphs' in data else 1
         pl.B = B
@@ -489,7 +493,7 @@ class TensorProductScoreModel(nn.Module):
             _lib.DegreeJob(idx=es[nm].row(r), n_edges_dev=ptr(es[nm].n_dev), edge_cap=es[nm].cap,
                            start=Eb if nm == 'll' else 0, deg=ptr(es[nm].deg[r])) for (nm, r) in dyn])
         # scatter-sum arena: three updates per node type
-        pl.sum_arena = torch.zeros((pl.NL + pl.NA + pl.NR) * F + 64, **f32)
+        pl.sum_arena = torch.zeros((pl.NL + pl.NA + pl.NR) * F + 64, **sum_t)
         pl.sum_used = [min(pl.sum_arena.numel(), (pl.NL + pl.NA + pl.NR) * d + 16) for d in [tpmod.irreps_dim(tpmod.parse_irreps(q)) for q in self.irrep_seq]]
         pl.ones_F = torch.ones(F, **f32)
         pl.one_i32 = torch.ones(1, **i32)
@@ -513,19 +517,19 @@ class TensorProductScoreModel(nn.Module):
             es['center'].set_static(ce.to(dev))
             pl.center = torch.zeros(B, 3, **f32)
             pl.center_deg = (lp[1:] - lp[:-1]).to(**i32)
-            pl.g_sum = torch.zeros(B, 12, **f32)
+            pl.g_sum = torch.zeros(B, 12, **sum_t)
             pl.g = torch.zeros(B, 12, **f32)
             pl.tr_out, pl.rot_out = torch.zeros(B, 3, **f32), torch.zeros(B, 3, **f32)
             if T > 0:
                 bonds = bond_ei[:, lig.edge_mask.bool()].long()
                 pl.tor_batch_h = lb[bonds[0]]
-                pl.tor = self._bond_head_plan(bonds, pl.tor_batch_h, B, pl.NL, int(nl_g.max()), dev)
+                pl.tor = self._bond_head_plan(bonds, pl.tor_batch_h, B, pl.NL, int(nl_g.max()), dev, pl.deterministic)
             if S > 0:
                 fr = data['flexResidues']
                 frb = fr.batch.cpu() if 'batch' in fr else torch.zeros(S, dtype=torch.long)
                 bonds = ap[:-1][frb] + fr.edge_idx.T.long().cpu()          # get_sc_tor_bonds, :638-652
                 pl.sc_batch_h = frb
-                pl.sc = self._bond_head_plan(bonds, frb, B, pl.NA, int(na_g.max()), dev)
+                pl.sc = self._bond_head_plan(bonds, frb, B, pl.NA, int(na_g.max()), dev, pl.deterministic)
             pl.tor_out = torch.zeros(max(T, 1), **f32)
             pl.sc_out = torch.zeros(max(S, 1), **f32)
         else:
@@ -542,7 +546,7 @@ class TensorProductScoreModel(nn.Module):
                 pl.flex_ptr = torch.cat([torch.zeros(1, dtype=torch.long), fcnt.cumsum(0)]).to(**i32)
         return pl
 
-    def _bond_head_plan(self, bonds, bond_batch, B, n_nodes, max_seg, dev):
+    def _bond_head_plan(self, bonds, bond_batch, B, n_nodes, max_seg, dev, det=False):
         i32 = dict(dtype=torch.int32, device=dev)
         f32 = dict(dtype=torch.float32, device=dev)
         h = Plan()
@@ -556,7 +560,7 @@ class TensorProductScoreModel(nn.Module):
         h.es = _EdgeSet(n * min(32, max_seg), self.ns, self.sh_dim, dev, with_slab=(n, min(32, max_seg)))
         h.sh_tor = torch.zeros(h.es.cap, self._tor_ftp['dim'], **f32)
         h.deg = torch.zeros(n, **i32)
-        h.sum = torch.zeros(n, 2 * self.ns, **f32)
+        h.sum = torch.zeros(n, 2 * self.ns, dtype=_lib.sum_dtype(det), device=dev)
         h.feat = torch.zeros(n, 2 * self.ns, **f32)
         return h
 
@@ -601,14 +605,16 @@ class TensorProductScoreModel(nn.Module):
                             sh=ptr(es.sh_conv if hasattr(es, 'sh_conv') else es.sh), agg=es.row(agg_r), ew=None,
                             n_edges_dev=ptr(es.n_dev), edge_cap=es.cap, out_scale=ptr(out_scale), agg_deg=ptr(agg_deg))
 
-    def _conv_group(self, L, st, items):
+    def _conv_group(self, L, st, items, status=None):
         """Fused tensor-product convolutions that share irreps (the convs of one interaction layer, or a single
         head conv).  items: (layer, packed, edge set, flip, x, p1, i1_row, p2, i2_row, sum_buf[, out_scale, agg_deg]).  On the tensor-core
-        path they run as ONE persistent kernel over the union of their edge tiles (ddp_tpconv_umma_group)."""
+        path they run as ONE persistent kernel over the union of their edge tiles (ddp_tpconv_umma_group).  ``status``: the
+        plan's status word in the deterministic mode (int64 fixed-point sum buffers, the *_fixed kernels), else None."""
         if len(items) > 1 and not getattr(self, 'group_convs', True):      # one launch per conv (per-conv timing)
             for it in items:
-                self._conv_group(L, st, [it])
+                self._conv_group(L, st, [it], status)
             return
+        det = status is not None
         prof = getattr(self, 'profile', None)
         if prof is not None:
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -624,10 +630,16 @@ class TensorProductScoreModel(nn.Module):
             imgs = (C.c_void_p * n)(*[ptr(it[1].umma_image(it[0], mode, it[4].device)) for it in items])
             edp = (C.c_void_p * n)(*[C.addressof(e) for e in eds])
             sums = (C.c_void_p * n)(*[ptr(it[9]) for it in items])
-            _lib.check(L.ddp_tpconv_umma_group(convs, imgs, mode, edp, sums, n, st), 'ddp_tpconv_umma_group')
+            if det:
+                _lib.check(L.ddp_tpconv_umma_group_fixed(convs, imgs, mode, edp, sums, n, ptr(status), st), 'ddp_tpconv_umma_group_fixed')
+            else:
+                _lib.check(L.ddp_tpconv_umma_group(convs, imgs, mode, edp, sums, n, st), 'ddp_tpconv_umma_group')
         else:
             for it, e in zip(items, eds):
-                _lib.check(L.ddp_tpconv_fp32(C.byref(it[1].cdesc), C.byref(e), ptr(it[9]), st), 'ddp_tpconv_fp32')
+                if det:
+                    _lib.check(L.ddp_tpconv_fp32_fixed(C.byref(it[1].cdesc), C.byref(e), ptr(it[9]), ptr(status), st), 'ddp_tpconv_fp32_fixed')
+                else:
+                    _lib.check(L.ddp_tpconv_fp32(C.byref(it[1].cdesc), C.byref(e), ptr(it[9]), st), 'ddp_tpconv_fp32')
         if prof is not None:
             ev1.record()
             if tc:
@@ -659,7 +671,8 @@ class TensorProductScoreModel(nn.Module):
         record: ~0.5 ms of host time per forward instead of ~2.8 ms of Python descriptor building.  (The recorded closures
         capture tensors, never the plan itself: a plan -> record -> plan cycle would keep freed plans away from the caching
         allocator until the cyclic GC runs, and every new plan would pay cudaMalloc.)"""
-        key = (self.conv_mode, torch.cuda.current_stream().cuda_stream, getattr(self, 'group_convs', True), id(self.packed()))
+        key = (self.conv_mode, torch.cuda.current_stream().cuda_stream, getattr(self, 'group_convs', True), id(self.packed()),
+               pl.deterministic)
         debug = return_layers or getattr(self, 'profile', None) is not None or getattr(self, 'profile_small', None) is not None or not self.replay_launches
         prog = getattr(pl, 'program', None)
         if prog is not None and prog[0] == key and not debug:
@@ -716,6 +729,9 @@ class TensorProductScoreModel(nn.Module):
         es = pl.es
         t_dev, tr_sigma, so3n, cutoff = pl.scal[0:B], pl.scal[B:2 * B], pl.scal[2 * B:3 * B], pl.scal[3 * B:4 * B]
         chk = _lib.check
+        # readers of the conv sums: the fixed-point forms in the deterministic mode (int64 sum buffers)
+        node_update = L.ddp_node_update_fixed if pl.deterministic else L.ddp_node_update
+        node_update_multi = L.ddp_node_update_multi_fixed if pl.deterministic else L.ddp_node_update_multi
         names = P['proj_names']
         scale = float(self.timestep_emb_func.keywords.get('scale', 1.0)) if hasattr(self.timestep_emb_func, 'keywords') else float(getattr(self.timestep_emb_func, 'scale', 1.0))
         chk(L.ddp_graph_sigma_proj(ptr(t_dev), B, scale, ptr(P['freq']), self.sigma_embed_dim, ptr(P['proj_w']), ptr(P['proj_b']),
@@ -812,7 +828,7 @@ class TensorProductScoreModel(nn.Module):
                             job(9 * l + 8, 'ar', True, xa, xr, 1, xa, 0, s_r)]
             # largest edge sets first: the round-robin tile walk then ends on the small ones
             grp.sort(key=lambda it: -it[2].cap)
-            self._conv_group(L, st, grp)
+            self._conv_group(L, st, grp, pl.status)
 
             def update(key, x_old, n, buf, items):
                 # the buffer is already normalised (deg = NULL); every live conv still contributes its BatchNorm shift
@@ -835,7 +851,7 @@ class TensorProductScoreModel(nn.Module):
                     node_jobs.append(Jr)
                 xa = xa_new
             t0 = self._small_begin()
-            chk(L.ddp_node_update_multi((_lib.NodeUpdateJob * len(node_jobs))(*node_jobs), len(node_jobs), st), 'ddp_node_update_multi')
+            chk(node_update_multi((_lib.NodeUpdateJob * len(node_jobs))(*node_jobs), len(node_jobs), st), 'ddp_node_update_multi')
             # algorithmic bytes per node: old features + the accumulated update in, new features out
             self._small_end(t0, 'node_update_multi', lambda jobs_=tuple((J.n, J.f_old, J.f_new) for J in node_jobs): sum(4 * n * (fo + 2 * fn) for n, fo, fn in jobs_))
             xl = xl_new
@@ -883,9 +899,9 @@ class TensorProductScoreModel(nn.Module):
             self._py(lambda a=h.sum, b=h.deg: (a.zero_(), b.zero_()))
             chk(L.ddp_degree(e.row(0), ptr(e.n_dev), e.cap, ptr(h.deg), st_), 'ddp_degree')
             pk = P[key + '_conv']
-            self._conv_group(L, st_, [(conv, pk, e, False, xn, xn, 1, h.attr, 0, h.sum)])
+            self._conv_group(L, st_, [(conv, pk, e, False, xn, xn, 1, h.attr, 0, h.sum)], pl.status)
             up = _lib.Update(sum=ptr(h.sum), deg=ptr(h.deg), scale=ptr(pk.bn_scale), shift=ptr(pk.bn_shift), n_edges_dev=ptr(e.n_dev))
-            chk(L.ddp_node_update(None, 0, 0, C.byref(up), 1, n, 2 * ns, ptr(h.feat), 2 * ns, st_), 'ddp_node_update')
+            chk(node_update(None, 0, 0, C.byref(up), 1, n, 2 * ns, ptr(h.feat), 2 * ns, st_), 'ddp_node_update')
             (w1, _), (w2, _) = P[mlp_key]
             arr = (_lib.MlpLayer * 2)(_lib.MlpLayer(wt=ptr(w1), b=None, n_in=2 * ns, n_out=ns, act=2),
                                       _lib.MlpLayer(wt=ptr(w2), b=None, n_in=ns, n_out=1, act=0))
@@ -909,10 +925,11 @@ class TensorProductScoreModel(nn.Module):
         chk(L.ddp_edge_embed(ptr(pl.center), ptr(pl.lig_pos), ptr(ec.edge), ec.cap, ptr(ec.n_dev), None, None, 0, ptr(U['center']),
                              C.byref(em['center']['desc']), ptr(ec.sh), ptr(ec.emb), st), 'ddp_edge_embed(center)')
         self._py(lambda a=pl.g_sum: a.zero_())
-        self._conv_group(L, st, [(self.final_conv, P['final_conv'], ec, False, xl, xl, 1 if self.fixed_center_conv else 0, None, 0, pl.g_sum)])
+        self._conv_group(L, st, [(self.final_conv, P['final_conv'], ec, False, xl, xl, 1 if self.fixed_center_conv else 0, None, 0, pl.g_sum)],
+                         pl.status)
         fc = P['final_conv']
         up = _lib.Update(sum=ptr(pl.g_sum), deg=ptr(pl.center_deg), scale=ptr(fc.bn_scale), shift=ptr(fc.bn_shift), n_edges_dev=ptr(ec.n_dev))
-        chk(L.ddp_node_update(None, 0, 0, C.byref(up), 1, B, 12, ptr(pl.g), 12, st), 'ddp_node_update')
+        chk(node_update(None, 0, 0, C.byref(up), 1, B, 12, ptr(pl.g), 12, st), 'ddp_node_update')
         (tw1, tb1, tw2, tb2), (rw1, rb1, rw2, rb2) = P['tr'], P['rot']
         if self.scale_by_sigma:
             trs, son = tr_sigma, so3n
@@ -935,4 +952,6 @@ class TensorProductScoreModel(nn.Module):
             if node_t is not None:
                 data[key].node_sigma_emb = self.timestep_emb_func(torch.as_tensor(node_t['t' if self.asyncronous_noise_schedule else 'tr'], dtype=torch.float32).to(pl.device))
         self._last_plan = pl
+        if pl.deterministic:
+            _lib.check_status(pl.device)          # (the k-NN edge list above was already read back: no extra stall)
         return out

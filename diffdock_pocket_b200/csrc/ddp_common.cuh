@@ -39,6 +39,21 @@ static inline cudaError_t ddp_smem_opt_in(K kernel, size_t bytes, bool *done) {
     return e;
 }
 
+// Fixed-point accumulation of the deterministic mode (DDP_ACC_FIXED_SHIFT, include/ddp_b200.h).  The range test also
+// rejects NaN; a rejected partial adds 0 and raises the status bit instead of wrapping into a wrong integer.
+__device__ __forceinline__ unsigned long long ddp_to_fixed(float v, uint32_t *status) {
+    constexpr float kScale = (float)(1ull << DDP_ACC_FIXED_SHIFT);
+    constexpr float kRange = (float)(1ull << (63 - DDP_ACC_FIXED_SHIFT));     // 2^31: |v * 2^S| < 2^63
+    if (!(fabsf(v) < kRange)) {
+        atomicOr(status, DDP_STATUS_FIXED_RANGE);
+        return 0ull;
+    }
+    return (unsigned long long)__float2ll_rn(v * kScale);
+}
+__device__ __forceinline__ float ddp_from_fixed(long long q) {
+    return __ll2float_rn(q) * (1.f / (float)(1ull << DDP_ACC_FIXED_SHIFT));
+}
+
 __device__ __forceinline__ int ddp_find_segment(const int32_t *__restrict__ ptr, int n_seg, int i) {
     // largest b with ptr[b] <= i  (ptr ascending, ptr[n_seg] = total)
     int lo = 0, hi = n_seg;

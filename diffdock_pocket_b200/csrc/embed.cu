@@ -291,7 +291,23 @@ edge_embed_fold_kernel(const float *__restrict__ pos_a, const float *__restrict_
 constexpr int kMaxUpdates = 4;
 struct UpdatePack { ddp_update_t u[kMaxUpdates]; int n; };
 
+// FIXED: the sums are int64 fixed point (ddp_node_update*_fixed, DDP_ACC_FIXED_SHIFT), converted on load.
+template <bool FIXED>
+__device__ __forceinline__ float load_sum(const float *sum, size_t off) {
+    if (FIXED) return ddp_from_fixed(reinterpret_cast<const long long *>(sum)[off]);
+    return sum[off];
+}
+template <bool FIXED>
+__device__ __forceinline__ float2 load_sum2(const float *sum, size_t off) {
+    if (FIXED) {
+        const long long *q = reinterpret_cast<const long long *>(sum) + off;
+        return make_float2(ddp_from_fixed(q[0]), ddp_from_fixed(q[1]));
+    }
+    return *reinterpret_cast<const float2 *>(sum + off);
+}
+
 // Flat float2 form: one thread per channel pair, few registers, full occupancy (f_new, strides even, 8-byte aligned bases).
+template <bool FIXED>
 __global__ void __launch_bounds__(256) node_update_vec_kernel(const float *__restrict__ old_x, int f_old, int ld_old, UpdatePack up,
                                                               int n, int f_new, float *__restrict__ new_x, int ld_new) {
     const int h = f_new >> 1;
@@ -305,7 +321,7 @@ __global__ void __launch_bounds__(256) node_update_vec_kernel(const float *__res
             if (k < up.n && __ldg(up.u[k].n_edges_dev) > 0) {
                 float2 m = make_float2(0.f, 0.f);
                 if (up.u[k].sum != nullptr) {
-                    m = *reinterpret_cast<const float2 *>(up.u[k].sum + (size_t)node * f_new + c);
+                    m = load_sum2<FIXED>(up.u[k].sum, (size_t)node * f_new + c);
                     if (up.u[k].deg != nullptr) {
                         const int dg = __ldg(up.u[k].deg + node);
                         const float cnt = (float)(dg < 1 ? 1 : dg);
@@ -328,6 +344,7 @@ __global__ void __launch_bounds__(256) node_update_vec_kernel(const float *__res
 constexpr int kMaxNodeJobs = 3;
 struct NodeJobs { ddp_node_update_job_t j[kMaxNodeJobs]; };
 constexpr int kNodesPerThread = 4;
+template <bool FIXED>
 __global__ void __launch_bounds__(256) node_update_multi_kernel(NodeJobs jobs) {
     // one thread = one channel pair of kNodesPerThread consecutive nodes: the per-channel scale / shift and the live
     // flags are loaded once, the node rows (old features, sums) are issued together before the arithmetic
@@ -363,7 +380,7 @@ __global__ void __launch_bounds__(256) node_update_multi_kernel(NodeJobs jobs) {
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
             m[k][i] = make_float2(0.f, 0.f);
-            if (has_sum[k] && node < J.n) m[k][i] = *reinterpret_cast<const float2 *>(J.updates[k].sum + (size_t)node * J.f_new + c);
+            if (has_sum[k] && node < J.n) m[k][i] = load_sum2<FIXED>(J.updates[k].sum, (size_t)node * J.f_new + c);
         }
     }
 #pragma unroll
@@ -390,6 +407,7 @@ __global__ void __launch_bounds__(256) node_update_multi_kernel(NodeJobs jobs) {
     }
 }
 
+template <bool FIXED>
 __global__ void node_update_kernel(const float *__restrict__ old_x, int f_old, int ld_old, UpdatePack up, int n,
                                    int f_new, float *__restrict__ new_x, int ld_new) {
     const int lane = threadIdx.x & 31;
@@ -412,7 +430,7 @@ __global__ void node_update_kernel(const float *__restrict__ old_x, int f_old, i
 #pragma unroll
             for (int k = 0; k < kMaxUpdates; ++k) {
                 if (live[k]) {
-                    const float m = up.u[k].sum ? __fdiv_rn(up.u[k].sum[(size_t)node * f_new + c], cnt[k]) : 0.f;
+                    const float m = up.u[k].sum ? __fdiv_rn(load_sum<FIXED>(up.u[k].sum, (size_t)node * f_new + c), cnt[k]) : 0.f;
                     const float sc = (up.u[k].scale && up.u[k].deg) ? __ldg(up.u[k].scale + c) : 1.f;
                     const float sf = up.u[k].shift ? __ldg(up.u[k].shift + c) : 0.f;
                     v += fmaf(m, sc, sf);
@@ -656,8 +674,9 @@ extern "C" int ddp_edge_embed(const float *pos_a, const float *pos_b, const int3
     return 0;
 }
 
-extern "C" int ddp_node_update(const float *old_x, int32_t f_old, int32_t ld_old, const ddp_update_t *updates,
-                               int32_t n_updates, int32_t n, int32_t f_new, float *new_x, int32_t ld_new, void *stream) {
+template <bool FIXED>
+static int node_update(const float *old_x, int32_t f_old, int32_t ld_old, const ddp_update_t *updates, int32_t n_updates, int32_t n,
+                       int32_t f_new, float *new_x, int32_t ld_new, void *stream) {
     if (!updates || !new_x || n_updates < 0 || n_updates > kMaxUpdates) return DDP_E_ARG;
     if (n <= 0) return 0;
     UpdatePack up;
@@ -670,15 +689,26 @@ extern "C" int ddp_node_update(const float *old_x, int32_t f_old, int32_t ld_old
     for (int i = 0; i < n_updates; ++i)
         vec = vec && (reinterpret_cast<uintptr_t>(updates[i].scale) % 8 == 0) && (reinterpret_cast<uintptr_t>(updates[i].shift) % 8 == 0);
     if (vec)
-        node_update_vec_kernel<<<(int)(((size_t)n * (f_new / 2) + 255) / 256), 256, 0, (cudaStream_t)stream>>>(old_x, f_old, ld_old, up, n,
+        node_update_vec_kernel<FIXED><<<(int)(((size_t)n * (f_new / 2) + 255) / 256), 256, 0, (cudaStream_t)stream>>>(old_x, f_old, ld_old, up, n,
                                                                                                       f_new, new_x, ld_new);
     else
-        node_update_kernel<<<grid_for((size_t)n * 32, 256), 256, 0, (cudaStream_t)stream>>>(old_x, f_old, ld_old, up, n, f_new, new_x, ld_new);
+        node_update_kernel<FIXED><<<grid_for((size_t)n * 32, 256), 256, 0, (cudaStream_t)stream>>>(old_x, f_old, ld_old, up, n, f_new, new_x, ld_new);
     DDP_LAUNCH_CHECK();
     return 0;
 }
 
-extern "C" int ddp_node_update_multi(const ddp_node_update_job_t *jobs_host, int32_t n_jobs, void *stream) {
+extern "C" int ddp_node_update(const float *old_x, int32_t f_old, int32_t ld_old, const ddp_update_t *updates,
+                               int32_t n_updates, int32_t n, int32_t f_new, float *new_x, int32_t ld_new, void *stream) {
+    return node_update<false>(old_x, f_old, ld_old, updates, n_updates, n, f_new, new_x, ld_new, stream);
+}
+
+extern "C" int ddp_node_update_fixed(const float *old_x, int32_t f_old, int32_t ld_old, const ddp_update_t *updates,
+                                     int32_t n_updates, int32_t n, int32_t f_new, float *new_x, int32_t ld_new, void *stream) {
+    return node_update<true>(old_x, f_old, ld_old, updates, n_updates, n, f_new, new_x, ld_new, stream);
+}
+
+template <bool FIXED>
+static int node_update_multi(const ddp_node_update_job_t *jobs_host, int32_t n_jobs, void *stream) {
     if (!jobs_host || n_jobs < 0 || n_jobs > kMaxNodeJobs) return DDP_E_ARG;
     NodeJobs jobs;
     size_t most = 0;
@@ -698,9 +728,17 @@ extern "C" int ddp_node_update_multi(const ddp_node_update_job_t *jobs_host, int
         most = tot > most ? tot : most;
     }
     if (m == 0) return 0;
-    node_update_multi_kernel<<<dim3((unsigned)((most + 255) / 256), m), 256, 0, (cudaStream_t)stream>>>(jobs);
+    node_update_multi_kernel<FIXED><<<dim3((unsigned)((most + 255) / 256), m), 256, 0, (cudaStream_t)stream>>>(jobs);
     DDP_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int ddp_node_update_multi(const ddp_node_update_job_t *jobs_host, int32_t n_jobs, void *stream) {
+    return node_update_multi<false>(jobs_host, n_jobs, stream);
+}
+
+extern "C" int ddp_node_update_multi_fixed(const ddp_node_update_job_t *jobs_host, int32_t n_jobs, void *stream) {
+    return node_update_multi<true>(jobs_host, n_jobs, stream);
 }
 
 extern "C" int ddp_segment_mean(const float *src, const int32_t *idx, const int32_t *ptr, int32_t n_seg, int32_t width,

@@ -9,7 +9,9 @@
 // (2 x 4 B x w_numel per edge), not the fused tensor-core form of the forward.
 //
 // One thread per (edge, input row u of a group): it walks the group's mul_out weight columns of that row, so the
-// contributions to g_x[u] / g_sh are summed in registers and leave with d1 + d2 atomics per thread.
+// contributions to g_x[u] / g_sh are summed in registers and leave with d1 + d2 atomics per thread.  FIXED
+// (ddp_tp_backward_fixed): those atomics add int64 fixed point (DDP_ACC_FIXED_SHIFT), so the gradients do not depend on
+// the order in which the threads of one node / edge arrive.
 #include "ddp_common.cuh"
 
 namespace {
@@ -17,12 +19,13 @@ namespace {
 constexpr int kMaxGroups = 64;
 constexpr int kMaxD = 5;      // 2l + 1 for l <= 2
 
+template <bool FIXED>
 __global__ void __launch_bounds__(256)
 tp_bwd_kernel(const ddp_tp_group_t *__restrict__ groups, int n_groups, const float *__restrict__ ctab, int rows_per_edge,
               const float *__restrict__ x, const int32_t *__restrict__ gather, int ldx,
               const float *__restrict__ sh, int sh_dim, const float *__restrict__ w, int w_numel,
               const float *__restrict__ g_out, int f_out, int n_edges,
-              float *__restrict__ g_w, float *__restrict__ g_x, float *__restrict__ g_sh) {
+              float *__restrict__ g_w, float *__restrict__ g_x, float *__restrict__ g_sh, uint32_t *status) {
     __shared__ ddp_tp_group_t sg[kMaxGroups];
     __shared__ int row_start[kMaxGroups + 1];
     if (threadIdx.x < n_groups) sg[threadIdx.x] = groups[threadIdx.x];
@@ -78,18 +81,32 @@ tp_bwd_kernel(const ddp_tp_group_t *__restrict__ groups, int n_groups, const flo
         }
         gwr[o] = acc;
     }
+    if (FIXED) {
+        unsigned long long *qx = reinterpret_cast<unsigned long long *>(g_x), *qs = reinterpret_cast<unsigned long long *>(g_sh);
+        if (qx != nullptr)
+            for (int i = 0; i < g.d1; ++i) atomicAdd(qx + (size_t)node * ldx + g.x_off + u * g.d1 + i, ddp_to_fixed(gx[i], status));
+        if (qs != nullptr)
+            for (int j = 0; j < g.d2; ++j) atomicAdd(qs + (size_t)e * sh_dim + g.sh_off + j, ddp_to_fixed(gs[j], status));
+        return;
+    }
     if (g_x != nullptr)
         for (int i = 0; i < g.d1; ++i) atomicAdd(g_x + (size_t)node * ldx + g.x_off + u * g.d1 + i, gx[i]);
     if (g_sh != nullptr)
         for (int j = 0; j < g.d2; ++j) atomicAdd(g_sh + (size_t)e * sh_dim + g.sh_off + j, gs[j]);
 }
 
+__global__ void fixed_to_float_kernel(const long long *__restrict__ src, long long n, float *__restrict__ dst) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        dst[i] = ddp_from_fixed(src[i]);
+}
+
 }  // namespace
 
-extern "C" int ddp_tp_backward(const ddp_tpconv_t *conv, int32_t rows_per_edge, const float *x, const int32_t *gather, int32_t ldx,
-                               const float *sh, const float *w, const float *g_out, int32_t n_edges, float *g_w, float *g_x, float *g_sh,
-                               void *stream) {
-    if (!conv || !x || !gather || !sh || !w || !g_out || !g_w) return DDP_E_ARG;
+template <bool FIXED>
+static int tp_backward(const ddp_tpconv_t *conv, int32_t rows_per_edge, const float *x, const int32_t *gather, int32_t ldx,
+                       const float *sh, const float *w, const float *g_out, int32_t n_edges, float *g_w, float *g_x, float *g_sh,
+                       uint32_t *status, void *stream) {
+    if (!conv || !x || !gather || !sh || !w || !g_out || !g_w || (FIXED && !status)) return DDP_E_ARG;
     const ddp_tpconv_t &c = *conv;
     if (!c.groups || !c.ctab) return DDP_E_ARG;
     if (c.n_groups <= 0 || c.n_groups > kMaxGroups || rows_per_edge <= 0) return DDP_E_SHAPE;
@@ -98,8 +115,31 @@ extern "C" int ddp_tp_backward(const ddp_tpconv_t *conv, int32_t rows_per_edge, 
     // l <= 2, are the caller's contract -- the host mirror checks them against its spec)
     const long long total = (long long)n_edges * rows_per_edge;
     const int grid = (int)((total + 255) / 256);
-    tp_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(c.groups, c.n_groups, c.ctab, rows_per_edge, x, gather, ldx, sh, c.sh_dim, w,
-                                                          c.w_numel, g_out, c.f_out, n_edges, g_w, g_x, g_sh);
+    tp_bwd_kernel<FIXED><<<grid, 256, 0, (cudaStream_t)stream>>>(c.groups, c.n_groups, c.ctab, rows_per_edge, x, gather, ldx, sh, c.sh_dim,
+                                                                 w, c.w_numel, g_out, c.f_out, n_edges, g_w, g_x, g_sh, status);
+    DDP_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int ddp_tp_backward(const ddp_tpconv_t *conv, int32_t rows_per_edge, const float *x, const int32_t *gather, int32_t ldx,
+                               const float *sh, const float *w, const float *g_out, int32_t n_edges, float *g_w, float *g_x, float *g_sh,
+                               void *stream) {
+    return tp_backward<false>(conv, rows_per_edge, x, gather, ldx, sh, w, g_out, n_edges, g_w, g_x, g_sh, nullptr, stream);
+}
+
+extern "C" int ddp_tp_backward_fixed(const ddp_tpconv_t *conv, int32_t rows_per_edge, const float *x, const int32_t *gather, int32_t ldx,
+                                     const float *sh, const float *w, const float *g_out, int32_t n_edges, float *g_w, int64_t *g_x,
+                                     int64_t *g_sh, uint32_t *status, void *stream) {
+    return tp_backward<true>(conv, rows_per_edge, x, gather, ldx, sh, w, g_out, n_edges, g_w, reinterpret_cast<float *>(g_x),
+                             reinterpret_cast<float *>(g_sh), status, stream);
+}
+
+extern "C" int ddp_fixed_to_float(const int64_t *src, int64_t n, float *dst, void *stream) {
+    if (!src || !dst || n < 0) return DDP_E_ARG;
+    if (n == 0) return 0;
+    const long long blocks = (n + 255) / 256;
+    const int grid = (int)(blocks < 8 * ddp_num_sms() ? blocks : 8 * ddp_num_sms());
+    fixed_to_float_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const long long *>(src), (long long)n, dst);
     DDP_LAUNCH_CHECK();
     return 0;
 }

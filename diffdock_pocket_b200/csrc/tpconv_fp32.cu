@@ -2,6 +2,9 @@
 // One CTA = 32 edges.  The per-edge weight vector w = W2 relu(W1 a + b1) + b2 exists only as an
 // 8-edge register tile per weight column; it is contracted with the table-driven Clebsch-Gordan
 // basis immediately and accumulated in shared memory, then scattered with red.global.add.
+// FIXED (deterministic mode, ddp_tpconv_fp32_fixed): the shared-memory tile and the global sums are int64 fixed point
+// (DDP_ACC_FIXED_SHIFT), so neither the order of the warps' shared atomics nor that of the CTAs' global ones shows in
+// the result.
 #include "ddp_common.cuh"
 
 namespace {
@@ -16,7 +19,7 @@ struct Smem {
     int *agg;
 };
 
-template <int TE>
+template <int TE, bool FIXED>
 __device__ __forceinline__ Smem carve(float *base, const ddp_tpconv_t &c, int ctab_len) {
     constexpr int LDS_E = TE + 4;
     Smem s;
@@ -25,19 +28,20 @@ __device__ __forceinline__ Smem carve(float *base, const ddp_tpconv_t &c, int ct
     s.x = s.h + c.hid * LDS_E;
     s.sh = s.x + c.f_in * LDS_E;
     s.out = s.sh + c.sh_dim * LDS_E;
-    s.ctab = s.out + c.f_out * LDS_E;
+    s.ctab = s.out + c.f_out * LDS_E * (FIXED ? 2 : 1);     // (FIXED: int64 tile, 8-byte aligned: every stride above is even)
     s.agg = reinterpret_cast<int *>(s.ctab + ctab_len);
     return s;
 }
 
-template <int TE>
+template <int TE, bool FIXED>
 __global__ void __launch_bounds__(NT, 2)
-tpconv_fp32_kernel(ddp_tpconv_t c, ddp_tpconv_edges_t ed, int ctab_len, float *__restrict__ sum) {
+tpconv_fp32_kernel(ddp_tpconv_t c, ddp_tpconv_edges_t ed, int ctab_len, float *__restrict__ sum, uint32_t *status) {
     constexpr int LDS_E = TE + 4;
     constexpr int NEG = TE / EG;          // edge groups per tile
     constexpr int TPG = NT / NEG;         // threads per edge group in the weight-column phase
     extern __shared__ __align__(16) float smem[];
-    Smem s = carve<TE>(smem, c, ctab_len);
+    Smem s = carve<TE, FIXED>(smem, c, ctab_len);
+    unsigned long long *out_q = reinterpret_cast<unsigned long long *>(s.out);     // FIXED only
     const int tid = threadIdx.x;
     const int n_edges = min(*ed.n_edges_dev, ed.edge_cap);
     for (int i = tid; i < ctab_len; i += NT) s.ctab[i] = c.ctab[i];
@@ -67,7 +71,10 @@ tpconv_fp32_kernel(ddp_tpconv_t c, ddp_tpconv_edges_t ed, int ctab_len, float *_
             const int el = idx / c.sh_dim, k = idx % c.sh_dim, e = e0 + el;
             s.sh[k * LDS_E + el] = (e < n_edges) ? ed.sh[(size_t)e * c.sh_dim + k] : 0.f;
         }
-        for (int idx = tid; idx < c.f_out * LDS_E; idx += NT) s.out[idx] = 0.f;
+        if (FIXED)
+            for (int idx = tid; idx < c.f_out * LDS_E; idx += NT) out_q[idx] = 0ull;
+        else
+            for (int idx = tid; idx < c.f_out * LDS_E; idx += NT) s.out[idx] = 0.f;
         if (tid < TE) s.agg[tid] = (e0 + tid < n_edges) ? ed.agg[e0 + tid] : -1;
         __syncthreads();
 
@@ -144,11 +151,17 @@ tpconv_fp32_kernel(ddp_tpconv_t c, ddp_tpconv_edges_t ed, int ctab_len, float *_
                     for (int i = 0; i < EG; ++i) {
                         float v = acc[i] * b[i];
                         for (int off = 16; off >= g.mul_out; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
-                        if ((tid & 31) < g.mul_out) atomicAdd(op + kk * LDS_E + i, v);
+                        if ((tid & 31) < g.mul_out) {
+                            if (FIXED) atomicAdd(out_q + (op - s.out) + kk * LDS_E + i, ddp_to_fixed(v, status));
+                            else atomicAdd(op + kk * LDS_E + i, v);
+                        }
                     }
                 } else if (active) {
 #pragma unroll
-                    for (int i = 0; i < EG; ++i) atomicAdd(op + kk * LDS_E + i, acc[i] * b[i]);
+                    for (int i = 0; i < EG; ++i) {
+                        if (FIXED) atomicAdd(out_q + (op - s.out) + kk * LDS_E + i, ddp_to_fixed(acc[i] * b[i], status));
+                        else atomicAdd(op + kk * LDS_E + i, acc[i] * b[i]);
+                    }
                 }
             }
         }
@@ -159,11 +172,12 @@ tpconv_fp32_kernel(ddp_tpconv_t c, ddp_tpconv_edges_t ed, int ctab_len, float *_
             const int el = idx / c.f_out, k = idx % c.f_out;
             const int node = s.agg[el];
             if (node >= 0) {
-                float v = s.out[k * LDS_E + el];
+                float v = FIXED ? ddp_from_fixed((long long)out_q[k * LDS_E + el]) : s.out[k * LDS_E + el];
                 if (ed.ew != nullptr) v *= ed.ew[e0 + el];
                 if (ed.out_scale != nullptr) v *= ed.out_scale[k];
                 if (ed.agg_deg != nullptr) v *= __frcp_rn((float)max(ed.agg_deg[node], 1));
-                atomicAdd(sum + (size_t)node * c.f_out + k, v);
+                if (FIXED) atomicAdd(reinterpret_cast<unsigned long long *>(sum) + (size_t)node * c.f_out + k, ddp_to_fixed(v, status));
+                else atomicAdd(sum + (size_t)node * c.f_out + k, v);
             }
         }
     }
@@ -171,8 +185,9 @@ tpconv_fp32_kernel(ddp_tpconv_t c, ddp_tpconv_edges_t ed, int ctab_len, float *_
 
 }  // namespace
 
-extern "C" int ddp_tpconv_fp32(const ddp_tpconv_t *conv, const ddp_tpconv_edges_t *edges, float *sum, void *stream) {
-    if (!conv || !edges || !sum) return DDP_E_ARG;
+template <bool FIXED>
+static int tpconv_fp32(const ddp_tpconv_t *conv, const ddp_tpconv_edges_t *edges, float *sum, uint32_t *status, void *stream) {
+    if (!conv || !edges || !sum || (FIXED && !status)) return DDP_E_ARG;
     const ddp_tpconv_t &c = *conv;
     const ddp_tpconv_edges_t &e = *edges;
     if (!c.w1t || !c.b1 || !c.w2t || !c.b2 || !c.groups || !c.ctab || !c.col_group) return DDP_E_ARG;
@@ -186,20 +201,29 @@ extern "C" int ddp_tpconv_fp32(const ddp_tpconv_t *conv, const ddp_tpconv_edges_
     if (ctab_len <= 0 || ctab_len > 64 * 125) return DDP_E_SHAPE;
     const bool small = e.edge_cap <= 8 * 2 * ddp_num_sms();          // few edges: 8-edge tiles keep all SMs busy
     const int TE = small ? 8 : 32;
-    const size_t smem = ((size_t)(c.k1 + c.hid + c.f_in + c.sh_dim + c.f_out) * (TE + 4) + ctab_len) * sizeof(float) + TE * sizeof(int);
+    const size_t smem = ((size_t)(c.k1 + c.hid + c.f_in + c.sh_dim + c.f_out * (FIXED ? 2 : 1)) * (TE + 4) + ctab_len) * sizeof(float) + TE * sizeof(int);
     if (smem > 200 * 1024) return DDP_E_SHAPE;
-    static size_t configured[DDP_MAX_DEVICES][2] = {{0, 0}};      // largest opt-in so far, per device and tile size
+    static size_t configured[DDP_MAX_DEVICES][2] = {{0, 0}};      // largest opt-in so far, per device and tile size (per FIXED)
     size_t &cfg = configured[ddp_current_device()][small];
     if (smem > cfg) {
-        cudaError_t err = small ? cudaFuncSetAttribute(tpconv_fp32_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                                : cudaFuncSetAttribute(tpconv_fp32_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t err = small ? cudaFuncSetAttribute(tpconv_fp32_kernel<8, FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                                : cudaFuncSetAttribute(tpconv_fp32_kernel<32, FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (err != cudaSuccess) return (int)err;
         cfg = smem;
     }
     int tiles = (e.edge_cap + TE - 1) / TE;
     int grid = tiles < 2 * ddp_num_sms() ? tiles : 2 * ddp_num_sms();
-    if (small) tpconv_fp32_kernel<8><<<grid, NT, smem, (cudaStream_t)stream>>>(c, e, ctab_len, sum);
-    else tpconv_fp32_kernel<32><<<grid, NT, smem, (cudaStream_t)stream>>>(c, e, ctab_len, sum);
+    if (small) tpconv_fp32_kernel<8, FIXED><<<grid, NT, smem, (cudaStream_t)stream>>>(c, e, ctab_len, sum, status);
+    else tpconv_fp32_kernel<32, FIXED><<<grid, NT, smem, (cudaStream_t)stream>>>(c, e, ctab_len, sum, status);
     DDP_LAUNCH_CHECK();
     return 0;
+}
+
+extern "C" int ddp_tpconv_fp32(const ddp_tpconv_t *conv, const ddp_tpconv_edges_t *edges, float *sum, void *stream) {
+    return tpconv_fp32<false>(conv, edges, sum, nullptr, stream);
+}
+
+extern "C" int ddp_tpconv_fp32_fixed(const ddp_tpconv_t *conv, const ddp_tpconv_edges_t *edges, int64_t *sum, uint32_t *status,
+                                     void *stream) {
+    return tpconv_fp32<true>(conv, edges, reinterpret_cast<float *>(sum), status, stream);
 }

@@ -301,6 +301,26 @@ __device__ __forceinline__ void red_row(float *dst, const float (&acc)[NA]) {
     }
 }
 
+// Deterministic mode (ddp_tpconv_umma*_fixed): the same pre-reduced partial sums, each converted to int64 fixed point
+// (DDP_ACC_FIXED_SHIFT) and added with a 64-bit integer reduction -- associative, so the order in which CTAs, the two
+// epilogue warpgroups and the split work items land does not show.  There is no vector form of red.add.u64: N
+// reductions instead of N / 4.  dst is the row's first int64.
+__device__ __forceinline__ void red_add_u64(unsigned long long *p, unsigned long long v) {
+    asm volatile("red.global.add.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+template <int N, int NA>
+__device__ __forceinline__ void red_row_fixed(unsigned long long *dst, const float (&acc)[NA], uint32_t *status) {
+    static_assert(N <= NA, "block wider than the accumulator");
+#pragma unroll
+    for (int o = 0; o < N; ++o) red_add_u64(dst + o, ddp_to_fixed(acc[o], status));
+}
+// sum row of an output block: fp32 vector reductions, or fixed point in the deterministic mode
+template <int N, bool FIXED, int NA>
+__device__ __forceinline__ void flush_row(float *sum, size_t off, const float (&acc)[NA], uint32_t *status) {
+    if constexpr (FIXED) red_row_fixed<N>(reinterpret_cast<unsigned long long *>(sum) + off, acc, status);
+    else red_row<N>(sum + off, acc);
+}
+
 // Warp-level segmented inclusive scan of the output block over runs of consecutive edges with the same aggregation
 // node (off = position of the lane inside its run): afterwards the last lane of every run holds the run's sum and is
 // the only one that issues the atomics.  Edge lists whose aggregation side is sorted (receptor graph, ligand side of
@@ -391,6 +411,8 @@ struct Jobs {
     int32_t n, f_in, f_out;
     long long *trace;     // optional timing trace of CTA 0 (ddp_tpconv_umma_set_trace), NULL in production
     Job job[MAX_JOBS];
+    uint32_t *status;     // sticky status word of the deterministic mode (FIXED kernels only; after job[] so that the
+                          // parameter offsets of the default kernels stay where they were)
 };
 [[maybe_unused]] constexpr int TRACE_EVENTS = 8, TRACE_TILES = 256;
 // trace[(role * TRACE_TILES + tile iteration) * TRACE_EVENTS + event] = clock64 (CTA 0, one lane per role)
@@ -587,7 +609,7 @@ __device__ __forceinline__ void gather_rows(const ddp_tpconv_edges_t &ed, int n_
 
 // L2: the edge harmonics have 9 components (sh_lmax = 2, e3nn FullyConnectedTensorProduct trunk convs) and kind-5 tiles
 // exist; a separate instantiation so that the sh_lmax = 1 kernel keeps its register allocation.
-template <int NS, int NV, int KS, bool SPLIT, bool L2>
+template <int NS, int NV, int KS, bool SPLIT, bool L2, bool FIXED>
 __global__ void __launch_bounds__(N_THREADS, 1)
 tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
     using C = Cfg<NS, NV, KS, SPLIT>;
@@ -1064,7 +1086,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                         }
                         const int steps = (seg >> 8) & 0xff;
                         if (steps) seg_scan<NS>(acc, seg & 0xff, steps);
-                        if (valid && (steps == 0 || (seg >> 16))) red_row<NS>(sum + (size_t)agg * f_out + out_off, acc);
+                        if (valid && (steps == 0 || (seg >> 16))) flush_row<NS, FIXED>(sum, (size_t)agg * f_out + out_off, acc, jobs.status);
                     }
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 3);
                 } else if (kind == 2) {
@@ -1198,7 +1220,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                         }
                         const int steps = (seg >> 8) & 0xff;
                         if (steps) seg_scan<3 * NV>(acc, seg & 0xff, steps);
-                        if (valid && (steps == 0 || (seg >> 16))) red_row<3 * NV>(sum + (size_t)agg * f_out + out_off, acc);
+                        if (valid && (steps == 0 || (seg >> 16))) flush_row<3 * NV, FIXED>(sum, (size_t)agg * f_out + out_off, acc, jobs.status);
                     }
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 3);
                 }
@@ -1432,10 +1454,10 @@ extern "C" int64_t ddp_tpconv_pack(const ddp_tpconv_t *conv, const ddp_tp_group_
     return (dst - base) == h.total_bytes ? 0 : DDP_E_SHAPE;
 }
 
-template <int NS, int NV, int KS, bool SPLIT, bool L2>
+template <int NS, int NV, int KS, bool SPLIT, bool L2, bool FIXED>
 static int launch_umma_l(const umma::Jobs &jobs, int tiles_cap, cudaStream_t st) {
     using C = umma::Cfg<NS, NV, KS, SPLIT>;
-    auto kern = umma::tpconv_umma_kernel<NS, NV, KS, SPLIT, L2>;
+    auto kern = umma::tpconv_umma_kernel<NS, NV, KS, SPLIT, L2, FIXED>;
     static bool configured[DDP_MAX_DEVICES] = {false};
     cudaError_t err = ddp_smem_opt_in(kern, C::SMEM, configured);
     if (err != cudaSuccess) return (int)err;
@@ -1445,9 +1467,9 @@ static int launch_umma_l(const umma::Jobs &jobs, int tiles_cap, cudaStream_t st)
     return 0;
 }
 
-template <int NS, int NV, int KS, bool SPLIT>
+template <int NS, int NV, int KS, bool SPLIT, bool FIXED>
 static int launch_umma(const umma::Jobs &jobs, int tiles_cap, cudaStream_t st, bool l2) {
-    return l2 ? launch_umma_l<NS, NV, KS, SPLIT, true>(jobs, tiles_cap, st) : launch_umma_l<NS, NV, KS, SPLIT, false>(jobs, tiles_cap, st);
+    return l2 ? launch_umma_l<NS, NV, KS, SPLIT, true, FIXED>(jobs, tiles_cap, st) : launch_umma_l<NS, NV, KS, SPLIT, false, FIXED>(jobs, tiles_cap, st);
 }
 
 static long long *g_umma_trace = nullptr;
@@ -1461,9 +1483,10 @@ extern "C" int ddp_tpconv_umma_set_trace(void *trace_dev) {
 #endif
 }
 
-extern "C" int ddp_tpconv_umma_group(const ddp_tpconv_t *const *convs, const void *const *packed, int32_t mode,
-                                     const ddp_tpconv_edges_t *const *edges, float *const *sums, int32_t n_jobs, void *stream) {
-    if (!convs || !packed || !edges || !sums) return DDP_E_ARG;
+template <bool FIXED>
+static int tpconv_umma_group(const ddp_tpconv_t *const *convs, const void *const *packed, int32_t mode, const ddp_tpconv_edges_t *const *edges,
+                             float *const *sums, int32_t n_jobs, uint32_t *status, void *stream) {
+    if (!convs || !packed || !edges || !sums || (FIXED && !status)) return DDP_E_ARG;
     if (n_jobs <= 0) return 0;
     if (n_jobs > umma::MAX_JOBS) return DDP_E_SHAPE;
     umma::Jobs jobs;
@@ -1472,6 +1495,7 @@ extern "C" int ddp_tpconv_umma_group(const ddp_tpconv_t *const *convs, const voi
     jobs.f_in = c0.f_in;
     jobs.f_out = c0.f_out;
     jobs.trace = g_umma_trace;
+    jobs.status = status;
     int tiles_cap = 0;
     for (int j = 0; j < n_jobs; ++j) {
         if (!convs[j] || !packed[j] || !edges[j] || !sums[j]) return DDP_E_ARG;
@@ -1495,14 +1519,31 @@ extern "C" int ddp_tpconv_umma_group(const ddp_tpconv_t *const *convs, const voi
     if (jobs.n == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     const bool l2 = c0.sh_dim == 9;
-    if (c0.ns == 60) return mode ? launch_umma<60, 10, 64, true>(jobs, tiles_cap, st, l2) : launch_umma<60, 10, 64, false>(jobs, tiles_cap, st, l2);
-    if (c0.ns == 24) return mode ? launch_umma<24, 6, 32, true>(jobs, tiles_cap, st, l2) : launch_umma<24, 6, 32, false>(jobs, tiles_cap, st, l2);
-    if (c0.ns == 16) return mode ? launch_umma<16, 4, 32, true>(jobs, tiles_cap, st, l2) : launch_umma<16, 4, 32, false>(jobs, tiles_cap, st, l2);
+    if (c0.ns == 60) return mode ? launch_umma<60, 10, 64, true, FIXED>(jobs, tiles_cap, st, l2) : launch_umma<60, 10, 64, false, FIXED>(jobs, tiles_cap, st, l2);
+    if (c0.ns == 24) return mode ? launch_umma<24, 6, 32, true, FIXED>(jobs, tiles_cap, st, l2) : launch_umma<24, 6, 32, false, FIXED>(jobs, tiles_cap, st, l2);
+    if (c0.ns == 16) return mode ? launch_umma<16, 4, 32, true, FIXED>(jobs, tiles_cap, st, l2) : launch_umma<16, 4, 32, false, FIXED>(jobs, tiles_cap, st, l2);
     return DDP_E_UNSUPPORTED;
+}
+
+extern "C" int ddp_tpconv_umma_group(const ddp_tpconv_t *const *convs, const void *const *packed, int32_t mode,
+                                     const ddp_tpconv_edges_t *const *edges, float *const *sums, int32_t n_jobs, void *stream) {
+    return tpconv_umma_group<false>(convs, packed, mode, edges, sums, n_jobs, nullptr, stream);
 }
 
 extern "C" int ddp_tpconv_umma(const ddp_tpconv_t *conv, const void *packed, int32_t mode, const ddp_tpconv_edges_t *edges,
                                float *sum, void *stream) {
     if (!conv || !packed || !edges || !sum) return DDP_E_ARG;
     return ddp_tpconv_umma_group(&conv, &packed, mode, &edges, &sum, 1, stream);
+}
+
+extern "C" int ddp_tpconv_umma_group_fixed(const ddp_tpconv_t *const *convs, const void *const *packed, int32_t mode,
+                                           const ddp_tpconv_edges_t *const *edges, int64_t *const *sums, int32_t n_jobs,
+                                           uint32_t *status, void *stream) {
+    return tpconv_umma_group<true>(convs, packed, mode, edges, reinterpret_cast<float *const *>(sums), n_jobs, status, stream);
+}
+
+extern "C" int ddp_tpconv_umma_fixed(const ddp_tpconv_t *conv, const void *packed, int32_t mode, const ddp_tpconv_edges_t *edges,
+                                     int64_t *sum, uint32_t *status, void *stream) {
+    if (!conv || !packed || !edges || !sum) return DDP_E_ARG;
+    return ddp_tpconv_umma_group_fixed(&conv, &packed, mode, &edges, &sum, 1, status, stream);
 }

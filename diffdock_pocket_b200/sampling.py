@@ -40,6 +40,7 @@ from scipy.spatial.transform import Rotation as R
 from .diffusion_utils import PoseState, modify_conformer, modify_sidechains
 from .all_atom_score_model import STATIC_KEYS
 from .hetero import Batch
+from . import _lib
 
 
 def randomize_position(data_list, no_torsion, no_random, tr_sigma_max, pocket_knowledge=False, pocket_cutoff=7,
@@ -141,6 +142,26 @@ def _same_tables(a, b):
         elif not np.array_equal(np.asarray(x), np.asarray(y)):
             return False
     return True
+
+
+def _cache_key(model, confidence_model, device, batch_size, flexible_sidechains, no_torsion, use_graph, concurrent_batches,
+               deterministic, graph_keys):
+    """Key of one resident-state entry: everything its plans, recorded launch programs and captured step graphs were
+    built for -- including the accumulation mode, so that state built in one mode is never replayed in the other."""
+    return (id(model), id(confidence_model), getattr(model, 'conv_mode', None), getattr(model, 'group_convs', None), str(device),
+            batch_size, bool(flexible_sidechains), bool(no_torsion), bool(use_graph), bool(concurrent_batches), bool(deterministic),
+            tuple(graph_keys))
+
+
+def _cache_get(key, model, confidence_model, deterministic):
+    """The cached entry for ``key`` if it may be used now: not owned by an unfinished (deferred) call, built for these
+    model objects (ids can be recycled) and in this accumulation mode."""
+    e = _PLAN_CACHE.get(key)
+    if e is None or e['busy'] or e['models'][0]() is not model or e['deterministic'] != bool(deterministic):
+        return None
+    if confidence_model is not None and e['models'][1]() is not confidence_model:
+        return None
+    return e
 
 
 def clear_plan_cache():
@@ -349,6 +370,8 @@ def _sampling(data_list, model, inference_steps, tr_schedule, rot_schedule, tor_
     chunks = [list(range(i, min(i + batch_size, N))) for i in range(0, N, batch_size)]
     use_graph = bool(use_graph) and trace is None
     runners = [None] * len(chunks)
+    # accumulation mode of this call's plans (fixed-point sums under torch.use_deterministic_algorithms: bitwise reproducible)
+    det = bool(torch.are_deterministic_algorithms_enabled())
     # resident state of an earlier call on the same input (see the module docstring)
     cache_key = cached = full_key = cache_sig = None
     LAST_CALL['plan_reused'] = False
@@ -366,9 +389,8 @@ def _sampling(data_list, model, inference_steps, tr_schedule, rot_schedule, tor_
             memo.append((tabs, shape, _graph_key(g, flexible_sidechains)))
             return memo[-1][2]
         def full_key():
-            return (id(model), id(confidence_model), getattr(model, 'conv_mode', None), getattr(model, 'group_convs', None),
-                    str(device), batch_size, bool(flexible_sidechains), bool(ma.no_torsion), use_graph, bool(concurrent_batches),
-                    tuple(gkey(g) for g in data_list))
+            return _cache_key(model, confidence_model, device, batch_size, flexible_sidechains, ma.no_torsion, use_graph,
+                              concurrent_batches, det, (gkey(g) for g in data_list))
         # the content key costs ~0.1 ms per graph: on the critical path only when an entry of the same shape signature exists
         # (a possible hit); otherwise it is computed after this call's launches are enqueued, under the GPU work
         cache_sig = (N, tuple((g['ligand'].pos.shape[0], g['atom'].pos.shape[0], g['receptor'].pos.shape[0]) for g in data_list))
@@ -384,10 +406,7 @@ def _sampling(data_list, model, inference_steps, tr_schedule, rot_schedule, tor_
             full_key = None
         if retain and any(e['sig'] == cache_sig for e in _PLAN_CACHE.values()):
             cache_key = full_key()
-            cached = _PLAN_CACHE.get(cache_key)
-            if cached is not None and (cached['busy'] or cached['models'][0]() is not model or
-                                       (confidence_model is not None and cached['models'][1]() is not confidence_model)):
-                cached = None                                         # still owned by an unfinished (deferred) call / stale ids
+            cached = _cache_get(cache_key, model, confidence_model, det)
     # independent mini-batches alternate between two streams (see StepRunner.ctx); host-visible intermediates
     # (trace, trajectories, visualisation) keep the single-stream order
     single = len(chunks) < 2 or trace is not None or return_full_trajectory or visualization_list is not None \
@@ -534,7 +553,11 @@ def _sampling(data_list, model, inference_steps, tr_schedule, rot_schedule, tor_
             if confidence is not None:
                 conf_host = torch.empty(confidence.shape, dtype=confidence.dtype, pin_memory=True)
                 conf_host.copy_(confidence, non_blocking=True)
-            staged = (torch.cuda.Event(), conf_host)
+            status_host = None
+            if det:                                                   # the status word travels with the results
+                status_host = torch.empty(1, dtype=torch.int32, pin_memory=True)
+                status_host.copy_(_lib.status_word(device), non_blocking=True)
+            staged = (torch.cuda.Event(), conf_host, status_host)
             staged[0].record()
 
     if full_key is not None and cache_key is None and n_steps > 0:
@@ -546,10 +569,13 @@ def _sampling(data_list, model, inference_steps, tr_schedule, rot_schedule, tor_
             staged[0].synchronize()
             confidence = staged[1]
         write_back_all()                                              # the one device->host read of the poses
+        if det:                                                       # fixed-point range / NaN errors of the whole call
+            _lib.check_status(device, None if staged is None else int(staged[2][0]))
         if cache_key is not None and all(r is not None for r in runners) and n_steps > 0:
             # hand the resident state to the cache (or back to it): the next call on this input starts from here
             import weakref
             _PLAN_CACHE[cache_key] = {'runners': runners, 'conf_plans': conf_plans, 'streams': streams, 'single': single, 'busy': False, 'sig': cache_sig,
+                                      'deterministic': det,
                                       'models': (weakref.ref(model), weakref.ref(confidence_model) if confidence_model is not None else None)}
             _PLAN_CACHE.move_to_end(cache_key)
             while len(_PLAN_CACHE) > PLAN_CACHE_SIZE:

@@ -297,7 +297,9 @@ class _ConvFn(torch.autograd.Function):
         Hpre = torch.addmm(B1, A, W1.T)
         H = torch.relu(Hpre)
         Wn = W2.shape[0]
-        g_x, g_sh = torch.zeros_like(x), torch.zeros_like(sh)
+        det = _lib.deterministic()
+        acc_dtype = _lib.sum_dtype(det)                               # deterministic mode: fixed-point g_x / g_sh
+        g_x, g_sh = torch.zeros_like(x, dtype=acc_dtype), torch.zeros_like(sh, dtype=acc_dtype)
         g_W2, g_b2, g_H = torch.zeros_like(W2), torch.zeros_like(B2), torch.empty_like(H)
         chunk = max(1024, (1 << 27) // max(Wn, 1))                    # two [chunk, weight_numel] fp32 buffers of <= 0.5 GB each
         for c0 in range(0, E, chunk):
@@ -308,12 +310,24 @@ class _ConvFn(torch.autograd.Function):
                 ge = ge * ew.detach().float().reshape(-1, 1)[c0:c1]
             ge = ge.contiguous()
             g_w = torch.empty_like(Wt)
-            _lib.check(L.ddp_tp_backward(C.byref(bd['cdesc']), bd['rows'], ptr(x), src[c0:c1].data_ptr(), x.shape[1], sh[c0:c1].data_ptr(), ptr(Wt),
-                                         ptr(ge), c1 - c0, ptr(g_w), ptr(g_x), g_sh[c0:c1].data_ptr(), _lib.stream_ptr()),
-                       'ddp_tp_backward')
+            if det:
+                _lib.check(L.ddp_tp_backward_fixed(C.byref(bd['cdesc']), bd['rows'], ptr(x), src[c0:c1].data_ptr(), x.shape[1],
+                                                   sh[c0:c1].data_ptr(), ptr(Wt), ptr(ge), c1 - c0, ptr(g_w), ptr(g_x),
+                                                   g_sh[c0:c1].data_ptr(), ptr(_lib.status_word(dev)), _lib.stream_ptr()),
+                           'ddp_tp_backward_fixed')
+            else:
+                _lib.check(L.ddp_tp_backward(C.byref(bd['cdesc']), bd['rows'], ptr(x), src[c0:c1].data_ptr(), x.shape[1], sh[c0:c1].data_ptr(),
+                                             ptr(Wt), ptr(ge), c1 - c0, ptr(g_w), ptr(g_x), g_sh[c0:c1].data_ptr(), _lib.stream_ptr()),
+                           'ddp_tp_backward')
             g_W2.addmm_(g_w.T, H[c0:c1])
             g_b2 += g_w.sum(0)
             g_H[c0:c1] = g_w @ W2
+        if det:
+            q_x, q_sh = g_x, g_sh
+            g_x, g_sh = torch.empty_like(x), torch.empty_like(sh)
+            for q, f in ((q_x, g_x), (q_sh, g_sh)):
+                _lib.check(L.ddp_fixed_to_float(ptr(q), q.numel(), ptr(f), _lib.stream_ptr()), 'ddp_fixed_to_float')
+            _lib.check_status(dev)
         g_pre = g_H * (Hpre > 0)
         g_W1, g_b1, g_A = g_pre.T @ A, g_pre.sum(0), g_pre @ W1
         need = ctx.needs_input_grad
@@ -422,17 +436,27 @@ class TensorProductConvLayer(nn.Module):
             ed = _lib.TpEdges(emb=ptr(ea), p1=None, i1=None, ld1=0, p2=None, i2=None, ld2=0, x=ptr(x), gather=ei[1].data_ptr(),
                               ldx=x.shape[1], sh=ptr(sh), agg=ei[0].data_ptr(), ew=ptr(ew), n_edges_dev=ptr(n_dev), edge_cap=E)
         f_out = pk.spec.f_out
-        s = torch.zeros(out_nodes, f_out, device=dev)
+        det = _lib.deterministic()                                    # fixed-point sums: bitwise reproducible
+        s = torch.zeros(out_nodes, f_out, device=dev, dtype=_lib.sum_dtype(det))
+        status = ptr(_lib.status_word(dev)) if det else None
         if use_tc:
             mode = 0 if self.conv_mode == 'bf16' else 1
             img = pk.umma_image(self, mode, dev)
-            _lib.check(L.ddp_tpconv_umma(C.byref(pk.cdesc), ptr(img), mode, C.byref(ed), ptr(s), _lib.stream_ptr()), 'ddp_tpconv_umma')
+            if det:
+                _lib.check(L.ddp_tpconv_umma_fixed(C.byref(pk.cdesc), ptr(img), mode, C.byref(ed), ptr(s), status, _lib.stream_ptr()),
+                           'ddp_tpconv_umma_fixed')
+            else:
+                _lib.check(L.ddp_tpconv_umma(C.byref(pk.cdesc), ptr(img), mode, C.byref(ed), ptr(s), _lib.stream_ptr()), 'ddp_tpconv_umma')
+        elif det:
+            _lib.check(L.ddp_tpconv_fp32_fixed(C.byref(pk.cdesc), C.byref(ed), ptr(s), status, _lib.stream_ptr()), 'ddp_tpconv_fp32_fixed')
         else:
             _lib.check(L.ddp_tpconv_fp32(C.byref(pk.cdesc), C.byref(ed), ptr(s), _lib.stream_ptr()), 'ddp_tpconv_fp32')
         deg = torch.zeros(out_nodes, dtype=torch.int32, device=dev)
         _lib.check(L.ddp_degree(ei[0].data_ptr(), ptr(n_dev), E, ptr(deg), _lib.stream_ptr()), 'ddp_degree')
         up = _lib.Update(sum=ptr(s), deg=ptr(deg), scale=ptr(pk.bn_scale), shift=ptr(pk.bn_shift), n_edges_dev=ptr(n_dev))
         out = torch.empty(out_nodes, f_out, device=dev)
-        _lib.check(L.ddp_node_update(None, 0, 0, C.byref(up), 1, out_nodes, f_out, ptr(out), f_out, _lib.stream_ptr()),
-                   'ddp_node_update')
+        update = L.ddp_node_update_fixed if det else L.ddp_node_update
+        _lib.check(update(None, 0, 0, C.byref(up), 1, out_nodes, f_out, ptr(out), f_out, _lib.stream_ptr()), 'ddp_node_update')
+        if det:
+            _lib.check_status(dev)                                    # (synchronises: a stand-alone call returns checked results)
         return out

@@ -29,6 +29,26 @@ extern "C" {
 const char *ddp_version(void);
 
 /* ------------------------------------------------------------------------------------------------
+ * Deterministic accumulation.  The scatter-adds of the convolutions (forward and backward) add partial sums that
+ * arrive in whatever order the GPU schedules them; in fp32 the low bits of the result then depend on that order.  The
+ * *_fixed entry points below accumulate instead in signed 64-bit fixed point with ONE binary scale 2^S:
+ *   q = llrint(v * 2^S)   per partial sum v (multiplying by a power of two is exact: one rounding, to 2^-S absolute),
+ *   sum += q              integer addition is associative, so every arrival order gives the same bits,
+ *   v' = (float)sum * 2^-S  once, by the consumer (ddp_node_update*_fixed, ddp_fixed_to_float).
+ * S = 32: a partial may lie in (-2^31, 2^31) and is resolved to 2.3e-10.  The convolution outputs are O(1) to O(100)
+ * (BatchNorm-scaled features and their mean over <= a few hundred edges), so the range leaves > 20 bits of headroom, and
+ * a sum of even 10^5 partials carries at most 10^5 * 2^-33 = 1.2e-5 of rounding in ABSOLUTE terms -- more than 1e3 below the
+ * 1e-4 relative / per-channel gates the fp32 path is held to, and a sum of 2^32 full-range partials cannot wrap the
+ * int64.  A partial that is not finite or lies outside the range is not converted (it adds 0) and sets
+ * DDP_STATUS_FIXED_RANGE in the caller's sticky device status word (uint32, zeroed by the caller, bits are OR-ed in;
+ * kernels never trap): the host reads the word at a synchronisation point it already has and reports the error. */
+#define DDP_ACC_FIXED_SHIFT 32
+#define DDP_STATUS_FIXED_RANGE 1u
+
+/* dst[i] = (float)src[i] * 2^-DDP_ACC_FIXED_SHIFT for i < n (the single conversion back of a fixed-point sum). */
+int ddp_fixed_to_float(const int64_t *src, int64_t n, float *dst, void *stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Graph construction.  Replaces torch_cluster.radius / radius_graph / knn_graph (pytorch-cluster
  * 1.6.1 CUDA kernels; reference call sites models/all_atom_score_model.py:457,524,545-550,563,607,627).
  * Bit-exact with those kernels: fp32 squared distance accumulated x,y,z with FMA, strict `<`,
@@ -193,6 +213,11 @@ typedef struct {
 /* fp32 CUDA-core path: exact-arithmetic mode and fallback for irreps the tensor-core kernel does not
  * specialise (lmax = 2, torsion FCTP).  sum: [n_out][f_out], zeroed by the caller. */
 int ddp_tpconv_fp32(const ddp_tpconv_t *conv, const ddp_tpconv_edges_t *edges, float *sum, void *stream);
+/* Same convolution with deterministic accumulation (see DDP_ACC_FIXED_SHIFT): both the per-tile accumulation in shared
+ * memory and the scatter-add into sum are fixed point.  sum: int64 [n_out][f_out], zeroed by the caller; status: the
+ * sticky device status word. */
+int ddp_tpconv_fp32_fixed(const ddp_tpconv_t *conv, const ddp_tpconv_edges_t *edges, int64_t *sum, uint32_t *status,
+                          void *stream);
 
 /* Tensor-core path (tcgen05 / TMEM, bf16 operands, fp32 accumulate), for FasterTensorProduct-shaped
  * convs (l <= 1 row groups, k1 == hid == 3*ns).  mode: 0 = bf16 single pass, 1 = bf16x3 split
@@ -214,6 +239,14 @@ int ddp_tpconv_umma(const ddp_tpconv_t *conv, const void *packed, int32_t mode,
  * their 128-edge tiles, so small edge sets do not leave SMs idle.  Arrays of n_jobs HOST pointers. */
 int ddp_tpconv_umma_group(const ddp_tpconv_t *const *convs, const void *const *packed, int32_t mode,
                           const ddp_tpconv_edges_t *const *edges, float *const *sums, int32_t n_jobs, void *stream);
+/* Deterministic accumulation (see DDP_ACC_FIXED_SHIFT): the same kernels, but every partial sum of the segmented
+ * pre-reduction is converted to fixed point and added with a 64-bit integer reduction.  sums: int64 [n_out][f_out] each,
+ * zeroed by the caller; status: the sticky device status word.  Same packed images, modes and restrictions. */
+int ddp_tpconv_umma_fixed(const ddp_tpconv_t *conv, const void *packed, int32_t mode, const ddp_tpconv_edges_t *edges,
+                          int64_t *sum, uint32_t *status, void *stream);
+int ddp_tpconv_umma_group_fixed(const ddp_tpconv_t *const *convs, const void *const *packed, int32_t mode,
+                                const ddp_tpconv_edges_t *const *edges, int64_t *const *sums, int32_t n_jobs, uint32_t *status,
+                                void *stream);
 
 /* Training path (SURVEY 8(f) row 3): backward of the tensor product of one TensorProductConvLayer.  Replaces what
  * autograd does for `self.tp(node_attr[edge_dst], edge_sh, self.fc(edge_attr))` under `loss.backward()`
@@ -229,6 +262,12 @@ int ddp_tpconv_umma_group(const ddp_tpconv_t *const *convs, const void *const *p
 int ddp_tp_backward(const ddp_tpconv_t *conv, int32_t rows_per_edge /* sum of mul_in over conv->groups */, const float *x,
                     const int32_t *gather, int32_t ldx, const float *sh, const float *w, const float *g_out, int32_t n_edges,
                     float *g_w, float *g_x, float *g_sh, void *stream);
+/* Same, with g_x / g_sh accumulated deterministically in fixed point (see DDP_ACC_FIXED_SHIFT): int64 buffers of the same
+ * shapes, zeroed by the caller (they may collect several chunks of edges) and converted once with ddp_fixed_to_float;
+ * status: the sticky device status word.  g_w is written directly, as above. */
+int ddp_tp_backward_fixed(const ddp_tpconv_t *conv, int32_t rows_per_edge, const float *x, const int32_t *gather, int32_t ldx,
+                          const float *sh, const float *w, const float *g_out, int32_t n_edges, float *g_w, int64_t *g_x,
+                          int64_t *g_sh, uint32_t *status, void *stream);
 
 /* Developer aid: when trace_dev != NULL, CTA 0 of every following tensor-core conv launch records clock64()
  * timestamps of its MMA-issue and epilogue roles per weight tile into trace_dev (device int64 buffer); NULL turns
@@ -254,6 +293,12 @@ typedef struct {
     int32_t n, f_new; float *new_x; int32_t ld_new;
 } ddp_node_update_job_t;
 int ddp_node_update_multi(const ddp_node_update_job_t *jobs_host, int32_t n_jobs, void *stream);
+/* The same two updates for sums accumulated in fixed point by the *_fixed convolutions: every non-NULL
+ * ddp_update_t.sum points at int64 [n][f_new] (cast to const float * in the struct), converted with 2^-DDP_ACC_FIXED_SHIFT
+ * before the divide-by-degree, scale and shift above.  Everything else is unchanged. */
+int ddp_node_update_fixed(const float *old_x, int32_t f_old, int32_t ld_old, const ddp_update_t *updates, int32_t n_updates,
+                          int32_t n, int32_t f_new, float *new_x, int32_t ld_new, void *stream);
+int ddp_node_update_multi_fixed(const ddp_node_update_job_t *jobs_host, int32_t n_jobs, void *stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Heads (all_atom_score_model.py:329-434). */
