@@ -77,7 +77,6 @@ _SIGS = {
     'ddp_version': (C.c_char_p, []),
     'ddp_radius': (i32, [vp, vp, vp, vp, i32, i32, vp, f32, i32, i32, i32, vp, i32, vp, vp, i32, vp, vp]),
     'ddp_knn_graph': (i32, [vp, vp, i32, i32, i32, vp, i32, vp, vp, i32, vp, vp]),
-    'ddp_knn_set_grid': (i32, [i32]),
     'ddp_calpha_graph': (i32, [vp, vp, i32, i32, f32, i32, vp, i32, vp, vp, i32, vp, vp]),
     'ddp_degree': (i32, [vp, vp, i32, vp, vp]),
     'ddp_edge_embed': (i32, [vp, vp, vp, i32, vp, vp, vp, i32, vp, C.POINTER(EdgeMlp), vp, vp, vp]),
@@ -114,7 +113,7 @@ _SIGS = {
 EXPORTS = sorted(_SIGS)
 _LIB = None
 # kernels launched per C-ABI call (for the bench's gpu_launches claim)
-KERNELS_PER_CALL = {'ddp_radius': 3, 'ddp_knn_graph': 3, 'ddp_calpha_graph': 3, 'ddp_version': 0, 'ddp_pose_max_ligand_atoms': 0, 'ddp_tpconv_pack': 0, 'ddp_tpconv_umma_set_trace': 0, 'ddp_knn_set_grid': 0}
+KERNELS_PER_CALL = {'ddp_radius': 3, 'ddp_knn_graph': 3, 'ddp_calpha_graph': 3, 'ddp_version': 0, 'ddp_pose_max_ligand_atoms': 0, 'ddp_tpconv_pack': 0, 'ddp_tpconv_umma_set_trace': 0}
 COUNTS = {}
 
 

@@ -3,8 +3,6 @@
 // warp-per-query ordered scans (radius) and shared-memory-staged per-thread scans (kNN) that keep
 // the exact fp32 arithmetic and the first-K-by-index / tie-by-index rules, with device-side edge
 // counts (no host synchronisation) and a scan + compaction into fixed-capacity edge buffers.
-#include <cstdlib>
-
 #include "ddp_common.cuh"
 
 namespace {
@@ -240,191 +238,6 @@ knn_scan_filter_kernel(const float *__restrict__ x, const int32_t *__restrict__ 
     counts[j] = o;
 }
 
-// Grid-binned form of the filtered search (opt-in, DDP_KNN_GRID=1; see the measurement note at the launcher): every block stages ONE example's coordinates
-// in shared memory, bins them into a uniform cell grid there (cell edge >= the first filter radius, counting sort by cell)
-// and then serves a slice of the example's centres, 32 at a time, kKnnFSub threads per centre: the candidates of a centre
-// are the points of its 27 neighbouring cells that pass the SAME radius test as the plain filter above (the ball of the
-// first radius lies inside those cells), so the recorded candidate set, the selection by (distance, index) and hence the
-// result are identical -- only the ~1100 distance tests per centre of a protein pocket shrink to the ~140 points of 27
-// cells.  Centres with too few candidates (surface atoms) fall back to the wider radii over the whole staged example.
-constexpr int kGridMaxDim = 12;                               // cells per axis (the cell edge grows for larger extents)
-constexpr int kGridMaxCells = kGridMaxDim * kGridMaxDim * kGridMaxDim;
-constexpr float kGridR0 = 5.5f;                               // = radii2[0] of the filter
-template <int KP>
-__global__ void __launch_bounds__(kKnnFC * kKnnFSub)
-knn_grid_kernel(const float *__restrict__ x, const int32_t *__restrict__ ptr, int num_examples, int n, int blocks_per_example,
-                int32_t *__restrict__ slab, int slab_w, int32_t *__restrict__ counts) {
-    extern __shared__ __align__(16) unsigned char knn_smem[];
-    float *sx = reinterpret_cast<float *>(knn_smem);                              // [kKnnStage * 3]
-    int *cand = reinterpret_cast<int *>(sx + kKnnStage * 3);                       // [kKnnFilterCap][kKnnFC]
-    int *cnt = cand + kKnnFilterCap * kKnnFC;                                      // [kKnnFC]
-    int *cell_start = cnt + kKnnFC;                                                // [kGridMaxCells + 1]
-    int *cell_fill = cell_start + kGridMaxCells + 1;                               // [kGridMaxCells]
-    unsigned short *order = reinterpret_cast<unsigned short *>(cell_fill + kGridMaxCells);   // [kKnnStage] points sorted by cell
-    unsigned short *cell_of = order + kKnnStage;                                   // [kKnnStage]
-    __shared__ float red[6][kKnnFC * kKnnFSub / 32];
-    __shared__ float box[7];                                                       // min xyz, 1 / cell edge, dims as floats
-    constexpr int NT = kKnnFC * kKnnFSub;
-    const int tid = threadIdx.x, sub = tid % kKnnFSub, c = tid / kKnnFSub;
-    const int b = blockIdx.x / blocks_per_example, slice = blockIdx.x % blocks_per_example;
-    if (b >= num_examples) return;
-    const int beg = ptr[b], m = ptr[b + 1] - beg;
-    if (m <= 0) return;
-    const int per_slice = (m + blocks_per_example - 1) / blocks_per_example;
-    const int s0 = slice * per_slice, s1 = min(m, s0 + per_slice);
-    if (s0 >= s1) return;
-    if (m > kKnnStage) {                                                         // example too large to stage: plain scan from global memory
-        for (int tj = s0 + tid; tj < s1; tj += NT) {
-            const int j = beg + tj;
-            const float yx = x[3 * j], yy = x[3 * j + 1], yz = x[3 * j + 2];
-            float bd[KP];
-            int bi[KP];
-#pragma unroll
-            for (int e = 0; e < KP; ++e) { bd[e] = 1e10f; bi[e] = -1; }
-            for (int i = beg; i < beg + m; ++i) knn_insert<KP>(bd, bi, ddp_sqdist(x[3 * i], x[3 * i + 1], x[3 * i + 2], yx, yy, yz), i);
-            int o = 0;
-#pragma unroll
-            for (int e = 0; e < KP; ++e)
-                if (bi[e] != -1 && bi[e] != j) { slab[(size_t)j * slab_w + o] = bi[e]; ++o; }
-            counts[j] = o;
-        }
-        return;
-    }
-    // ---- stage + bounding box ---------------------------------------------------------------------------------
-    float lo[3] = {1e30f, 1e30f, 1e30f}, hi[3] = {-1e30f, -1e30f, -1e30f};
-    for (int t = tid; t < m; t += NT) {
-#pragma unroll
-        for (int a = 0; a < 3; ++a) {
-            const float v = x[3 * (beg + t) + a];
-            sx[3 * t + a] = v;
-            lo[a] = fminf(lo[a], v); hi[a] = fmaxf(hi[a], v);
-        }
-    }
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
-            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
-        }
-        if ((tid & 31) == 0) { red[a][tid >> 5] = lo[a]; red[3 + a][tid >> 5] = hi[a]; }
-    }
-    for (int t = tid; t < kGridMaxCells; t += NT) cell_fill[t] = 0;
-    __syncthreads();
-    if (tid == 0) {
-        float l[3], h[3], ext = 0.f;
-        for (int a = 0; a < 3; ++a) {
-            l[a] = red[a][0]; h[a] = red[3 + a][0];
-            for (int w = 1; w < NT / 32; ++w) { l[a] = fminf(l[a], red[a][w]); h[a] = fmaxf(h[a], red[3 + a][w]); }
-            ext = fmaxf(ext, h[a] - l[a]);
-        }
-        // cell edge: the first filter radius (plus a rounding margin), larger when the example would need more cells per axis
-        const float edge = fmaxf(kGridR0 * 1.001f, ext / (float)(kGridMaxDim - 1) * 1.001f);
-        for (int a = 0; a < 3; ++a) { box[a] = l[a]; box[4 + a] = floorf((h[a] - l[a]) / edge) + 1.f; }
-        box[3] = 1.f / edge;
-    }
-    __syncthreads();
-    const float inv = box[3];
-    const int dx = (int)box[4], dy = (int)box[5], dz = (int)box[6];
-    auto cell_coord = [&](float v, int a, int d) { return min(d - 1, max(0, (int)((v - box[a]) * inv))); };
-    // ---- counting sort of the points by cell -------------------------------------------------------------------
-    for (int t = tid; t < m; t += NT) {
-        const int cid = (cell_coord(sx[3 * t], 0, dx) * dy + cell_coord(sx[3 * t + 1], 1, dy)) * dz + cell_coord(sx[3 * t + 2], 2, dz);
-        cell_of[t] = (unsigned short)cid;
-        atomicAdd(&cell_fill[cid], 1);
-    }
-    __syncthreads();
-    const int n_cells = dx * dy * dz;
-    if (tid < 32) {                                                              // exclusive scan of the cell counts, one warp
-        int carry = 0;
-        for (int base = 0; base < n_cells; base += 32) {
-            const int i = base + tid;
-            const int v = i < n_cells ? cell_fill[i] : 0;
-            int sc = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int u = __shfl_up_sync(0xffffffffu, sc, o);
-                if (tid >= o) sc += u;
-            }
-            if (i < n_cells) { cell_start[i] = carry + sc - v; cell_fill[i] = carry + sc - v; }
-            carry += __shfl_sync(0xffffffffu, sc, 31);
-        }
-        if (tid == 0) cell_start[n_cells] = carry;
-    }
-    __syncthreads();
-    for (int t = tid; t < m; t += NT) order[atomicAdd(&cell_fill[cell_of[t]], 1)] = (unsigned short)t;
-    __syncthreads();
-    // ---- centres of this slice, kKnnFC at a time --------------------------------------------------------------------
-    const unsigned group = ((1u << kKnnFSub) - 1u) << ((tid & 31) - sub);        // the kKnnFSub lanes of this centre
-    const float radii2[3] = {kGridR0 * kGridR0, 7.25f * 7.25f, 10.f * 10.f};
-    for (int base = s0; base < s1; base += kKnnFC) {
-        const int tj = base + c;                                                 // staged index of this thread's centre
-        const bool live = tj < s1;
-        const int j = beg + tj;
-        float yx = 0.f, yy = 0.f, yz = 0.f;
-        if (live) { yx = sx[3 * tj]; yy = sx[3 * tj + 1]; yz = sx[3 * tj + 2]; }
-        bool need = live;
-#pragma unroll 1
-        for (int pass = 0; pass < 3; ++pass) {
-            if (sub == 0) cnt[c] = 0;
-            __syncwarp(group);
-            if (need) {
-                const float r2 = radii2[pass];
-                if (pass == 0) {
-                    const int cx = cell_coord(yx, 0, dx), cy = cell_coord(yy, 1, dy), cz = cell_coord(yz, 2, dz);
-                    // the (up to) 9 columns of cells along z around the centre: each is one contiguous range of `order`
-                    for (int q = sub; q < 9; q += kKnnFSub) {
-                        const int ax = cx + q / 3 - 1, ay = cy + q % 3 - 1;
-                        if (ax < 0 || ax >= dx || ay < 0 || ay >= dy) continue;
-                        const int c0 = (ax * dy + ay) * dz + max(cz - 1, 0), c1 = (ax * dy + ay) * dz + min(cz + 1, dz - 1);
-                        for (int k = cell_start[c0]; k < cell_start[c1 + 1]; ++k) {
-                            const int t = order[k];
-                            if (ddp_sqdist(sx[3 * t], sx[3 * t + 1], sx[3 * t + 2], yx, yy, yz) < r2) {
-                                const int pos = atomicAdd(&cnt[c], 1);
-                                if (pos < kKnnFilterCap) cand[pos * kKnnFC + c] = beg + t;
-                            }
-                        }
-                    }
-                } else {
-                    const int per = (m + kKnnFSub - 1) / kKnnFSub;
-                    for (int t = sub * per; t < min(m, (sub + 1) * per); ++t) {
-                        if (ddp_sqdist(sx[3 * t], sx[3 * t + 1], sx[3 * t + 2], yx, yy, yz) < r2) {
-                            const int pos = atomicAdd(&cnt[c], 1);
-                            if (pos < kKnnFilterCap) cand[pos * kKnnFC + c] = beg + t;
-                        }
-                    }
-                }
-            }
-            __syncwarp(group);
-            const int got = cnt[c];
-            need = need && !((got >= KP || got == m) && got <= kKnnFilterCap);
-            if (!__any_sync(group, need)) break;
-        }
-        if (live && sub == 0) {
-            float bd[KP];
-            int bi[KP];
-#pragma unroll
-            for (int e = 0; e < KP; ++e) { bd[e] = 1e10f; bi[e] = -1; }
-            if (!need) {
-                const int got = cnt[c];
-                for (int k = 0; k < got; ++k) {
-                    const int i = cand[k * kKnnFC + c] - beg;
-                    knn_insert_lex<KP>(bd, bi, ddp_sqdist(sx[3 * i], sx[3 * i + 1], sx[3 * i + 2], yx, yy, yz), beg + i);
-                }
-            } else {
-                for (int t = 0; t < m; ++t) knn_insert<KP>(bd, bi, ddp_sqdist(sx[3 * t], sx[3 * t + 1], sx[3 * t + 2], yx, yy, yz), beg + t);
-            }
-            int o = 0;
-#pragma unroll
-            for (int e = 0; e < KP; ++e) {
-                if (bi[e] != -1 && bi[e] != j) { slab[(size_t)j * slab_w + o] = bi[e]; ++o; }
-            }
-            counts[j] = o;
-        }
-        __syncwarp(group);
-    }
-}
-
 // Generic-k fallback (k + 1 <= 101, arrays in local memory).
 __global__ void knn_scan_generic_kernel(const float *__restrict__ x, const int32_t *__restrict__ ptr, int num_examples,
                                         int n, int kp, int32_t *__restrict__ slab, int slab_w,
@@ -601,13 +414,6 @@ extern "C" int ddp_radius(const float *x, const float *y, const int32_t *ptr_x, 
     return 0;
 }
 
-static int g_knn_grid_mode = -1;      // -1: take DDP_KNN_GRID from the environment on first use; 0 plain filtered scan; 1 grid-binned
-extern "C" int ddp_knn_set_grid(int32_t mode) {
-    const int prev = g_knn_grid_mode;
-    g_knn_grid_mode = mode ? 1 : 0;
-    return prev;
-}
-
 extern "C" int ddp_knn_graph(const float *x, const int32_t *ptr, int32_t num_examples, int32_t n, int32_t k,
                              int32_t *slab, int32_t slab_w, int32_t *counts, int32_t *edge, int32_t edge_cap,
                              int32_t *n_edges_dev, void *stream) {
@@ -625,25 +431,6 @@ extern "C" int ddp_knn_graph(const float *x, const int32_t *ptr, int32_t num_exa
         if (e1 != cudaSuccess || e2 != cudaSuccess) return (int)(e1 != cudaSuccess ? e1 : e2);
         const bool filt = kp == 9 || kp == 13;
         const int fgrid = (n + kKnnFC - 1) / kKnnFC + num_examples;
-        // Grid-binned search, opt-in (DDP_KNN_GRID=1 in the environment).  Measured on B200 on the atom graph of a resident
-        // mini-batch (20 pockets x 1098 heavy atoms, k = 8; scripts/dbg/knn_time.py, profiles/r2_knn_grid_ab.txt): 129 us per call
-        // against 77 us for the plain filtered scan, search + scan + compaction.  At ~1100 points per example the block-local
-        // binning (bounding box, counting sort by cell, cell-offset scan: six barriers) and the three centre rounds a block
-        // then serves serially cost more than the ~137 distance tests per thread they save; identical edge lists either way
-        // (tests/test_gpu_parity.py::test_grid_binned_knn_graph_bit_exact_on_pockets_and_edge_cases runs both).
-        // Blocks per example from the MEAN example size -- the sizes live on the device.
-        if (g_knn_grid_mode < 0) { const char *v = getenv("DDP_KNN_GRID"); g_knn_grid_mode = (v && v[0] == '1') ? 1 : 0; }
-        const bool g_knn_grid = g_knn_grid_mode == 1;
-        const size_t gsm = fsm + (size_t)(2 * kGridMaxCells + 1) * sizeof(int) + (size_t)2 * kKnnStage * sizeof(unsigned short);
-        static bool configured_g9[DDP_MAX_DEVICES] = {false}, configured_g13[DDP_MAX_DEVICES] = {false};
-        if (filt && g_knn_grid) {
-            cudaError_t e3 = kp == 9 ? ddp_smem_opt_in(knn_grid_kernel<9>, gsm, configured_g9) : ddp_smem_opt_in(knn_grid_kernel<13>, gsm, configured_g13);
-            if (e3 != cudaSuccess) return (int)e3;
-            int bpe = (2 * ddp_num_sms() + num_examples - 1) / num_examples;
-            bpe = max(1, min(bpe, (n / num_examples + kKnnFC - 1) / kKnnFC));
-            if (kp == 9) knn_grid_kernel<9><<<num_examples * bpe, kKnnFC * kKnnFSub, gsm, st>>>(x, ptr, num_examples, n, bpe, slab, slab_w, counts);
-            else knn_grid_kernel<13><<<num_examples * bpe, kKnnFC * kKnnFSub, gsm, st>>>(x, ptr, num_examples, n, bpe, slab, slab_w, counts);
-        } else
         if (filt && kp == 9) knn_scan_filter_kernel<9><<<fgrid, kKnnFC * kKnnFSub, fsm, st>>>(x, ptr, num_examples, n, slab, slab_w, counts);
         else if (filt) knn_scan_filter_kernel<13><<<fgrid, kKnnFC * kKnnFSub, fsm, st>>>(x, ptr, num_examples, n, slab, slab_w, counts);
         else if (kp == 9) knn_scan_kernel<9><<<grid_sub, kKnnThreads, 0, st>>>(x, ptr, num_examples, n, slab, slab_w, counts);

@@ -81,20 +81,11 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "W_%=:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@!p bra W_%=;\n\t}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
 // Waits with slack (the gather warp is a whole edge tile ahead, the TMA producer a ring of slabs): let the hardware park
 // the warp (suspend-time hint) and back off between polls instead of spinning -- in profiles/r1_ncu_umma_v23_summary.txt
 // the plain try_wait loops of these two roles are 22 % of all executed warp instructions, i.e. issue energy under a
-// power cap.  The latency-critical waits (issuers, epilogue) use the hint without the back-off (-DDDP_UMMA_SPIN restores
-// the plain loops).
+// power cap.  The latency-critical waits (issuers, epilogue) use the hint without the back-off (SLEEP_NS = 0): they wake
+// on completion.
 template <int SLEEP_NS>
 __device__ __forceinline__ void mbar_wait_relaxed(uint64_t *bar, uint32_t parity) {
     uint32_t done;
@@ -110,64 +101,24 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint64_t *bar, uint32_t parity
         if (SLEEP_NS > 0) __nanosleep(SLEEP_NS);
     }
 }
-// Debug build (-DDDP_UMMA_WATCHDOG, with -DDDP_UMMA_TRACE): a wait that has polled ~2^18 times records
-// (code, a, b, barrier parity asked for) of its warp in the host-visible trace buffer, so a deadlock can be read
-// from the host while the kernel still hangs (scripts/umma_watchdog.py).
-#ifdef DDP_UMMA_WATCHDOG
-__device__ __forceinline__ void mbar_wait_wd(uint64_t *bar, uint32_t parity, long long *trace, int code, int a, int b) {
-    uint32_t done = 0;
-    unsigned long long polls = 0;
-    while (!done) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}\n"
-            : "=r"(done)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-        if (!done && ++polls == (1ull << 18) && trace != nullptr && (threadIdx.x & 31) == 0) {
-            long long *rec = trace + ((size_t)blockIdx.x * 12 + (threadIdx.x >> 5)) * 4;   // 12 warps per CTA
-            rec[0] = code; rec[1] = a; rec[2] = b; rec[3] = parity;
-            __threadfence_system();
-        }
-    }
+// Split-phase barrier test for the MMA issue loop: mbar_test starts a non-blocking phase test whose predicate lives in a
+// PTX register declared once per kernel (DDP_DECLARE_TEST_PRED); mbar_finish consumes it later (falling back to the
+// blocking wait), so the ~100-cycle shared-memory round trip overlaps the tcgen05.mma issue in between.
+#define DDP_DECLARE_TEST_PRED() asm volatile(".reg .pred ddp_p0;")
+__device__ __forceinline__ void mbar_test(uint64_t *bar, uint32_t parity) {
+    asm volatile("mbarrier.test_wait.parity.shared::cta.b64 ddp_p0, [%0], %1;" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
 }
-#define DDP_WAIT(bar, par, code, a, b) mbar_wait_wd(bar, par, jobs.trace, code, a, b)
-#else
-#ifdef DDP_UMMA_SPIN
-#define DDP_WAIT(bar, par, code, a, b) mbar_wait(bar, par)
-#else
-#define DDP_WAIT(bar, par, code, a, b) mbar_wait_relaxed<0>(bar, par)   // suspend-time hint, no back-off: wakes on completion
-#endif
-#endif
-#if defined(DDP_UMMA_WATCHDOG) || defined(DDP_UMMA_SPIN)
-#define DDP_WAIT_RELAXED(SLEEP, bar, par, code, a, b) DDP_WAIT(bar, par, code, a, b)
-#else
-#define DDP_WAIT_RELAXED(SLEEP, bar, par, code, a, b) mbar_wait_relaxed<SLEEP>(bar, par)
-#endif
-// Split-phase barrier test for the MMA issue loop: mbar_test_pN starts a non-blocking phase test whose predicate
-// lives in a PTX register declared once per kernel (DDP_DECLARE_TEST_PREDS); mbar_finish_pN consumes it later (falling
-// back to the blocking wait), so the ~100-cycle shared-memory round trip overlaps the tcgen05.mma issue in between.
-#define DDP_DECLARE_TEST_PREDS() asm volatile(".reg .pred ddp_p0, ddp_p1, ddp_p2;")
-#define DDP_MBAR_SPLIT(N)                                                                                                   \
-    __device__ __forceinline__ void mbar_test_p##N(uint64_t *bar, uint32_t parity) {                                        \
-        asm volatile("mbarrier.test_wait.parity.shared::cta.b64 ddp_p" #N ", [%0], %1;" ::"r"(smem_u32(bar)), "r"(parity)   \
-                     : "memory");                                                                                           \
-    }                                                                                                                       \
-    __device__ __forceinline__ void mbar_finish_p##N(uint64_t *bar, uint32_t parity) {                                      \
-        asm volatile(                                                                                                       \
-            "{\n\t"                                                                                                         \
-            "@ddp_p" #N " bra D_%=;\n\t"                                                                                    \
-            "W_%=:\n\t"                                                                                                     \
-            "mbarrier.try_wait.parity.shared::cta.b64 ddp_p" #N ", [%0], %1;\n\t"                                           \
-            "@!ddp_p" #N " bra W_%=;\n\t"                                                                                   \
-            "D_%=:\n\t}\n" ::"r"(smem_u32(bar)),                                                                           \
-            "r"(parity)                                                                                                     \
-            : "memory");                                                                                                    \
-    }
-DDP_MBAR_SPLIT(0)
-DDP_MBAR_SPLIT(1)
-DDP_MBAR_SPLIT(2)
+__device__ __forceinline__ void mbar_finish(uint64_t *bar, uint32_t parity) {
+    asm volatile(
+        "{\n\t"
+        "@ddp_p0 bra D_%=;\n\t"
+        "W_%=:\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 ddp_p0, [%0], %1;\n\t"
+        "@!ddp_p0 bra W_%=;\n\t"
+        "D_%=:\n\t}\n" ::"r"(smem_u32(bar)),
+        "r"(parity)
+        : "memory");
+}
 __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
                  "l"(src), "r"(bytes), "r"(smem_u32(bar))
@@ -187,17 +138,9 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t ncols) {
 __device__ __forceinline__ void umma_commit(uint64_t *bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// D[tmem] (+)= A[smem] * B[smem]^T, bf16 inputs, fp32 accumulate, both operands K-major
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// Same with the descriptors given as their low words (start address >> 4 | LBO >> 4 << 16); the high word is the
-// constant SBO = 128 B (8 x 16 B core-matrix rows) | descriptor version 1, so advancing along K is one 32-bit add.
+// D[tmem] (+)= A[smem] * B[smem]^T, bf16 inputs, fp32 accumulate, both operands K-major, no-swizzle core matrices.
+// The shared-memory descriptors are given as their low words (start address >> 4 | LBO >> 4 << 16); the high word is
+// the constant SBO = 128 B (8 x 16 B core-matrix rows) | descriptor version 1, so advancing along K is one 32-bit add.
 constexpr uint32_t DESC_HI = 8u | (1u << 14);
 __device__ __forceinline__ void umma_bf16_lo(uint32_t tmem_d, uint32_t a_lo, uint32_t b_lo, uint32_t idesc, uint32_t accumulate) {
     asm volatile(
@@ -209,23 +152,6 @@ __device__ __forceinline__ void umma_bf16_lo(uint32_t tmem_d, uint32_t a_lo, uin
         "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(DESC_HI)
         : "memory");
 }
-// A operand from tensor memory (lane = row, column c = packed bf16 pair k = 2c, 2c + 1): no shared-memory read of A,
-// which in the SS form costs ~43 exposed cycles per MMA (profiles/r1_umma_microbench.txt)
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint32_t b_lo, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 db;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "mov.b64 db, {%2, %5};\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], db, %3, p;\n\t}\n" ::"r"(tmem_d),
-        "r"(tmem_a), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(DESC_HI)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t (&r)[8]) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]), "r"(r[1]),
-                 "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-                 : "memory");
-}
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // One lane of the (converged) warp: the tcgen05 / TMA issue paths run warp-uniform and only the instruction itself
 // is predicated, which keeps descriptors in uniform registers instead of per-lane broadcasts.
 __device__ __forceinline__ bool elect_one() {
@@ -236,16 +162,6 @@ __device__ __forceinline__ bool elect_one() {
         "selp.u32 %0, 1, 0, P;\n\t}\n"
         : "=r"(pred));
     return pred != 0;
-}
-// no-swizzle K-major shared-memory descriptor: 8x(16 B) core matrices, LBO = stride between the two
-// K-chunks of one MMA, SBO = stride between 8-row groups (cute::UMMA::SmemDescriptor, version 1)
-__device__ __forceinline__ uint64_t smem_desc(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    uint64_t d = 0;
-    d |= (uint64_t)((addr >> 4) & 0x3FFF);
-    d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-    d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-    d |= (uint64_t)1 << 46;
-    return d;
 }
 __device__ __forceinline__ uint32_t instr_desc(int n) {
     // c=f32 (1<<4), a=bf16 (1<<7), b=bf16 (1<<10), K-major A and B, N>>3 at bit 17, M>>4 at bit 24
@@ -349,48 +265,11 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
 // still holds ~2 weight tiles in flight (whole-tile slabs with 2 slots measured slower: the first MMA of a tile then
 // waits for all of its 72 KB).
 __host__ __device__ constexpr int stage_k_of(int ks, bool split) { return ks == 64 ? (split ? 32 : 64) : (split ? 16 : 32); }
-// Tile shapes.  TS variant (hidden activations as a TMEM-resident A operand, single-pass bf16 only): a scalar tile
-// covers ROWS_S basis rows x NS outputs padded to N = 192; TMEM holds two such fp32 accumulators next to the bf16
-// hidden activations (2 x 208 + 96 columns = 512).  SS variant (A from shared memory; always used by the split mode):
-// N = 240 scalar tiles, two 256-column accumulators.  A vector tile covers up to 2 NV basis rows x NV outputs, which
-// the epilogue reads in two passes of NV rows.
-// Measured on B200 (3dpf batch of 20, W = 10000 layers): SS 1.24 PFLOP/s, TS 1.04 PFLOP/s.  TS issues faster MMAs
-// (106 vs 148 cycles) but its smaller tiles pay the per-tile hand-over (~500 cycles on both the issue and the epilogue
-// side) more often and leave the tensor pipe idle in between, whereas in SS mode the exposed A-operand read hides
-// those gaps.  TS stays selectable (-DDDP_UMMA_TS=1) for further work on the hand-over.
-#ifndef DDP_UMMA_TS
-#define DDP_UMMA_TS 0
-#endif
-#ifndef DDP_UMMA_DUAL
-#define DDP_UMMA_DUAL 1
-#endif
-// DDP_UMMA_TOKEN = 1: the two issuers hand an issue-order token back and forth, so tiles reach the tensor pipe in tile
-// order.  The token is REQUIRED for correctness with a ring shorter than two tiles' slabs (4 slots, 3 slabs per tile in the
-// big-model configuration), not only an ordering nicety: an issuer that skips the other issuer's tile tests slot s for
-// fill F while fill F-1 of s is one of the OTHER issuer's slabs, and bulk copies that are in flight together may land out
-// of order (one misses in L2, a later one hits).  If that foreign slab is still in the air the parity test passes on the
-// stale phase; the MMAs read a slot that is being written, their commit frees it early and the producer's
-// mbarrier.arrive.expect_tx hits a barrier whose previous phase is still pending -> "Warp Illegal Instruction" at that
-// SYNCS.ARRIVE.TRANS64 (cuda-gdb, profiles/r2_token0_rootcause.txt; seen only with two conv kernels in flight on two
-// streams, where L2 contention reorders the copies; compute-sanitizer memcheck / synccheck / racecheck are clean for both
-// builds).  The token is released after an issuer has ISSUED its tile -- so after it has seen every slab of that tile
-// land -- and awaited before the first non-blocking parity test of the next tile, which closes the hole.
-// tests/test_umma_protocol_model.py reproduces both the failure (no token, out-of-order landing) and the fix.
-// 0 is a debug switch only.
-#ifndef DDP_UMMA_TOKEN
-#define DDP_UMMA_TOKEN 1
-#endif
-#ifndef DDP_UMMA_SEGSCAN
-#define DDP_UMMA_SEGSCAN 1
-#endif
-// Diagnostic only (wrong results): 2 = full epilogue (default); 1 = TMEM loads kept, tensor-product FMAs skipped -- "what
-// would the launch cost if the CUDA-core part of the epilogue were free" (profiles/r2_conv_energy_diag.txt).
-#ifndef DDP_DIAG_EPI
-#define DDP_DIAG_EPI 2
-#endif
-__host__ __device__ constexpr bool use_ts(bool split) { return DDP_UMMA_TS != 0 && !split; }
-__host__ __device__ constexpr int rows_scalar(int ns, bool ts) { return (ts ? 192 : 240) / ns; }
-__host__ __device__ constexpr int ncol_scalar(int ns, bool ts) { return (rows_scalar(ns, ts) * ns + 15) / 16 * 16; }
+// Tile shapes (A from shared memory): a scalar tile covers ROWS_S basis rows x NS outputs padded to N = 240, TMEM holds
+// two 256-column accumulators.  A vector tile covers up to 2 NV basis rows x NV outputs, which the epilogue reads in two
+// passes of NV rows.
+__host__ __device__ constexpr int rows_scalar(int ns) { return 240 / ns; }
+__host__ __device__ constexpr int ncol_scalar(int ns) { return (rows_scalar(ns) * ns + 15) / 16 * 16; }
 __host__ __device__ constexpr int rows_vector(int nv) { return 2 * nv; }
 __host__ __device__ constexpr int ncol_vector(int nv, int n_rows) { return (n_rows * nv + 15) / 16 * 16; }
 
@@ -430,32 +309,30 @@ template <int NS, int NV, int KS, bool SPLIT>
 struct Cfg {
     static constexpr int KP = 3 * KS;                       // padded K of both GEMMs (and padded hidden width N1)
     static constexpr int N1 = KP;
-    static constexpr bool TS = use_ts(SPLIT);               // hidden activations as a TMEM-resident A operand
-    static constexpr int ROWS_S = rows_scalar(NS, TS);
+    static constexpr int ROWS_S = rows_scalar(NS);
     static constexpr int NVAL_S = ROWS_S * NS;              // weight columns of a scalar tile
-    static constexpr int NCOL_S = ncol_scalar(NS, TS);      // ... padded to the UMMA N granularity
+    static constexpr int NCOL_S = ncol_scalar(NS);          // ... padded to the UMMA N granularity
     static constexpr int ROWS_V = rows_vector(NV);
     static constexpr int PASS_COLS = NV * NV;               // weight columns the epilogue handles per pass (NV rows)
     static constexpr int NCOL_V = ncol_vector(NV, ROWS_V);
     static constexpr int NCOL_MAX = (NCOL_S > N1 ? (NCOL_S > NCOL_V ? NCOL_S : NCOL_V) : (N1 > NCOL_V ? N1 : NCOL_V));
-    static constexpr int ACC_STRIDE = TS ? 208 : 256;       // TMEM columns between the two accumulators
-    static constexpr int H_COL = 2 * ACC_STRIDE;            // TS: first TMEM column of the hidden activations (KP / 2 columns)
+    static constexpr int ACC_STRIDE = 256;                  // TMEM columns between the two accumulators
     static constexpr int STAGE_K = stage_k_of(KS, SPLIT);
     static constexpr int STAGE_BYTES = NCOL_MAX * STAGE_K * 2 * (SPLIT ? 2 : 1);
     static constexpr int A_BYTES = TILE_M * KP * 2;         // one bf16 A image
-    // A operand buffers in shared memory.  TS: one (free again as soon as GEMM1 has run); SS: two, so that the next
-    // edge tile is gathered under the current GEMM2 (split mode: one, its hi + lo images are already 96 KB)
-    static constexpr int NBUF = (TS || SPLIT) ? 1 : 2;
+    // A operand buffers in shared memory: two, so that the next edge tile is gathered under the current GEMM2 (split
+    // mode: one, its hi + lo images are already 96 KB)
+    static constexpr int NBUF = SPLIT ? 1 : 2;
     static constexpr int A_TOTAL = A_BYTES * (SPLIT ? 2 : 1) * NBUF;
     static constexpr int MAX_TILES = 64;
     static constexpr int FIXED = 1024 + A_TOTAL + MAX_TILES * (int)sizeof(TileDesc) + 1024;
     static constexpr int STAGES_FIT = (220 * 1024 - FIXED) / STAGE_BYTES;
     static constexpr int STAGES = STAGES_FIT > 12 ? 12 : STAGES_FIT;
     static constexpr size_t SMEM = (size_t)FIXED + (size_t)STAGES * STAGE_BYTES;
-    static constexpr bool DUAL = DDP_UMMA_DUAL != 0 && STAGES >= KP / STAGE_K + 1;   // two MMA issuers (see the issue loop)
+    static constexpr bool DUAL = STAGES >= KP / STAGE_K + 1;   // two MMA issuers (see the issue loop)
     static constexpr int XN_RAW = 3 * NV > 3 * ROWS_S ? 3 * NV : 3 * ROWS_S;   // floats of x one tile reads (x (x) s1 tiles: 2 NV,
     static constexpr int XN = XN_RAW + (XN_RAW & 1);                              //  stride-3 kinds: NV or ROWS_S rows of 3)
-    static_assert(N1 % 16 == 0 && NCOL_MAX <= ACC_STRIDE && (TS ? H_COL + KP / 2 : H_COL) <= 512, "UMMA N / TMEM budget");
+    static_assert(N1 % 16 == 0 && NCOL_MAX <= ACC_STRIDE && 2 * ACC_STRIDE <= 512, "UMMA N / TMEM budget");
     static_assert(KS >= NS + 1 && KP % STAGE_K == 0, "K padding");
     static_assert(STAGES >= 2, "weight ring too small");
     static_assert(XN % 2 == 0, "x prefetch registers are loaded in pairs");
@@ -552,11 +429,7 @@ __device__ __forceinline__ void gather_rows(const ddp_tpconv_edges_t &ed, int n_
         srcs[h][1] = valid ? ed.p1 + (size_t)__ldg(ed.i1 + e) * ed.ld1 : nullptr;
         srcs[h][2] = valid ? ed.p2 + (size_t)__ldg(ed.i2 + e) * ed.ld2 : nullptr;
     }
-#ifdef DDP_UMMA_SPIN
-    mbar_wait(free_bar, free_parity);
-#else
     mbar_wait_relaxed<500>(free_bar, free_parity);
-#endif
 #pragma unroll
     for (int h = 0; h < ROWS; ++h) {
         const int r = row0 + lane + h * 32;
@@ -641,7 +514,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
         for (int s = 0; s < C::STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
         for (int b = 0; b < 2; ++b) {
             mbar_init(&tmem_full[b], 1); mbar_init(&tmem_empty[b], N_EPI);
-            mbar_init(&a_ready[b], N_GATHER); mbar_init(&a_free[b], (C::TS || !C::DUAL) ? 1 : 2);
+            mbar_init(&a_ready[b], N_GATHER); mbar_init(&a_free[b], C::DUAL ? 2 : 1);
         }
         mbar_init(h_ready, N_EPI);
         mbar_init(&tok[0], 1); mbar_init(&tok[1], 1);
@@ -724,7 +597,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                 const uint32_t bytes = slab_bytes(ncol, C::STAGE_K, SPLIT);
 #pragma unroll 1
                 for (int ks = 0; ks < C::KP / C::STAGE_K; ++ks) {
-                    DDP_WAIT_RELAXED(0, &empty[stage], phase ^ 1, 1, w, tt * 8 + ks);
+                    mbar_wait_relaxed<0>(&empty[stage], phase ^ 1);
                     if (elect_one()) {
                         mbar_expect_tx(&full[stage], bytes);
                         bulk_g2s(ring + (size_t)stage * C::STAGE_BYTES, src, bytes, &full[stage]);
@@ -747,7 +620,19 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
         // slab is split-phase (started before the group is issued, consumed after it).
         // (Configurations whose ring is shorter than one tile's slabs + 1 keep a single issuer: an issuer that skips a
         // whole foreign tile could otherwise wait on a slab whose slot is still two fills behind -- parity aliasing.)
-        DDP_DECLARE_TEST_PREDS();
+        // The two issuers hand an issue-order token back and forth, so tiles reach the tensor pipe in tile order.  The
+        // token is REQUIRED for correctness with a ring shorter than two tiles' slabs (4 slots, 3 slabs per tile in the
+        // big-model configuration), not only an ordering nicety: an issuer that skips the other issuer's tile tests slot s
+        // for fill F while fill F-1 of s is one of the OTHER issuer's slabs, and bulk copies that are in flight together
+        // may land out of order (one misses in L2, a later one hits).  If that foreign slab is still in the air the parity
+        // test passes on the stale phase; the MMAs read a slot that is being written, their commit frees it early and the
+        // producer's mbarrier.arrive.expect_tx hits a barrier whose previous phase is still pending -> "Warp Illegal
+        // Instruction" at that SYNCS.ARRIVE.TRANS64 (profiles/r2_token0_rootcause.txt; seen only with two conv kernels
+        // in flight on two streams, where L2 contention reorders the copies).  The token is released after an issuer has
+        // ISSUED its tile -- so after it has seen every slab of that tile land -- and awaited before the first
+        // non-blocking parity test of the next tile, which closes the hole.  tests/test_umma_protocol_model.py reproduces
+        // both the failure (no token, out-of-order landing) and the fix.
+        DDP_DECLARE_TEST_PRED();
         const uint32_t me = warp == 5 ? 0u : 1u;
         uint32_t stage = 0, phase = 0;
         uint32_t te_phase = 0;               // bit b: parity to wait on tmem_empty[b]
@@ -782,23 +667,22 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                 // B: LBO = ncol rows x 16 B; one K = 16 step advances the start address by 2 * LBO
                 const uint32_t b_lbo_word = ncol << 16;
                 const uint32_t b_step = 2u * ncol;                      // (2 * ncol * 16 B) >> 4
-                const bool ts = C::TS && t >= 0;                        // GEMM2 reads the hidden activations from TMEM
-                // the A buffer is free once its last reader has run: GEMM1 (TS) / both issuers' last tiles (SS)
-                const bool last_reader = C::TS ? tt < 0 : tt + (C::DUAL ? 2 : 1) >= nt;
+                // the A buffer is free once its last reader has run: both issuers' last tiles
+                const bool last_reader = tt + (C::DUAL ? 2 : 1) >= nt;
                 trace_ev(jobs.trace, 0, titer, 0);
-                if (tt < 0) DDP_WAIT(&a_ready[ab], (uint32_t)(it / C::NBUF) & 1u, 2, it, tt);
+                if (tt < 0) mbar_wait_relaxed<0>(&a_ready[ab], (uint32_t)(it / C::NBUF) & 1u);
                 // the first GEMM2 tile this warp issues in the item needs the hidden activations (tile 0, and tile 1 where
                 // it belongs to the other issuer); every warp toggles its phase once per item
-                if (tt == 0 || (C::DUAL && tt == 1)) DDP_WAIT(h_ready, hr_phase, 3, it, tt);
-                DDP_WAIT(&tmem_empty[buf], ((te_phase >> buf) & 1u) ^ 1u, 4, it, tt);
+                if (tt == 0 || (C::DUAL && tt == 1)) mbar_wait_relaxed<0>(h_ready, hr_phase);
+                mbar_wait_relaxed<0>(&tmem_empty[buf], ((te_phase >> buf) & 1u) ^ 1u);
                 te_phase ^= 1u << buf;
-                DDP_WAIT(&full[stage], phase, 5, it, tt * 16 + (int)stage);
-                if (C::DUAL && DDP_UMMA_TOKEN) {
+                mbar_wait_relaxed<0>(&full[stage], phase);
+                if (C::DUAL) {
                     // tiles are issued in tile order: everything above overlapped the other issuer's tile, only the
                     // first tcgen05.mma waits for its last one
                     // (one token per run of the other issuer's tiles: warp 5 owns GEMM1 and tile 0 of an even-length item
                     // back to back and signals only after the second)
-                    if (tok_pending > 0) { DDP_WAIT(&tok[me ^ 1u], tok_phase, 6, it, tt); tok_phase ^= 1u; tok_pending = 0; }
+                    if (tok_pending > 0) { mbar_wait_relaxed<0>(&tok[me ^ 1u], tok_phase); tok_phase ^= 1u; tok_pending = 0; }
                 }
                 tc_fence_after();
                 trace_ev(jobs.trace, 0, titer, 1);
@@ -808,20 +692,16 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                     // the slab of this group has landed (blocking wait above, or the finish of the previous group)
                     uint32_t ns_ = stage + 1, np_ = phase;
                     if (ns_ == C::STAGES) { ns_ = 0; np_ ^= 1; }
-#ifndef DDP_UMMA_WATCHDOG
-                    if (ks + 1 < NG) mbar_test_p0(&full[ns_], np_);
-#endif
+                    if (ks + 1 < NG) mbar_test(&full[ns_], np_);
                     const uint32_t b_addr = smem_u32(ring + (size_t)stage * C::STAGE_BYTES);
                     const uint32_t b_lo0 = ((b_addr >> 4) & 0x3FFFu) | b_lbo_word;
                     const uint32_t a_k = (uint32_t)(ks * (C::STAGE_K / 8)) * (uint32_t)(TILE_M * 16 >> 4);
-                    const uint32_t a_t = tmem_base + (uint32_t)C::H_COL + (uint32_t)(ks * (C::STAGE_K / 2));
                     if (elect_one()) {
 #pragma unroll
                         for (int kk = 0; kk < C::STAGE_K / 16; ++kk) {
                             const uint32_t a_off = a_k + (uint32_t)(2 * kk) * (uint32_t)(TILE_M * 16 >> 4);
                             const uint32_t b_lo = b_lo0 + (uint32_t)kk * b_step;
-                            if (ts) umma_bf16_ts(d_tmem, a_t + (uint32_t)(8 * kk), b_lo, idesc, (ks | kk) != 0);
-                            else umma_bf16_lo(d_tmem, a_hi_lo + a_off, b_lo, idesc, (ks | kk) != 0);
+                            umma_bf16_lo(d_tmem, a_hi_lo + a_off, b_lo, idesc, (ks | kk) != 0);
                             if (SPLIT) {
                                 const uint32_t bl_lo = b_lo + ((ncol * (uint32_t)C::STAGE_K * 2u) >> 4);
                                 umma_bf16_lo(d_tmem, a_lo_lo + a_off, b_lo, idesc, 1);
@@ -832,15 +712,11 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                         if (ks == NG - 1) {
                             umma_commit(&tmem_full[buf]);
                             if (last_reader) umma_commit(&a_free[ab]);
-                            if (C::DUAL && DDP_UMMA_TOKEN && !(tt < 0 && acc_of(0, nt) == 0u)) mbar_arrive(&tok[me]);
+                            if (C::DUAL && !(tt < 0 && acc_of(0, nt) == 0u)) mbar_arrive(&tok[me]);
                         }
                     }
                     __syncwarp();
-#ifndef DDP_UMMA_WATCHDOG
-                    if (ks + 1 < NG) { mbar_finish_p0(&full[ns_], np_); tc_fence_after(); }
-#else
-                    if (ks + 1 < NG) { DDP_WAIT(&full[ns_], np_, 11, it, tt * 16 + (int)ns_); tc_fence_after(); }
-#endif
+                    if (ks + 1 < NG) { mbar_finish(&full[ns_], np_); tc_fence_after(); }
                     stage = ns_; phase = np_;
                 }
                 trace_ev(jobs.trace, 0, titer, 3);
@@ -884,15 +760,14 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
         const uint32_t a_row_off = (uint32_t)((r >> 3) * 128 + (r & 7) * 16);
         const uint32_t taddr = tmem_base + lane_base + wg * (uint32_t)C::ACC_STRIDE;
         int it = 0;
-        // Warpgroup 0 only.  GEMM1 result -> ReLU -> hidden activations become the A operand of GEMM2 (TS: packed bf16 pairs
-        // into tensor memory, column c of the lane = k 2c, 2c + 1; SS: hi (/ lo) images back into the shared-memory A buffer
-        // in core-matrix order).  At an item boundary warpgroup 0's last own tile is the last but one of the item, and the next
-        // item's GEMM1 is issued behind the last tile: the ~2400 cycles until its result exists take the warpgroup's last flush
-        // and the next item's per-edge set-up (dependent global loads), so that after the conversion tile 0's epilogue is
-        // ready when its MMAs are (profiles/r2_umma_timeline_*.txt).
+        // Warpgroup 0 only.  GEMM1 result -> ReLU -> hidden activations become the A operand of GEMM2 (hi (/ lo) images back
+        // into the shared-memory A buffer in core-matrix order).  At an item boundary warpgroup 0's last own tile is the last
+        // but one of the item, and the next item's GEMM1 is issued behind the last tile: the ~2400 cycles until its result
+        // exists take the warpgroup's last flush and the next item's per-edge set-up (dependent global loads), so that after
+        // the conversion tile 0's epilogue is ready when its MMAs are (profiles/r2_umma_timeline_*.txt).
         auto convert_hidden = [&](uint8_t *a_hi_, uint8_t *a_lo_, int it_) {
             if (tracer) trace_ev(jobs.trace, 1, it_ * (n_tiles + 1), 0);
-            DDP_WAIT(&tmem_full[0], tf_phase, 8, it_, -1);
+            mbar_wait_relaxed<0>(&tmem_full[0], tf_phase);
             tf_phase ^= 1u;
             tc_fence_after();
             if (tracer) trace_ev(jobs.trace, 1, it_ * (n_tiles + 1), 1);
@@ -906,36 +781,28 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                     float v[16];
 #pragma unroll
                     for (int q = 0; q < 16; ++q) v[q] = fmaxf(__uint_as_float(w[c16 & 1][q]), 0.f);
-                    if (C::TS) {
-                        uint32_t pk[8];
 #pragma unroll
-                        for (int q = 0; q < 8; ++q) pk[q] = pack_bf16x2(v[2 * q], v[2 * q + 1]);
-                        tmem_st8(tmem_base + lane_base + (uint32_t)(C::H_COL + c16 * 8), pk);
-                    } else {
+                    for (int h8 = 0; h8 < 2; ++h8) {
+                        uint4 hi;
+                        hi.x = pack_bf16x2(v[8 * h8 + 0], v[8 * h8 + 1]); hi.y = pack_bf16x2(v[8 * h8 + 2], v[8 * h8 + 3]);
+                        hi.z = pack_bf16x2(v[8 * h8 + 4], v[8 * h8 + 5]); hi.w = pack_bf16x2(v[8 * h8 + 6], v[8 * h8 + 7]);
+                        const uint32_t off = (uint32_t)((c16 * 2 + h8) * (TILE_M * 16)) + a_row_off;
+                        *reinterpret_cast<uint4 *>(a_hi_ + off) = hi;
+                        if (SPLIT) {
+                            float u[8];
 #pragma unroll
-                        for (int h8 = 0; h8 < 2; ++h8) {
-                            uint4 hi;
-                            hi.x = pack_bf16x2(v[8 * h8 + 0], v[8 * h8 + 1]); hi.y = pack_bf16x2(v[8 * h8 + 2], v[8 * h8 + 3]);
-                            hi.z = pack_bf16x2(v[8 * h8 + 4], v[8 * h8 + 5]); hi.w = pack_bf16x2(v[8 * h8 + 6], v[8 * h8 + 7]);
-                            const uint32_t off = (uint32_t)((c16 * 2 + h8) * (TILE_M * 16)) + a_row_off;
-                            *reinterpret_cast<uint4 *>(a_hi_ + off) = hi;
-                            if (SPLIT) {
-                                float u[8];
-#pragma unroll
-                                for (int q = 0; q < 8; ++q) u[q] = v[8 * h8 + q] - __bfloat162float(__float2bfloat16_rn(v[8 * h8 + q]));
-                                uint4 lo;
-                                lo.x = pack_bf16x2(u[0], u[1]); lo.y = pack_bf16x2(u[2], u[3]);
-                                lo.z = pack_bf16x2(u[4], u[5]); lo.w = pack_bf16x2(u[6], u[7]);
-                                *reinterpret_cast<uint4 *>(a_lo_ + off) = lo;
-                            }
+                            for (int q = 0; q < 8; ++q) u[q] = v[8 * h8 + q] - __bfloat162float(__float2bfloat16_rn(v[8 * h8 + q]));
+                            uint4 lo;
+                            lo.x = pack_bf16x2(u[0], u[1]); lo.y = pack_bf16x2(u[2], u[3]);
+                            lo.z = pack_bf16x2(u[4], u[5]); lo.w = pack_bf16x2(u[6], u[7]);
+                            *reinterpret_cast<uint4 *>(a_lo_ + off) = lo;
                         }
                     }
                 }
             }
             if (tracer) trace_ev(jobs.trace, 1, it_ * (n_tiles + 1), 3);
-            if (C::TS) tmem_wait_st();
             tc_fence_before();
-            if (!C::TS) fence_proxy_async();
+            fence_proxy_async();
             mbar_arrive(h_ready);
             mbar_arrive(&tmem_empty[0]);
             if (tracer) trace_ev(jobs.trace, 1, it_ * (n_tiles + 1), 2);
@@ -999,7 +866,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                 const unsigned heads = __ballot_sync(0xffffffffu, lane_ == 0 || prev != key);
                 const int off = lane_ - (31 - __clz((int)(heads & (0xffffffffu >> (31 - lane_)))));
                 const int maxoff = __reduce_max_sync(0xffffffffu, off);
-                if (DDP_UMMA_SEGSCAN && __popc(heads) <= 16)
+                if (__popc(heads) <= 16)
                     seg = off | ((32 - __clz(maxoff)) << 8) | ((lane_ == 31 || ((heads >> (lane_ + 1)) & 1u)) ? 1 << 16 : 0);
             }
             if (tracer && wg == 0) trace_ev(jobs.trace, 2, it * (n_tiles + 1), 2);
@@ -1055,7 +922,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                     }
                     if (own_next) x_prefetch_tile<NS, NV, C::ROWS_S, C::XN>(xg, tdn, f_in, xn);
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 0);
-                    DDP_WAIT(&tmem_full[wg], tf_phase, 9, it, tt);
+                    mbar_wait_relaxed<0>(&tmem_full[wg], tf_phase);
                     tf_phase ^= 1u;
                     tc_fence_after();
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 1);
@@ -1068,7 +935,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
 #pragma unroll
                         for (int q = 0; q < 16; ++q) {
                             const int c = c16 * 16 + q;
-                            if (DDP_DIAG_EPI >= 2 && c < C::NVAL_S) acc[c % NS] = fmaf(__uint_as_float(w[c16 & 1][q]), b[c / NS], acc[c % NS]);
+                            if (c < C::NVAL_S) acc[c % NS] = fmaf(__uint_as_float(w[c16 & 1][q]), b[c / NS], acc[c % NS]);
                         }
                     }
                     tc_fence_before();
@@ -1101,7 +968,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
 #pragma unroll
                     for (int rr = 0; rr < C::ROWS_V; ++rr) xn[rr] = rr < n_rows ? xn[rr] : 0.f;     // padding columns are zero, their x is not
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 0);
-                    DDP_WAIT(&tmem_full[wg], tf_phase, 10, it, tt);
+                    mbar_wait_relaxed<0>(&tmem_full[wg], tf_phase);
                     tf_phase ^= 1u;
                     tc_fence_after();
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 1);
@@ -1117,7 +984,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
 #pragma unroll
                             for (int q = 0; q < 16; ++q) {
                                 const int c = c16 * 16 + q;
-                                if (DDP_DIAG_EPI >= 2 && c < NCOLS) u[c % NV] = fmaf(__uint_as_float(w[c16 & 1][q]), xn[c / NV], u[c % NV]);
+                                if (c < NCOLS) u[c % NV] = fmaf(__uint_as_float(w[c16 & 1][q]), xn[c / NV], u[c % NV]);
                             }
                         }
                     }
@@ -1179,7 +1046,7 @@ tpconv_umma_kernel(const __grid_constant__ Jobs jobs) {
                     // the basis rows are in registers: fetch the next own tile's node features
                     if (own_next) x_prefetch_tile<NS, NV, C::ROWS_S, C::XN>(xg, tdn, f_in, xn);
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 0);
-                    DDP_WAIT(&tmem_full[wg], tf_phase, 10, it, tt);
+                    mbar_wait_relaxed<0>(&tmem_full[wg], tf_phase);
                     tf_phase ^= 1u;
                     tc_fence_after();
                     if (tracer) trace_ev(jobs.trace, 1 + wg, titer, 1);
@@ -1271,8 +1138,7 @@ static int build_plan(const ddp_tpconv_t &c, const ddp_tp_group_t *groups, const
     if (nv == 0) nv = (ns == 60) ? 10 : (ns == 24 ? 6 : 4);
     if (!pick_cfg(ns, nv, ks)) return DDP_E_UNSUPPORTED;
     if (c.k1 != 3 * ns || c.hid != 3 * ns || c.n_emb != ns || (c.sh_dim != 4 && c.sh_dim != 9)) return DDP_E_UNSUPPORTED;
-    const bool ts = use_ts(mode != 0);
-    const int rows_s = rows_scalar(ns, ts), rows_v = rows_vector(nv);
+    const int rows_s = rows_scalar(ns), rows_v = rows_vector(nv);
     Header &h = P.h;
     memset(&h, 0, sizeof(h));
     h.magic = MAGIC; h.mode = mode; h.ns = ns; h.nv = nv; h.ks = ks; h.kp = 3 * ks; h.n1 = 3 * ks;
@@ -1306,7 +1172,7 @@ static int build_plan(const ddp_tpconv_t &c, const ddp_tp_group_t *groups, const
                 const int nr = std::min(per, groups[q].mul_in - r0);
                 TileDesc td;
                 memset(&td, 0, sizeof(td));
-                td.n_cols = (uint16_t)(vec ? ncol_vector(nv, nr) : ncol_scalar(ns, ts));
+                td.n_cols = (uint16_t)(vec ? ncol_vector(nv, nr) : ncol_scalar(ns));
                 td.kind = (uint8_t)kind;
                 td.ctab5 = (uint8_t)table5;
                 td.n_rows = (uint8_t)nr;
@@ -1476,7 +1342,7 @@ static long long *g_umma_trace = nullptr;
 extern "C" int ddp_tpconv_umma_set_trace(void *trace_dev) {
 #ifdef DDP_UMMA_TRACE
     g_umma_trace = static_cast<long long *>(trace_dev);
-    return 3 * umma::TRACE_TILES * umma::TRACE_EVENTS;      // int64 slots the buffer must hold (watchdog build: 148 x 12 x 4 of them)
+    return 3 * umma::TRACE_TILES * umma::TRACE_EVENTS;      // int64 slots the buffer must hold
 #else
     (void)trace_dev;
     return DDP_E_UNSUPPORTED;                               // library built without -DDDP_UMMA_TRACE

@@ -78,10 +78,6 @@ int ddp_radius(const float *x, const float *y, const int32_t *ptr_x, const int32
 int ddp_knn_graph(const float *x, const int32_t *ptr, int32_t num_examples, int32_t n, int32_t k,
                   int32_t *slab, int32_t slab_w, int32_t *counts, int32_t *edge, int32_t edge_cap,
                   int32_t *n_edges_dev, void *stream);
-/* Search strategy of the filtered k-NN (k = 8 / 12): 0 = ordered scan of the staged example (default), 1 = grid-binned
- * (cell list built per block in shared memory; same edge lists, measured slower at pocket sizes -- see csrc/graph.cu).
- * Returns the previous setting (-1: not set yet, DDP_KNN_GRID in the environment decides on first use). */
-int ddp_knn_set_grid(int32_t mode);
 
 /* ddp_calpha_graph: the receptor's residue contact graph, built once per complex by the reference's preprocessing
  * (datasets/process_mols.py:661-677): for every residue i of its complex the residues closer than r, in index order;

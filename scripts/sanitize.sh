@@ -1,16 +1,10 @@
 #!/bin/bash
-# compute-sanitizer passes over the tensor-core conv kernel (run on the GPU box: gpurun -- 'bash scripts/sanitize.sh').
-#   stage 1: the production library under memcheck / synccheck / racecheck / initcheck on the grouped-launch operator test
-#            and a full forward of the big model through the tensor-core path;
-#   stage 2: the same with a library built without the issue-order token (-DDDP_UMMA_TOKEN=0, scripts/micro/libddp_token0.so,
-#            built here with `bash scripts/sanitize.sh build`), first plain (does it fail at all?), then under the tools.
+# compute-sanitizer passes over the tensor-core conv kernel (run on a machine with a B200: bash scripts/sanitize.sh):
+# the production library under memcheck / synccheck / racecheck on the grouped-launch operator test and a full forward
+# of the big model through the tensor-core path.
 # Logs: gpurun_out/sanitize/*.log (summaries are copied to profiles/ by hand).
 set -u
 cd "$(dirname "$0")/.."
-if [ "${1:-}" = "build" ]; then
-  DDP_NVCC_FLAGS="-DDDP_UMMA_TOKEN=0" DDP_LIB=$PWD/scripts/micro/libddp_token0.so python -c "from diffdock_pocket_b200 import _lib; _lib.build(verbose=True)"
-  exit $?
-fi
 OUT=gpurun_out/sanitize
 mkdir -p $OUT
 T1="tests/test_gpu_umma.py::test_grouped_launch_equals_single_launches"
@@ -27,13 +21,4 @@ for tool in memcheck synccheck racecheck; do
   run ${tool}_token1_grouped compute-sanitizer --tool $tool --print-limit 20 --log-file $OUT/${tool}_token1_grouped.log python -m pytest -x -q "$T1"
 done
 run synccheck_token1_forward compute-sanitizer --tool synccheck --print-limit 20 --log-file $OUT/synccheck_token1_forward.log python -m pytest -x -q "$T2"
-if [ -f scripts/micro/libddp_token0.so ]; then
-  export DDP_LIB=$PWD/scripts/micro/libddp_token0.so
-  for i in 1 2 3; do run plain_token0_grouped_$i python -m pytest -x -q "$T1"; done
-  run plain_token0_forward python -m pytest -x -q "$T2" tests/test_gpu_parity.py::test_forward_batch64_equals_sub_batches
-  for tool in memcheck synccheck racecheck; do
-    run ${tool}_token0_grouped compute-sanitizer --tool $tool --print-limit 20 --log-file $OUT/${tool}_token0_grouped.log python -m pytest -x -q "$T1"
-  done
-  run synccheck_token0_forward compute-sanitizer --tool synccheck --print-limit 20 --log-file $OUT/synccheck_token0_forward.log python -m pytest -x -q "$T2"
-fi
 for f in $OUT/*.log; do echo "--- $f"; grep -E "ERROR SUMMARY|RACECHECK SUMMARY|Error|hazard" "$f" | sort | uniq -c | head -20; done | tee -a $OUT/summary.txt

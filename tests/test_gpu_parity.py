@@ -562,27 +562,19 @@ def test_conv_layer_backward_vs_autograd_of_the_oracle(case, mode):
     assert T.rel_err(got2, want2) < 1e-4
 
 
-def test_grid_binned_knn_graph_bit_exact_on_pockets_and_edge_cases():
-    """The atom graph (k = 8 and k = 12) through the grid-binned search: protein-pocket-like clouds (dense ball + sparse surface
+def test_filtered_knn_graph_bit_exact_on_pockets_and_edge_cases():
+    """The atom graph (k = 8 and k = 12) through the filtered search: protein-pocket-like clouds (dense ball + sparse surface
     atoms that need the wider retry radii), an example larger than one shared-memory stage (plain-scan fallback inside the kernel),
-    examples smaller than k + 1, coincident points, points far apart (one point per cell) -- identical edge lists, order included."""
+    examples smaller than k + 1, coincident points, points far apart -- identical edge lists, order included."""
     g = torch.Generator().manual_seed(7)
     parts = [torch.randn(1100, 3, generator=g) * 9.0,                                  # pocket-sized dense cloud
              torch.cat([torch.randn(600, 3, generator=g) * 6.0, torch.randn(40, 3, generator=g) * 40.0]),   # core + far outliers
              torch.randn(2500, 3, generator=g) * 12.0,                                  # > kKnnStage points
              torch.randn(5, 3, generator=g), torch.randn(1, 3, generator=g),            # fewer than k + 1 points
-             torch.rand(200, 3, generator=g) * 400.0,                                   # extent >> 12 cells of 5.5 A
+             torch.rand(200, 3, generator=g) * 400.0,                                   # wide extent: few neighbours within the radii
              torch.zeros(30, 3) + 2.5]                                                  # all coincident
     parts[0][100:120] = parts[0][100]
     x = torch.cat(parts)
     b = torch.cat([torch.full((p.shape[0],), i, dtype=torch.long) for i, p in enumerate(parts)])
-    from diffdock_pocket_b200 import _lib
-    L = _lib.lib()
-    prev = L.ddp_knn_set_grid(1)
-    try:
-        for grid in (1, 0):
-            L.ddp_knn_set_grid(grid)
-            for k in (8, 12):
-                assert torch.equal(ops.knn_graph(x.to(DEV), k, b.to(DEV)).cpu(), cluster.knn_graph(x, k, b)), (grid, k)
-    finally:
-        L.ddp_knn_set_grid(max(prev, 0))
+    for k in (8, 12):
+        assert torch.equal(ops.knn_graph(x.to(DEV), k, b.to(DEV)).cpu(), cluster.knn_graph(x, k, b)), k
