@@ -92,6 +92,9 @@ _SIGS = {
     'ddp_node_update': (i32, [vp, i32, i32, C.POINTER(Update), i32, i32, i32, vp, i32, vp]),
     'ddp_node_update_multi': (i32, [C.POINTER(NodeUpdateJob), i32, vp]),
     'ddp_degree_multi': (i32, [C.POINTER(DegreeJob), i32, vp]),
+    'ddp_mark_bond_nodes': (i32, [vp, vp, i32, i32, vp, i32, vp, f32, vp, vp]),
+    'ddp_mark_gathered': (i32, [vp, vp, vp, i32, vp, vp, vp]),
+    'ddp_live_edges': (i32, [vp, i32, vp, i32, vp, i32, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp]),
     'ddp_segment_mean': (i32, [vp, vp, vp, i32, i32, i32, vp, i32, vp]),
     'ddp_bond_geometry': (i32, [vp, vp, i32, vp, i32, i32, vp, vp, vp, vp]),
     'ddp_tor_edge_sh': (i32, [vp, i32, vp, vp, vp, vp, i32, vp, vp]),
@@ -113,7 +116,7 @@ _SIGS = {
 EXPORTS = sorted(_SIGS)
 _LIB = None
 # kernels launched per C-ABI call (for the bench's gpu_launches claim)
-KERNELS_PER_CALL = {'ddp_radius': 3, 'ddp_knn_graph': 3, 'ddp_calpha_graph': 3, 'ddp_version': 0, 'ddp_pose_max_ligand_atoms': 0, 'ddp_tpconv_pack': 0, 'ddp_tpconv_umma_set_trace': 0}
+KERNELS_PER_CALL = {'ddp_radius': 3, 'ddp_knn_graph': 3, 'ddp_calpha_graph': 3, 'ddp_live_edges': 3,'ddp_version': 0, 'ddp_pose_max_ligand_atoms': 0, 'ddp_tpconv_pack': 0, 'ddp_tpconv_umma_set_trace': 0}
 COUNTS = {}
 
 

@@ -58,6 +58,14 @@ class _EdgeSet:
         self.edge[self.cap:self.cap + n] = ei[1].to(torch.int32)
         self.n_dev.fill_(n)
 
+    def live_copy(self, ns, sh_dim, device):
+        """Buffer of the same capacity for the edges of this set whose aggregation node is live (``ddp_live_edges``).  It
+        shares the in-degrees of the full set: a live node keeps all of its edges, so its mean keeps its normaliser."""
+        c = _EdgeSet(self.cap, ns, sh_dim, device)
+        c.deg = self.deg
+        c.counts = torch.zeros((self.cap + 255) // 256 + 1, dtype=torch.int32, device=device)
+        return c
+
     def edge_index(self):
         """Host-synchronising view [2, E] int64 (tests / drop-in side effects only)."""
         n = int(self.n_dev.item())
@@ -347,6 +355,10 @@ class TensorProductScoreModel(nn.Module):
 
     # ------------------------------------------------------------------------------------------ plan
     STATIC_CACHE_SIZE = 256
+    # Plans built while this is set run the atom-aggregating convs of the last two interaction layers on the edges into
+    # atoms whose features are read afterwards only (_live_edges); the outputs that are read are the same.  Off: A/B runs.
+    prune_edges = True
+    LIVE_RADIUS_MARGIN = 0.01      # Å added to the torsion head's radius: the live set may be larger, never smaller
 
     def static_for(self, graph):
         """Time-independent node embeddings of ONE complex (``ddp_node_static_embed``: AtomEncoder sums + the part of its
@@ -540,10 +552,22 @@ class TensorProductScoreModel(nn.Module):
             if self.flexible_sidechains and S > 0:
                 fr = data['flexResidues']
                 frb = fr.batch.cpu() if 'batch' in fr else torch.zeros(S, dtype=torch.long)
-                fa = (ap[:-1][frb] + fr.edge_idx.T.long().cpu()).unique()
+                bonds = ap[:-1][frb] + fr.edge_idx.T.long().cpu()
+                fa = bonds.unique()
                 fcnt = torch.bincount(ab[fa], minlength=B)
                 pl.flex_atoms = fa.to(**i32)
                 pl.flex_ptr = torch.cat([torch.zeros(1, dtype=torch.long), fcnt.cumsum(0)]).to(**i32)
+                bcnt = torch.bincount(frb, minlength=B)
+                pl.live_bonds = (bonds.to(**i32).contiguous(), torch.cat([torch.zeros(1, dtype=torch.long), bcnt.cumsum(0)]).to(**i32), 0.0)
+        # live atoms and pruned atom-aggregating edge sets of the last two interaction layers (_live_edges)
+        nl = self.num_conv_layers
+        pl.prune_layers = [l for l in (nl - 2, nl - 1) if l >= 0 and (self.flexible_sidechains or l < nl - 1)] if self.prune_edges else []
+        pl.prune = bool(pl.prune_layers)
+        if pl.prune:
+            if not hasattr(pl, 'live_bonds'):
+                pl.live_bonds = (pl.sc.bonds, pl.sc.ptr, self.lig_max_radius + self.LIVE_RADIUS_MARGIN) if S > 0 and not self.confidence_mode else None
+            pl.live = torch.zeros(2, pl.NA, dtype=torch.uint8, device=dev)
+            pl.pruned = {(l, nm): es[nm].live_copy(ns, sh_dim, dev) for l in pl.prune_layers for nm in ('aa', 'ar')}
         return pl
 
     def _bond_head_plan(self, bonds, bond_batch, B, n_nodes, max_seg, dev, det=False):
@@ -672,7 +696,7 @@ class TensorProductScoreModel(nn.Module):
         capture tensors, never the plan itself: a plan -> record -> plan cycle would keep freed plans away from the caching
         allocator until the cyclic GC runs, and every new plan would pay cudaMalloc.)"""
         key = (self.conv_mode, torch.cuda.current_stream().cuda_stream, getattr(self, 'group_convs', True), id(self.packed()),
-               pl.deterministic)
+               pl.deterministic, pl.prune)
         debug = return_layers or getattr(self, 'profile', None) is not None or getattr(self, 'profile_small', None) is not None or not self.replay_launches
         prog = getattr(pl, 'program', None)
         if prog is not None and prog[0] == key and not debug:
@@ -720,6 +744,27 @@ class TensorProductScoreModel(nn.Module):
         fn()
         if _lib.RECORD is not None:
             _lib.RECORD.append((None, fn, torch.cuda.current_stream()))
+
+    def _live_edges(self, pl, L, st):
+        """Live atoms and the pruned edge sets of ``pl.prune_layers``, on stream ``st``.  live[0]: the atoms whose
+        last-layer features are read -- the side-chain torsion head's bond endpoints and every atom closer than
+        lig_max_radius (+ margin) to a bond midpoint (its radius graph takes the first 32 of those), or the confidence
+        model's flexible-bond atoms.  live[1]: the atoms whose layer L-2 features the last layer reads -- live[0] (the
+        residual), the k-NN neighbours its atom-atom conv gathers into live[0] and every atom of a ligand-atom edge (the
+        ligand-side conv gathers them).  Receptor features are not pruned: at t = 1 every ligand-residue pair is an edge."""
+        es, live, chk = pl.es, pl.live, _lib.check
+        bonds, bptr, r = pl.live_bonds if pl.live_bonds is not None else (None, None, 0.0)
+        chk(L.ddp_mark_bond_nodes(ptr(pl.atom_pos), ptr(pl.atom_ptr), pl.B, pl.NA, ptr(bonds), 0 if bonds is None else bonds.shape[1],
+                                  ptr(bptr), float(r), ptr(live[0]), st), 'ddp_mark_bond_nodes')
+        self._py(lambda a=live[1], b=live[0]: a.copy_(b))
+        aa, la = es['aa'], es['la']
+        chk(L.ddp_mark_gathered(aa.row(0), aa.row(1), ptr(aa.n_dev), aa.cap, ptr(live[0]), ptr(live[1]), st), 'ddp_mark_gathered(aa)')
+        chk(L.ddp_mark_gathered(None, la.row(1), ptr(la.n_dev), la.cap, None, ptr(live[1]), st), 'ddp_mark_gathered(la)')
+        for (l, nm), p in pl.pruned.items():
+            e = es[nm]
+            chk(L.ddp_live_edges(ptr(e.edge), e.cap, ptr(e.n_dev), 0, ptr(e.sh), self.sh_dim, ptr(e.emb), self.ns,
+                                 ptr(live[self.num_conv_layers - 1 - l]), ptr(p.counts), ptr(p.edge), p.cap, ptr(p.n_dev), ptr(p.sh),
+                                 ptr(p.emb), st), f'ddp_live_edges({nm})')
 
     def _launch_plan_body(self, pl, return_layers=False):
         P = self.packed()
@@ -792,6 +837,12 @@ class TensorProductScoreModel(nn.Module):
         self._py(lambda: br.join(main, 3))
         self._py(lambda a=pl.deg_arena, b=pl.deg_base: a.copy_(b))   # static edge sets + ligand bond edges
         chk(L.ddp_degree_multi(pl.deg_jobs, len(pl.deg_jobs), st), 'ddp_degree_multi')   # dynamic ones, one launch
+        # per-layer outputs of every node are returned unpruned
+        prune = pl.prune and not return_layers
+        if prune:
+            self._py(lambda: br.fork(1))                                 # joined before the first pruned layer
+            with torch.cuda.stream(br.side[0]):
+                self._live_edges(pl, L, _lib.stream_ptr())
         # ---- interaction layers (all_atom_score_model.py:271-324) --------------------------------
         layers_out = []
         seq_dims = [tpmod.irreps_dim(tpmod.parse_irreps(s)) for s in self.irrep_seq]
@@ -812,8 +863,10 @@ class TensorProductScoreModel(nn.Module):
             # BatchNorm scale, all_atom_score_model.py:315-324 + score_model.py:117,123) straight into it.
             def job(ci, nm, flip, x, p1, i1, p2, i2, buf):
                 agg_r = 1 if flip else 0
+                # atom-aggregating aa / ar convs of a pruned layer: the edges into live atoms; degrees of the full set
+                e_ = pl.pruned[(l, nm)] if prune and not flip and (l, nm) in pl.pruned else es[nm]
                 # BatchNorm scale lives in the packed weights (PackedConv fold_bn); without BatchNorm out_scale stays NULL
-                return (Cv[ci], Pk[ci], es[nm], flip, x, p1, i1, p2, i2, buf, None, es[nm].deg[agg_r])
+                return (Cv[ci], Pk[ci], e_, flip, x, p1, i1, p2, i2, buf, None, es[nm].deg[agg_r])
             s_l = take(pl.NL)
             grp = [job(9 * l, 'll', False, xl, xl, 0, xl, 1, s_l), job(9 * l + 1, 'lr', False, xr, xl, 0, xr, 1, s_l),
                    job(9 * l + 2, 'la', False, xa, xl, 0, xa, 1, s_l)]
@@ -828,6 +881,8 @@ class TensorProductScoreModel(nn.Module):
                             job(9 * l + 8, 'ar', True, xa, xr, 1, xa, 0, s_r)]
             # largest edge sets first: the round-robin tile walk then ends on the small ones
             grp.sort(key=lambda it: -it[2].cap)
+            if prune and l == pl.prune_layers[0]:
+                self._py(lambda: br.join(main, 1))
             self._conv_group(L, st, grp, pl.status)
 
             def update(key, x_old, n, buf, items):

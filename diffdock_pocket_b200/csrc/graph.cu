@@ -381,6 +381,89 @@ __global__ void degree_kernel(const int32_t *__restrict__ idx, const int32_t *__
     for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) atomicAdd(&deg[idx[e]], 1);
 }
 
+// live[i] = 1 if node i is an endpoint of one of its example's bonds or (r2 > 0) lies closer than sqrt(r2) to the midpoint
+// of one, else 0 (every entry is written).  The midpoint is formed as in bond_geometry_kernel (embed.cu).
+__global__ void mark_bond_nodes_kernel(const float *__restrict__ pos, const int32_t *__restrict__ node_ptr, int num_examples, int n,
+                                       const int32_t *__restrict__ bonds, int n_bonds, const int32_t *__restrict__ bond_ptr,
+                                       float r2, uint8_t *__restrict__ live) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint8_t hit = 0;
+    if (n_bonds > 0) {
+        const int b = ddp_find_segment(node_ptr, num_examples, i);
+        const float px = pos[3 * i], py = pos[3 * i + 1], pz = pos[3 * i + 2];
+        for (int k = bond_ptr[b]; k < bond_ptr[b + 1] && !hit; ++k) {
+            const int u = bonds[k], v = bonds[n_bonds + k];
+            hit = u == i || v == i;
+            if (!hit && r2 > 0.f)
+                hit = ddp_sqdist(px, py, pz, (pos[3 * u] + pos[3 * v]) / 2.f, (pos[3 * u + 1] + pos[3 * v + 1]) / 2.f,
+                                 (pos[3 * u + 2] + pos[3 * v + 2]) / 2.f) < r2;
+        }
+    }
+    live[i] = hit;
+}
+
+// live_out[gather[e]] = 1 for every live edge e whose aggregation node is live in live_in (every edge: live_in == NULL)
+__global__ void mark_gathered_kernel(const int32_t *__restrict__ agg, const int32_t *__restrict__ gather,
+                                     const int32_t *__restrict__ n_edges, int edge_cap, const uint8_t *__restrict__ live_in,
+                                     uint8_t *__restrict__ live_out) {
+    const int n = min(*n_edges, edge_cap);
+    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x)
+        if (live_in == nullptr || live_in[agg[e]]) live_out[gather[e]] = 1;
+}
+
+// Stable compaction of the edges whose aggregation node is live: count per block of kCompactBlock edges, exclusive scan of
+// the counts (scan_counts_kernel), then every block writes its live edges in order from its offset.
+constexpr int kCompactBlock = 256;
+__device__ __forceinline__ bool edge_is_live(const int32_t *__restrict__ agg, const int32_t *__restrict__ n_edges, int edge_cap,
+                                             const uint8_t *__restrict__ live, int e) {
+    return e < min(*n_edges, edge_cap) && live[agg[e]];
+}
+
+__global__ void __launch_bounds__(kCompactBlock) live_count_kernel(const int32_t *__restrict__ agg, const int32_t *__restrict__ n_edges,
+                                                                   int edge_cap, const uint8_t *__restrict__ live, int32_t *__restrict__ counts) {
+    const int c = __syncthreads_count(edge_is_live(agg, n_edges, edge_cap, live, blockIdx.x * kCompactBlock + threadIdx.x));
+    if (threadIdx.x == 0) counts[blockIdx.x] = c;
+}
+
+__global__ void __launch_bounds__(kCompactBlock) live_scatter_kernel(
+        const int32_t *__restrict__ edge, int edge_cap, const int32_t *__restrict__ n_edges, int agg_row,
+        const float *__restrict__ sh, int sh_dim, const float *__restrict__ emb, int ns, const uint8_t *__restrict__ live,
+        const int32_t *__restrict__ offs, int32_t *__restrict__ edge_out, int edge_cap_out, float *__restrict__ sh_out,
+        float *__restrict__ emb_out) {
+    __shared__ int warp_off[kCompactBlock / 32];
+    __shared__ int src[kCompactBlock];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int e = blockIdx.x * kCompactBlock + threadIdx.x;
+    const bool keep = edge_is_live(edge + (size_t)agg_row * edge_cap, n_edges, edge_cap, live, e);
+    const unsigned m = __ballot_sync(0xffffffffu, keep);
+    if (lane == 0) warp_off[wid] = __popc(m);
+    __syncthreads();
+    int before = 0, total = 0;
+#pragma unroll
+    for (int w = 0; w < kCompactBlock / 32; ++w) {
+        before += w < wid ? warp_off[w] : 0;
+        total += warp_off[w];
+    }
+    const int local = before + __popc(m & ((1u << lane) - 1u));
+    const int base = offs[blockIdx.x];
+    if (keep) {
+        src[local] = e;
+        edge_out[base + local] = edge[e];
+        edge_out[edge_cap_out + base + local] = edge[edge_cap + e];
+    }
+    __syncthreads();
+    // rows of the kept edges, copied by the whole block (consecutive threads -> consecutive floats)
+    for (int t = threadIdx.x; t < total * sh_dim; t += kCompactBlock) {
+        const int k = t / sh_dim, c = t - k * sh_dim;
+        sh_out[(size_t)(base + k) * sh_dim + c] = sh[(size_t)src[k] * sh_dim + c];
+    }
+    for (int t = threadIdx.x; t < total * ns; t += kCompactBlock) {
+        const int k = t / ns, c = t - k * ns;
+        emb_out[(size_t)(base + k) * ns + c] = emb[(size_t)src[k] * ns + c];
+    }
+}
+
 constexpr int kMaxDegJobs = 12;
 struct DegPack { ddp_degree_job_t j[kMaxDegJobs]; };
 __global__ void degree_multi_kernel(DegPack p) {
@@ -493,6 +576,50 @@ extern "C" int ddp_degree_multi(const ddp_degree_job_t *jobs_host, int32_t n_job
     int gx = (cap + 255) / 256;
     if (gx > 2 * ddp_num_sms()) gx = 2 * ddp_num_sms();
     degree_multi_kernel<<<dim3(gx, n_jobs), 256, 0, (cudaStream_t)stream>>>(p);
+    DDP_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int ddp_mark_bond_nodes(const float *pos, const int32_t *node_ptr, int32_t num_examples, int32_t n,
+                                   const int32_t *bonds, int32_t n_bonds, const int32_t *bond_ptr, float r, uint8_t *live,
+                                   void *stream) {
+    if (!pos || !node_ptr || !live || (n_bonds > 0 && (!bonds || !bond_ptr))) return DDP_E_ARG;
+    if (num_examples <= 0 || n < 0 || n_bonds < 0) return DDP_E_SHAPE;
+    if (n == 0) return 0;
+    const float r2 = r > 0.f ? (float)((double)r * (double)r) : 0.f;
+    mark_bond_nodes_kernel<<<(n + 255) / 256, 256, 0, (cudaStream_t)stream>>>(pos, node_ptr, num_examples, n, bonds, n_bonds,
+                                                                              bond_ptr, r2, live);
+    DDP_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int ddp_mark_gathered(const int32_t *agg, const int32_t *gather, const int32_t *n_edges_dev, int32_t edge_cap,
+                                 const uint8_t *live_in, uint8_t *live_out, void *stream) {
+    if (!gather || !n_edges_dev || !live_out || (live_in && !agg)) return DDP_E_ARG;
+    if (edge_cap <= 0) return 0;
+    int grid = (edge_cap + 255) / 256;
+    if (grid > 4 * ddp_num_sms()) grid = 4 * ddp_num_sms();
+    mark_gathered_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(agg, gather, n_edges_dev, edge_cap, live_in, live_out);
+    DDP_LAUNCH_CHECK();
+    return 0;
+}
+
+extern "C" int ddp_live_edges(const int32_t *edge, int32_t edge_cap, const int32_t *n_edges_dev, int32_t agg_row,
+                              const float *sh, int32_t sh_dim, const float *emb, int32_t ns, const uint8_t *live,
+                              int32_t *counts, int32_t *edge_out, int32_t edge_cap_out, int32_t *n_edges_out_dev,
+                              float *sh_out, float *emb_out, void *stream) {
+    if (!edge || !n_edges_dev || !sh || !emb || !live || !counts || !edge_out || !n_edges_out_dev || !sh_out || !emb_out)
+        return DDP_E_ARG;
+    if (edge_cap <= 0 || edge_cap_out < edge_cap || (agg_row != 0 && agg_row != 1) || sh_dim <= 0 || ns <= 0) return DDP_E_SHAPE;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int blocks = (edge_cap + kCompactBlock - 1) / kCompactBlock;
+    const int32_t *agg = edge + (size_t)agg_row * edge_cap;
+    live_count_kernel<<<blocks, kCompactBlock, 0, st>>>(agg, n_edges_dev, edge_cap, live, counts);
+    DDP_LAUNCH_CHECK();
+    scan_counts_kernel<<<1, 1024, 0, st>>>(counts, blocks, 0, n_edges_out_dev);
+    DDP_LAUNCH_CHECK();
+    live_scatter_kernel<<<blocks, kCompactBlock, 0, st>>>(edge, edge_cap, n_edges_dev, agg_row, sh, sh_dim, emb, ns, live, counts,
+                                                          edge_out, edge_cap_out, sh_out, emb_out);
     DDP_LAUNCH_CHECK();
     return 0;
 }

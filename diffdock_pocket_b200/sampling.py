@@ -147,8 +147,10 @@ def _same_tables(a, b):
 def _cache_key(model, confidence_model, device, batch_size, flexible_sidechains, no_torsion, use_graph, concurrent_batches,
                deterministic, graph_keys):
     """Key of one resident-state entry: everything its plans, recorded launch programs and captured step graphs were
-    built for -- including the accumulation mode, so that state built in one mode is never replayed in the other."""
-    return (id(model), id(confidence_model), getattr(model, 'conv_mode', None), getattr(model, 'group_convs', None), str(device),
+    built for -- including the accumulation mode, so that state built in one mode is never replayed in the other, and
+    whether the plans prune dead edges (``prune_edges``)."""
+    return (id(model), id(confidence_model), getattr(model, 'conv_mode', None), getattr(model, 'group_convs', None),
+            getattr(model, 'prune_edges', None), getattr(confidence_model, 'prune_edges', None), str(device),
             batch_size, bool(flexible_sidechains), bool(no_torsion), bool(use_graph), bool(concurrent_batches), bool(deterministic),
             tuple(graph_keys))
 

@@ -96,6 +96,30 @@ int ddp_degree(const int32_t *idx, const int32_t *n_edges_dev, int32_t edge_cap,
 typedef struct { const int32_t *idx; const int32_t *n_edges_dev; int32_t edge_cap; int32_t start; int32_t *deg; } ddp_degree_job_t;
 int ddp_degree_multi(const ddp_degree_job_t *jobs_host, int32_t n_jobs, void *stream);
 
+/* Live nodes and pruned edge sets.  The atom features of the last interaction layer (models/all_atom_score_model.py:271-324)
+ * are read only by the side-chain torsion head (bond endpoints, and the atoms its radius graph gathers around each bond
+ * midpoint, :386-434) and by the confidence model's mean over the flexible-bond atoms (:329-353); those of the layer
+ * before only where the last layer gathers them (its atom-atom convs and the ligand-side conv of the ligand-atom
+ * edges).  The atom-aggregating convs of those two layers run on the edges into live atoms only; the results that are
+ * read do not change.  Masks are uint8 [n] (0 / 1).
+ *
+ * ddp_mark_bond_nodes: live[i] = 1 if node i (example b from node_ptr) is an endpoint of a bond of example b, or, with
+ *   r > 0, lies closer than r to the midpoint (a + b) / 2 of one; else 0 -- every entry is written.  bonds: int32 [2, n_bonds]
+ *   grouped by example, bond_ptr [num_examples + 1] (may be NULL when n_bonds = 0).
+ * ddp_mark_gathered: live_out[gather[e]] = 1 for e < min(*n_edges_dev, edge_cap) when live_in[agg[e]] is set, or for every
+ *   edge when live_in is NULL.  Entries are only ever set: the caller initialises live_out.
+ * ddp_live_edges: stable compaction of the edges e < min(*n_edges_dev, edge_cap) whose aggregation node edge[agg_row][e]
+ *   is live: index pair, sh row (sh_dim floats) and emb row (ns floats) are copied in order to edge_out / sh_out / emb_out
+ *   (capacity edge_cap_out >= edge_cap, same row layout as the input: row r at edge_out + r * edge_cap_out) and the
+ *   number kept is written to *n_edges_out_dev.  counts: workspace int32 [ceil(edge_cap / 256) + 1]. */
+int ddp_mark_bond_nodes(const float *pos, const int32_t *node_ptr, int32_t num_examples, int32_t n, const int32_t *bonds,
+                        int32_t n_bonds, const int32_t *bond_ptr, float r, uint8_t *live, void *stream);
+int ddp_mark_gathered(const int32_t *agg, const int32_t *gather, const int32_t *n_edges_dev, int32_t edge_cap,
+                      const uint8_t *live_in, uint8_t *live_out, void *stream);
+int ddp_live_edges(const int32_t *edge, int32_t edge_cap, const int32_t *n_edges_dev, int32_t agg_row, const float *sh,
+                   int32_t sh_dim, const float *emb, int32_t ns, const uint8_t *live, int32_t *counts, int32_t *edge_out,
+                   int32_t edge_cap_out, int32_t *n_edges_out_dev, float *sh_out, float *emb_out, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Edge geometry + edge embedding.  Replaces the per-edge-set blocks of build_*_conv_graph
  * (all_atom_score_model.py:476-481, 501-508, 527-534, 552-556, 566-570, 575-579, 594-598, 609-613):
