@@ -49,7 +49,7 @@ struct TileDesc {
                           // 5 (sh_lmax = 2 only) C(1,2,1)(xv, s2): the l = 2 harmonics as a 3 x 3 matrix applied to xv
     uint8_t n_rows;       // basis rows covered
     uint16_t out_off;     // first output feature of the block
-    uint8_t flags;        // bit 0: first tile of its block; bit 1: swap the last input irrep into slot 0 first; bit 2: last tile
+    uint8_t flags;        // bit 0: first tile of its block; bit 1: reserved (never set, not read); bit 2: last tile
     uint8_t ctab5;        // kind 5: which 45-float coupling table of the image (Header::ctab5_off)
     uint16_t x_off;       // slot of the first input feature of row 0 (row rr reads x_off + rr * (kind 0/2 ? 1 : 3))
     uint16_t pad1;

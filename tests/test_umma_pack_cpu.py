@@ -1,109 +1,64 @@
 """CPU check of the tensor-core weight image (ddp_tpconv_pack): decode the UMMA core-matrix slabs and the tile
-table in numpy, replay the kernel's data flow (A operand with bias slot -> GEMM1 -> ReLU -> per-tile GEMM2 ->
-basis contraction) and compare with the oracle conv.  Validates layout, tile schedule, folded biases and folded
-path normalisation without a GPU; the kernel itself is covered by the -m gpu tests."""
-import ctypes as C
-import struct
-
+table (tests/_umma_image.py), replay the kernel's data flow (A operand with bias slot -> GEMM1 -> ReLU -> per-tile GEMM2 ->
+basis contraction, kind-5 coupling tables for sh_lmax = 2) and compare with the oracle conv.  Validates layout, tile
+schedule, folded biases and folded path normalisation without a GPU; the kernel itself is covered by the -m gpu tests
+(tests/test_gpu_umma_replay.py replays the same decoded image against it)."""
 import numpy as np
 import pytest
 import torch
 
-from diffdock_pocket_b200 import _lib, tp
+import _umma_image as U
 from diffdock_pocket_b200.score_model import TensorProductConvLayer
 from oracle import e3nn_mini as E
 from oracle.score_model_ref import TensorProductConvLayer as RefConv
 
 
-def _bf16_to_f32(u16):
-    return (u16.astype(np.uint32) << 16).view(np.float32)
-
-
-def _decode_operand(buf, off, n_cols, kp, stage_k, mode):
-    """-> ([n_cols, kp] hi (+ lo) as float32, new offset)"""
-    W = np.zeros((n_cols, kp), dtype=np.float32)
-    for ks in range(kp // stage_k):
-        n_el = n_cols * stage_k
-        hi = _bf16_to_f32(np.frombuffer(buf, dtype=np.uint16, count=n_el, offset=off))
-        part = hi.copy()
-        if mode:
-            part = part + _bf16_to_f32(np.frombuffer(buf, dtype=np.uint16, count=n_el, offset=off + 2 * n_el))
-        cm = part.reshape(stage_k // 8, n_cols // 8, 8, 8)                 # [k-chunk][row group][row][elem]
-        W[:, ks * stage_k:(ks + 1) * stage_k] = cm.transpose(1, 2, 0, 3).reshape(n_cols, stage_k)
-        off += 2 * n_el * (2 if mode else 1)
-    return W, off
-
-
-@pytest.mark.parametrize('ns,nv,layer', [(60, 10, 3), (60, 10, 0), (60, 10, 1), (60, 10, 2), (24, 6, 3), (16, 4, 3)])
-@pytest.mark.parametrize('mode', [0, 1])
-def test_packed_image_replays_conv(ns, nv, layer, mode):
+def _irreps(ns, nv, layer):
     seq = [f'{ns}x0e', f'{ns}x0e + {nv}x1o', f'{ns}x0e + {nv}x1o + {nv}x1e', f'{ns}x0e + {nv}x1o + {nv}x1e + {ns}x0o']
-    in_ir, out_ir = seq[min(layer, 3)], seq[min(layer + 1, 3)]
+    return seq[min(layer, 3)], seq[min(layer + 1, 3)]
+
+
+@pytest.mark.parametrize('ns,nv,layer,sh_lmax', [(60, 10, 3, 1), (60, 10, 0, 1), (60, 10, 1, 1), (60, 10, 2, 1), (24, 6, 3, 1),
+                                                 (16, 4, 3, 1), (16, 4, 3, 2), (16, 4, 1, 2)])
+@pytest.mark.parametrize('mode', [0, 1])
+def test_packed_image_replays_conv(ns, nv, layer, sh_lmax, mode):
+    in_ir, out_ir = _irreps(ns, nv, layer)
+    sh_ir = '1x0e+1x1o' if sh_lmax == 1 else '1x0e+1x1o+1x2e'
+    faster = sh_lmax == 1                   # sh_lmax = 2: e3nn FullyConnectedTensorProduct, kind-5 tiles
     torch.manual_seed(0)
-    prod = TensorProductConvLayer(in_ir, '1x0e+1x1o', out_ir, 3 * ns, residual=False, batch_norm=False, faster=True)
-    ref = RefConv(in_ir, '1x0e+1x1o', out_ir, 3 * ns, residual=False, batch_norm=False, faster=True)
+    prod = TensorProductConvLayer(in_ir, sh_ir, out_ir, 3 * ns, residual=False, batch_norm=False, faster=faster)
+    ref = RefConv(in_ir, sh_ir, out_ir, 3 * ns, residual=False, batch_norm=False, faster=faster)
     ref.load_state_dict(prod.state_dict())
     spec = prod.tp.spec
-    L = _lib.lib()
-    groups = (_lib.TpGroup * len(spec.groups))(*[_lib.TpGroup(**g) for g in spec.groups])
-    cdesc = _lib.TpConv(k1=3 * ns, hid=3 * ns, w_numel=spec.weight_numel, n_emb=ns, ns=ns, n_groups=len(spec.groups),
-                        f_in=spec.f_in, f_out=spec.f_out, sh_dim=4, ctab_len=len(spec.ctab))
-    ctab = torch.tensor(spec.ctab, dtype=torch.float32)
-    w1, b1 = prod.fc[0].weight.detach().contiguous(), prod.fc[0].bias.detach().contiguous()
-    w2, b2 = prod.fc[3].weight.detach().contiguous(), prod.fc[3].bias.detach().contiguous()
-    args = (C.byref(cdesc), groups, ctab.data_ptr(), w1.data_ptr(), b1.data_ptr(), w2.data_ptr(), b2.data_ptr(), mode)
-    size = L.ddp_tpconv_pack(*args, None)
-    assert size > 0
-    img = torch.zeros(size, dtype=torch.uint8)
-    assert L.ddp_tpconv_pack(*args, img.data_ptr()) == 0
-    buf = img.numpy().tobytes()
-    magic, md, ns_, nv_, ks, kp, n1, stage_k, n_tiles, _ = struct.unpack_from('<I9i', buf, 0)
-    assert magic == 0x44445055 and (md, ns_, nv_) == (mode, ns, nv) and kp == n1 == 3 * ks
-    tiles_off, slabs_off, total = struct.unpack_from('<3q', buf, 56)
-    assert total == size
-    # ---- replay ----------------------------------------------------------------------------------
+    size, buf = U.pack(spec, prod.fc[0].weight, prod.fc[0].bias, prod.fc[3].weight, prod.fc[3].bias, ns, mode)
+    assert buf is not None, size
+    img = U.Image(buf)
+    assert (img.mode, img.ns, img.nv, img.sh_dim) == (mode, ns, nv, 4 if sh_lmax == 1 else 9)
+    kinds = {td['kind'] for td in img.tiles}
+    assert (5 in kinds) == (sh_lmax == 2), kinds
+    # one accumulation per output block; zero padding columns
+    seen_first = set()
+    for td, hi, lo in zip(img.tiles, img.w2_hi, img.w2_lo):
+        if td['flags'] & 1:
+            assert td['out_off'] not in seen_first
+            seen_first.add(td['out_off'])
+        assert td['n_rows'] * img.mul(td['kind']) <= td['n_cols']
+        assert np.all(hi[td['n_rows'] * img.mul(td['kind']):] == 0) and np.all(lo[td['n_rows'] * img.mul(td['kind']):] == 0)
+    if mode == 0:
+        assert not img.w1_lo.any() and not any(lo.any() for lo in img.w2_lo)
+    # the hidden unit `hid` regenerates the constant one for GEMM2's bias row, every unit above it is zero
+    rp = U.Replay(img, 'cpu')
     n_e = 9
     g = torch.Generator().manual_seed(1)
     x = torch.randn(n_e, spec.f_in, generator=g)
     ea = torch.randn(n_e, 3 * ns, generator=g)
-    sh = E.spherical_harmonics('1x0e+1x1o', torch.randn(n_e, 3, generator=g))
-    A = np.zeros((n_e, kp), dtype=np.float32)
-    for s in range(3):
-        A[:, s * ks:s * ks + ns] = ea[:, s * ns:(s + 1) * ns].numpy()
-    A[:, ns] = 1.0
-    W1, off = _decode_operand(buf, slabs_off, n1, kp, stage_k, mode)
-    H = np.maximum(A.astype(np.float64) @ W1.astype(np.float64).T, 0)          # [n_e, n1]
-    assert np.allclose(H[:, 3 * ns], 1.0) and np.all(H[:, 3 * ns + 1:] == 0)
-    out = np.zeros((n_e, spec.f_out))
-    s0, s1 = sh[:, 0].numpy().astype(np.float64), sh[:, 1:].numpy().astype(np.float64)
-    xs = x.numpy().astype(np.float64)
-    seen_first = set()
-    for t in range(n_tiles):
-        n_cols, kind, n_rows, out_off, flags, _, x_off = struct.unpack_from('<HBBHBBH', buf, tiles_off + 16 * t)
-        assert not flags & 2
-        if flags & 1:
-            assert out_off not in seen_first                             # one accumulation per output block
-            seen_first.add(out_off)
-        W2, off = _decode_operand(buf, off, n_cols, kp, stage_k, mode)
-        w = H @ W2.astype(np.float64).T                                        # [n_e, n_cols]
-        mul = ns if kind < 2 else nv
-        assert n_cols % 16 == 0 and n_rows * mul <= n_cols
-        assert np.all(W2[n_rows * mul:] == 0)                            # zero padding columns
-        for rr in range(n_rows):
-            xo = x_off + rr * (1 if kind in (0, 2) else 3)
-            xv = xs[:, xo:xo + 3]
-            if kind == 0: b = xs[:, xo] * s0
-            elif kind == 1: b = (xv * s1).sum(-1)
-            elif kind == 2: b = xs[:, xo, None] * s1
-            elif kind == 3: b = xv * s0[:, None]
-            else: b = np.cross(xv, s1)
-            for o in range(mul):
-                if kind < 2:
-                    out[:, out_off + o] += w[:, rr * mul + o] * b
-                else:
-                    out[:, out_off + 3 * o:out_off + 3 * o + 3] += w[:, rr * mul + o, None] * b
-    assert off == total
+    sh = E.spherical_harmonics(sh_ir, torch.randn(n_e, 3, generator=g))
+    ident = torch.arange(n_e)
+    A = U.a_operand(img, ea[:, :ns], ea[:, ns:2 * ns], ident, ea[:, 2 * ns:], ident)
+    h_hi, h_lo = U.hidden(rp, A)
+    assert torch.all(h_hi[:, 3 * ns] == 1.0) and torch.all(h_lo[:, 3 * ns] == 0) and torch.all(h_hi[:, 3 * ns + 1:] == 0)
+    out = U.replay_edges(rp, A, x, sh).numpy()
     with torch.no_grad():
-        want = ref.tp(x, sh, ref.fc(ea)).numpy()
+        want = ref.tp(x.double(), sh.double(), ref.double().fc(ea.double())).numpy()
     err = np.abs(out - want).max() / np.abs(want).max()
     assert err < (2e-5 if mode else 2e-2), err
