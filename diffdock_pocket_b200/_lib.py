@@ -12,7 +12,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get('DDP_LIB', os.path.join(_HERE, 'libddp_b200.so'))     # DDP_LIB: A/B runs of two builds
 CSRC = os.path.join(_HERE, 'csrc')
-SOURCES = ['graph.cu', 'embed.cu', 'tpconv_fp32.cu', 'tpconv_umma.cu', 'tpconv_bwd.cu', 'pose.cu', 'capi.cu']
+SOURCES = ['graph.cu', 'embed.cu', 'tpconv_fp32.cu', 'tpconv_umma.cu', 'tpconv_bwd.cu', 'pose.cu', 'posecheck.cu', 'capi.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-shared']
 
@@ -73,6 +73,17 @@ class Pose(C.Structure):
                 ('sc_score', vp), ('tr_z', vp), ('rot_z', vp), ('tor_z', vp), ('sc_z', vp)]
 
 
+class ClashComplex(C.Structure):
+    _fields_ = [(k, i32) for k in ('lig_type_off', 'far_off', 'atom_off', 'moved_off', 'n_moved', 'excl_off', 'n_excl')]
+
+
+class ClashScreen(C.Structure):
+    _fields_ = [('n_poses', i32), ('max_lig_atoms', i32), ('max_atoms', i32), ('pose_complex', vp), ('lig_pos', vp),
+                ('lig_ptr', vp), ('atom_pos', vp), ('atom_ptr', vp), ('complexes', vp), ('lig_type', vp), ('atom_type', vp),
+                ('atom_owner', vp), ('moved', vp), ('excl', vp), ('far_mask', vp), ('radius', vp), ('ratio', f32),
+                ('count', vp), ('min_ratio', vp)]
+
+
 _SIGS = {
     'ddp_version': (C.c_char_p, []),
     'ddp_radius': (i32, [vp, vp, vp, vp, i32, i32, vp, f32, i32, i32, i32, vp, i32, vp, vp, i32, vp, vp]),
@@ -104,6 +115,8 @@ _SIGS = {
     'ddp_pose_update': (i32, [C.POINTER(Pose), C.POINTER(StepCoef), vp]),
     'ddp_pose_max_ligand_atoms': (i32, []),
     'ddp_pose_update_dev': (i32, [C.POINTER(Pose), vp, vp]),
+    'ddp_pose_rmsd': (i32, [vp, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
+    'ddp_clash_screen': (i32, [C.POINTER(ClashScreen), vp]),
     # deterministic mode (fixed-point accumulation, DDP_ACC_FIXED_SHIFT)
     'ddp_fixed_to_float': (i32, [vp, C.c_int64, vp, vp]),
     'ddp_tpconv_fp32_fixed': (i32, [C.POINTER(TpConv), C.POINTER(TpEdges), vp, vp, vp]),

@@ -24,6 +24,7 @@ import torch.distributed as dist
 
 from .diffusion_utils import get_t_schedule, t_to_sigma as t_to_sigma_compl
 from .parallel import shard_range
+from .posecheck import check_poses
 from .hetero import sample_copies
 from .sampling import randomize_position, sampling
 
@@ -43,9 +44,12 @@ def default_args(**over):
 
 def infer_single_complex(idx, protein_ligand_info_row, model, args, score_model_args, filtering_args=None,
                          filtering_model=None, filtering_model_args=None, filtering_complex_dict=None, t_schedule=None,
-                         tr_schedule=None, device=None, defer=False, writer=None, out_dir=None):
+                         tr_schedule=None, device=None, defer=False, writer=None, out_dir=None, pose_checks=False):
     """-> dict(name, ligand_pos [spc, N_l, 3], atom_pos [spc, N_a, 3], confidence [spc] or None), poses in the original
     frame and sorted by confidence (descending); ``None`` if the complex failed (the reference returns 0 and goes on).
+    ``pose_checks=True`` adds ``checks``: ``posecheck.check_poses`` of the ranked poses (clash counts and minimum ratios,
+    and ``rmsd`` / ``sc_rmsd`` against the row's ``ref_ligand_pos`` / ``ref_atom_pos``, original frame, when it has them;
+    see ``_pose_checks`` for how a failing check is reported without touching the poses).
     ``defer=True`` returns a zero-argument callable producing that result instead: all GPU work is enqueued, nothing has
     been waited for, so the caller can prepare the next complex meanwhile (``infer_multiple_complexes`` does)."""
     orig = protein_ligand_info_row['complex_graph']
@@ -88,9 +92,11 @@ def infer_single_complex(idx, protein_ligand_info_row, model, args, score_model_
             graphs, confidence = pending()
             res = _rank(orig, idx, graphs, confidence)              # inference.py:198-219
             _submit_write(writer, out_dir, protein_ligand_info_row, res, flex)
-            return res
         except Exception as e:
             return failed(e)
+        if pose_checks:
+            _pose_checks([(protein_ligand_info_row, res)])
+        return res
     return finish if defer else finish()
 
 
@@ -103,6 +109,33 @@ def _submit_write(writer, out_dir, row, res, flex):
     fr = g['flexResidues'] if flex and 'flexResidues' in g and 'edge_idx' in g['flexResidues'] else None
     writer.submit(os.path.join(out_dir or '.', str(res['name'])), res, row['ligand_sdf_lines'],
                   row.get('protein_pdb_lines') if fr is not None else None, fr)
+
+
+_CHECK_STREAMS = {}
+
+
+def _pose_checks(items):
+    """One ``check_poses`` call over the ranked poses of [(row, result), ...] (results of failed complexes skipped); adds
+    ``result['checks']``.  The checks are a diagnostic: they never change or drop a docking result.  A ligand above the
+    automorphism cap gets checks without RMSD (``rmsd_error``); any other failure is reported as ``checks = {'error': msg}``.
+    They run on a side stream of their own, from the host copies of the ranked poses, so that they do not wait for the
+    sampler work the pipeline of ``infer_multiple_complexes`` has already enqueued behind them."""
+    items = [(row, res) for row, res in items if res is not None]
+    if not items:
+        return
+    dev = torch.cuda.current_device()
+    if dev not in _CHECK_STREAMS:
+        _CHECK_STREAMS[dev] = torch.cuda.Stream(dev)
+    try:
+        with torch.cuda.stream(_CHECK_STREAMS[dev]):
+            out = check_poses([row['complex_graph'] for row, _ in items], [res['ligand_pos'] for _, res in items],
+                              [res['atom_pos'] for _, res in items], [row.get('ref_ligand_pos') for row, _ in items],
+                              [row.get('ref_atom_pos') for row, _ in items], strict=False)
+    except Exception as e:
+        print('Pose checks failed for', [getattr(row['complex_graph'], 'name', None) for row, _ in items], e)
+        out = [{'error': str(e)}] * len(items)
+    for (_, res), checks in zip(items, out):
+        res['checks'] = checks
 
 
 def _rank(orig, idx, graphs, confidence):
@@ -119,11 +152,12 @@ def _rank(orig, idx, graphs, confidence):
 
 
 def infer_complex_group(group, model, args, score_model_args, filtering_model=None, filtering_model_args=None,
-                        tr_schedule=None, t_schedule=None, device=None, defer=False, writer=None, out_dir=None):
+                        tr_schedule=None, t_schedule=None, device=None, defer=False, writer=None, out_dir=None, pose_checks=False):
     """Cross-complex batching (SURVEY.md 8(f)-1; the reference's sampler assumes one complex per call, F9): the samples
     of several complexes share one ``sampling()`` call, so that small ``samples_per_complex`` still fill the mini-batch
     (virtual screening).  ``group``: [(idx, row), ...].  Falls back to one call per complex if the joint call fails.
-    ``defer`` as in ``infer_single_complex`` (the callable returns the list of per-complex results)."""
+    ``defer`` and ``pose_checks`` as in ``infer_single_complex`` (the callable returns the list of per-complex results; the
+    checks of the whole group run as one ``check_poses`` call)."""
     spc = args.samples_per_complex
     flex = False if args.rigid else score_model_args.flexible_sidechains
 
@@ -131,7 +165,7 @@ def infer_complex_group(group, model, args, score_model_args, filtering_model=No
         print('Joint call failed for', [row['complex_graph'].name for _, row in group], e, '- retrying one complex at a time')
         return [infer_single_complex(idx, row, model, args, score_model_args, filtering_model=filtering_model,
                                      filtering_model_args=filtering_model_args, tr_schedule=tr_schedule, t_schedule=t_schedule,
-                                     device=device, writer=writer, out_dir=out_dir) for idx, row in group]
+                                     device=device, writer=writer, out_dir=out_dir, pose_checks=pose_checks) for idx, row in group]
     try:
         data_list = []
         for _, row in group:
@@ -159,15 +193,18 @@ def infer_complex_group(group, model, args, score_model_args, filtering_model=No
                          confidence[k * spc:(k + 1) * spc] if confidence is not None else None) for k, (idx, row) in enumerate(group)]
             for (idx, row), res in zip(group, out):
                 _submit_write(writer, out_dir, row, res, flex)
-            return out
         except Exception as e:
             return one_by_one(e)
+        if pose_checks:
+            _pose_checks([(row, res) for (_, row), res in zip(group, out)])
+        return out
     return finish if defer else finish()
 
 
 def infer_multiple_complexes(rows, *a, batch_complexes=False, pipeline=True, **kw):
     """inference.py:294-304 over a list of (idx, row) (rows: dicts with 'complex_graph'); -> (results, count_succeeded).
     ``batch_complexes``: pack floor(batch_size / samples_per_complex) complexes into each sampler call.
+    ``pose_checks``, like the other keyword arguments, is passed to every call.
     ``pipeline``: software pipeline of depth 2 -- the host prepares and enqueues call k + 1 (graph copies,
     ``randomize_position``, collation, plan upload, kernel launches) while the GPU still runs call k, and only then
     collects call k's poses; without it the GPU idles during every complex's host work (the reference's loop is serial)."""
@@ -178,7 +215,8 @@ def infer_multiple_complexes(rows, *a, batch_complexes=False, pipeline=True, **k
         items, wrap = list(rows), (lambda r: [r])
     else:
         model, score_model_args = (a[0] if a else kw['model']), (a[2] if len(a) > 2 else kw['score_model_args'])
-        passthrough = {k: kw[k] for k in ('filtering_model', 'filtering_model_args', 'tr_schedule', 't_schedule', 'device', 'writer', 'out_dir') if k in kw}
+        passthrough = {k: kw[k] for k in ('filtering_model', 'filtering_model_args', 'tr_schedule', 't_schedule', 'device', 'writer', 'out_dir',
+                                          'pose_checks') if k in kw}
         launch = lambda grp: infer_complex_group(grp, model, args, score_model_args, defer=True, **passthrough)
         items, wrap = [rows[j:j + per_call] for j in range(0, len(rows), per_call)], (lambda r: r)
     results, pending = [], None
@@ -196,16 +234,18 @@ def infer_multiple_complexes(rows, *a, batch_complexes=False, pipeline=True, **k
 
 
 def infer_sharded(rows, model, args, score_model_args, device, filtering_model=None, filtering_model_args=None, group=None,
-                  batch_complexes=False, pipeline=True):
+                  batch_complexes=False, pipeline=True, pose_checks=False):
     """Complexes split over the ranks like ``np.array_split`` (inference.py:468); every rank docks its shard with no
-    communication; one all-gather of (complex index, best confidence) at the end -> global ranking on every rank."""
+    communication; one all-gather of (complex index, best confidence) at the end -> global ranking on every rank.
+    ``pose_checks`` as in ``infer_single_complex`` (each rank checks its own shard)."""
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     lo, hi = shard_range(len(rows), rank, world)
     sched = get_t_schedule('expbeta', args.inference_steps, inf_sched_alpha=args.inf_sched_alpha, inf_sched_beta=args.inf_sched_beta)   # inference.py:457-459
     local, ok = infer_multiple_complexes([(i, rows[i]) for i in range(lo, hi)], model, args, score_model_args,
                                          filtering_model=filtering_model, filtering_model_args=filtering_model_args,
-                                         tr_schedule=sched, device=device, batch_complexes=batch_complexes, pipeline=pipeline)
+                                         tr_schedule=sched, device=device, batch_complexes=batch_complexes, pipeline=pipeline,
+                                         pose_checks=pose_checks)
     # the single collective of the path: all-gather of the shards' best confidences (padded to the largest shard)
     width = -(-len(rows) // world) if len(rows) else 1
     mine = torch.full((width,), float('-inf'), device=device)

@@ -396,6 +396,48 @@ int ddp_pose_max_ligand_atoms(void);
  * CUDA graph while the per-step scalars change. */
 int ddp_pose_update_dev(const ddp_pose_t *pose, const ddp_step_coef_t *coef_dev, void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Pose checks (DESIGN section 11; diffdock_pocket_b200/posecheck.py builds the tables).  Poses of several complexes are
+ * packed row-wise: pose p of complex pose_complex[p] owns rows [ptr[p], ptr[p+1]) of a position array [rows][3].
+ *
+ * ddp_pose_rmsd: rmsd[p] = min over automorphisms a of sqrt(mean_i |pos_p[i] - ref_c[perm_a[i]]|^2), squared deviations
+ *   summed in fp64; best[p] = the minimising a (the smallest on ties).  ref_c = ref + 3 * ref_off[c]; automorphism table
+ *   of complex c: int16 [n_auto[c]][n_c] at autos + auto_off[c] (row 0 the identity for a plain by-index RMSD).  At most
+ *   ddp_pose_max_ligand_atoms() rows per pose: a longer pose gets rmsd NaN and best -1. */
+int ddp_pose_rmsd(const float *pos, const int32_t *pos_ptr, const int32_t *pose_complex, int32_t n_poses, const float *ref,
+                  const int32_t *ref_off, const int16_t *autos, const int32_t *auto_off, const int32_t *n_auto, float *rmsd,
+                  int32_t *best, void *stream);
+
+/* ddp_clash_screen: a pair (i, j) clashes when |x_i - x_j|^2 < (ratio (R_i + R_j))^2 in fp32.  For each pose p and pair set
+ * k, count[3p + k] += clashing pairs and min_ratio[3p + k] = min(min_ratio[3p + k], |x_i - x_j| / (R_i + R_j)); the caller
+ * zeroes count and fills min_ratio with +inf (an empty set leaves +inf).  Sets: 0 every ligand atom x every pocket atom
+ * of the same pose; 1 every moved side-chain atom x every pocket atom of another residue, except the listed bonded
+ * pairs (ordered pairs: two moved atoms of different residues are counted twice); 2 ligand pairs i < j whose bit is set
+ * in the pair mask (atoms >= 4 bonds apart).  R = radius[type].  Ligands of more than ddp_pose_max_ligand_atoms() atoms
+ * get count -1.  Tables of complex c, all indices local to its rows: */
+typedef struct {
+    int32_t lig_type_off;        /* lig_type[lig_type_off + i]: radius index of ligand atom i */
+    int32_t far_off;             /* far_mask + far_off: n_l rows of ceil(n_l / 32) words, bit j of row i = pair (i, j) */
+    int32_t atom_off;            /* atom_type / atom_owner [atom_off + j]: radius index and residue of pocket atom j */
+    int32_t moved_off, n_moved;  /* moved[moved_off + k]: pocket atom of moved side-chain atom k */
+    int32_t excl_off, n_excl;    /* excl[2 (excl_off + e) + 0 / 1]: (k, j) bonded pairs left out of set 1 */
+} ddp_clash_complex_t;
+typedef struct {
+    int32_t n_poses;
+    int32_t max_lig_atoms, max_atoms;     /* largest n_l and n_a of the poses (sizes the grid) */
+    const int32_t *pose_complex;          /* [n_poses] */
+    const float *lig_pos; const int32_t *lig_ptr;     /* ligand rows, [n_poses + 1] */
+    const float *atom_pos; const int32_t *atom_ptr;   /* pocket rows of the same poses, [n_poses + 1] */
+    const ddp_clash_complex_t *complexes;
+    const int32_t *lig_type, *atom_type, *atom_owner, *moved, *excl;
+    const uint32_t *far_mask;
+    const float *radius;                  /* radius table */
+    float ratio;
+    int32_t *count;                       /* [n_poses][3] */
+    float *min_ratio;                     /* [n_poses][3] */
+} ddp_clash_screen_t;
+int ddp_clash_screen(const ddp_clash_screen_t *args, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
