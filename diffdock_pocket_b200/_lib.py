@@ -12,7 +12,7 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.environ.get('DDP_LIB', os.path.join(_HERE, 'libddp_b200.so'))     # DDP_LIB: A/B runs of two builds
 CSRC = os.path.join(_HERE, 'csrc')
-SOURCES = ['graph.cu', 'embed.cu', 'tpconv_fp32.cu', 'tpconv_umma.cu', 'tpconv_bwd.cu', 'pose.cu', 'posecheck.cu', 'capi.cu']
+SOURCES = ['graph.cu', 'embed.cu', 'tpconv_fp32.cu', 'tpconv_umma.cu', 'tpconv_bwd.cu', 'pose.cu', 'posecheck.cu', 'esm.cu', 'capi.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-shared']
 
@@ -117,6 +117,10 @@ _SIGS = {
     'ddp_pose_update_dev': (i32, [C.POINTER(Pose), vp, vp]),
     'ddp_pose_rmsd': (i32, [vp, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
     'ddp_clash_screen': (i32, [C.POINTER(ClashScreen), vp]),
+    'ddp_esm_embed': (i32, [vp, i32, i32, vp, i32, i32, i32, i32, vp, vp]),
+    'ddp_layer_norm': (i32, [vp, vp, vp, vp, i32, i32, f32, vp, vp]),
+    'ddp_bias_gelu': (i32, [vp, vp, i32, i32, vp]),
+    'ddp_esm_attention': (i32, [vp, vp, vp, i32, vp, C.POINTER(f32), i32, i32, i32, i32, vp, i32, vp]),
     # deterministic mode (fixed-point accumulation, DDP_ACC_FIXED_SHIFT)
     'ddp_fixed_to_float': (i32, [vp, C.c_int64, vp, vp]),
     'ddp_tpconv_fp32_fixed': (i32, [C.POINTER(TpConv), C.POINTER(TpEdges), vp, vp, vp]),

@@ -8,8 +8,9 @@ C-alpha graph and atom->residue edges datasets/process_mols.py:650-724; ligand b
 rotatable-bond masks utils/torsion.py:16-65; side-chain masks utils/torsion.py:163-248), (b) an
 ``.npz`` round trip so fixtures travel to machines without the reference tree, and (c) procedural
 synthetic complexes for the benchmark configurations.  Ligand categorical features use only what a
-text SDF gives (element, degree, H count, charge, ring membership); ESM-2 embeddings are replaced by
-seeded N(0, 0.25^2) features (no LM weights offline).
+text SDF gives (element, degree, H count, charge, ring membership).  The receptor's ESM-2 embeddings
+come from ``receptor_embeddings`` (``esm.ESM2`` on the device) when the caller passes a model or
+precomputed rows; otherwise they are seeded N(0, 0.25^2) features.
 """
 import numpy as np
 import torch
@@ -40,6 +41,9 @@ RESIDUE_ATOM_ORDER = {
     'VAL': ['N', 'CA', 'C', 'O', 'CB', 'CG1', 'CG2'],
 }
 NO_TORSION_RES = {'ALA', 'GLY', 'PRO'}
+ONE_LETTER = {'ALA': 'A', 'ARG': 'R', 'ASN': 'N', 'ASP': 'D', 'CYS': 'C', 'GLN': 'Q', 'GLU': 'E', 'GLY': 'G', 'HIS': 'H',
+              'ILE': 'I', 'LEU': 'L', 'LYS': 'K', 'MET': 'M', 'PHE': 'F', 'PRO': 'P', 'SER': 'S', 'THR': 'T', 'TRP': 'W',
+              'TYR': 'Y', 'VAL': 'V', 'MSE': 'M'}
 Z_OF = {'H': 1, 'B': 5, 'C': 6, 'N': 7, 'O': 8, 'F': 9, 'P': 15, 'S': 16, 'CL': 17, 'SE': 34, 'BR': 35, 'I': 53}
 
 
@@ -82,6 +86,33 @@ def parse_pdb_heavy(path):
             continue
         r['atoms'].sort(key=lambda a: 999 if a[0] == 'OXT' else (order.index(a[0]) if a[0] in order else 998))
         out.append(r)
+    return out
+
+
+# --------------------------------------------------------------------------------------- receptor language-model features
+def chain_sequences(residues):
+    """-> [(chain_id, sequence, residue_indices)]: one-letter sequence of every chain of ``parse_pdb_heavy``'s residues
+    (chains and residues in file order, MSE read as M) and the indices of its residues in ``residues``.
+
+    ``parse_pdb_heavy`` keeps ATOM records of standard residues (and MSE) only, so a chain with HETATM residues (MSE
+    written as HETATM, modified residues) gives a shorter sequence than the reference's walk over every residue with
+    N / CA / C atoms (DESIGN section 12)."""
+    chains = {}
+    for i, r in enumerate(residues):
+        chains.setdefault(r['chain'], []).append(i)
+    return [(c, ''.join(ONE_LETTER.get(residues[i]['name'], 'X') for i in idx), idx) for c, idx in chains.items()]
+
+
+def receptor_embeddings(esm_model, residues):
+    """ESM-2 last-layer embeddings of ``residues`` (``parse_pdb_heavy`` order) -> [len(residues), D] fp32 on the model's
+    device.  Every chain is embedded as its own sequence with BOS / EOS, as the reference does, all chains in one
+    ``esm.embed_sequences`` call; rows go back to residue order.  See ``chain_sequences`` for the HETATM deviation."""
+    from . import esm
+    chains = chain_sequences(residues)
+    reps = esm.embed_sequences(esm_model, [s for _, s, _ in chains])
+    out = torch.empty(len(residues), esm_model.embed_dim, dtype=torch.float32, device=reps[0].device if reps else 'cpu')
+    for (_, _, idx), rep in zip(chains, reps):
+        out[torch.as_tensor(idx, device=out.device)] = rep
     return out
 
 
@@ -207,9 +238,11 @@ def _sidechain_bonds(res_atom_names):
 # --------------------------------------------------------------------------------------- complex graph
 def build_complex_graph(lig, residues, name='complex', pocket_center=None, flexible=None, flexdist=3.5,
                         receptor_radius=15.0, c_alpha_max_neighbors=24, pocket_buffer=10.0, pocket_cutoff=5.0,
-                        esm_seed=1234):
+                        esm_seed=1234, lm_embeddings=None):
     """``lig`` = (x, pos, edge_index, edge_attr); ``flexible``: None -> no flexResidues store,
-    'auto' -> prism/flexdist rule, or an explicit list like ['A:160', 'A:193']."""
+    'auto' -> prism/flexdist rule, or an explicit list like ['A:160', 'A:193'].  ``lm_embeddings``: [len(residues), 1280]
+    rows aligned to ``residues`` (``receptor_embeddings``); the pocket residues take theirs as ``receptor.x[:, 1:]``.
+    Without it those columns are seeded N(0, 0.25^2) noise (``esm_seed``)."""
     lig_x, lig_pos, lig_ei, lig_ea = lig
     g = HeteroData()
     g['name'] = name
@@ -230,8 +263,9 @@ def build_complex_graph(lig, residues, name='complex', pocket_center=None, flexi
         radius = torch.linalg.vector_norm(g['ligand'].pos - g['ligand'].pos.mean(0, keepdim=True), dim=1).max()
     radius = float(radius) + pocket_buffer
     cen = center.numpy().astype(np.float64)
-    pocket = [r for r in residues
-              if (np.linalg.norm(np.array([a[2] for a in r['atoms']]) - cen, axis=1) < radius).any()]
+    pocket_idx = [i for i, r in enumerate(residues)
+                  if (np.linalg.norm(np.array([a[2] for a in r['atoms']]) - cen, axis=1) < radius).any()]
+    pocket = [residues[i] for i in pocket_idx]
     ca = np.array([[a[2] for a in r['atoms'] if a[0] == 'CA'][0] for r in pocket])
     n_res = len(pocket)
     dist = np.linalg.norm(ca[:, None] - ca[None], axis=-1)
@@ -246,7 +280,13 @@ def build_complex_graph(lig, residues, name='complex', pocket_center=None, flexi
         src += [i] * len(nb)
         dst += [int(j) for j in nb]
     aa = torch.tensor([[_safe_index(AMINO_ACIDS, r['name'])] for r in pocket], dtype=torch.float32)
-    esm = torch.from_numpy(np.random.RandomState(esm_seed).randn(n_res, 1280).astype(np.float32) * 0.25)
+    if lm_embeddings is None:
+        esm = torch.from_numpy(np.random.RandomState(esm_seed).randn(n_res, 1280).astype(np.float32) * 0.25)
+    else:
+        lm = torch.as_tensor(lm_embeddings)
+        if lm.shape != (len(residues), 1280):
+            raise ValueError(f'lm_embeddings must be [{len(residues)}, 1280] (one row per residue), got {tuple(lm.shape)}')
+        esm = lm[torch.as_tensor(pocket_idx, dtype=torch.long, device=lm.device)].detach().to('cpu', torch.float32)
     g['receptor'].x = torch.cat([aa, esm], 1)
     g['receptor'].pos = torch.from_numpy(ca).float()
     g['receptor', 'rec_contact', 'receptor'].edge_index = torch.tensor([src, dst], dtype=torch.long)
@@ -301,11 +341,14 @@ def build_complex_graph(lig, residues, name='complex', pocket_center=None, flexi
     return g
 
 
-def load_example_3dpf(example_dir, apo=False, flexible='auto', pocket_center=None):
+def load_example_3dpf(example_dir, apo=False, flexible='auto', pocket_center=None, esm_model=None):
+    """``esm_model``: an ``esm.ESM2`` on the device; given, the receptor features are its embeddings of the protein's
+    chains (``receptor_embeddings``) instead of seeded noise."""
     atoms, bonds = parse_sdf(f'{example_dir}/3dpf_ligand.sdf')
     residues = parse_pdb_heavy(f"{example_dir}/{'3dpf_protein_esm.pdb' if apo else '3dpf_protein.pdb'}")
+    lm = None if esm_model is None else receptor_embeddings(esm_model, residues)
     return build_complex_graph(ligand_graph_from_sdf(atoms, bonds), residues, name='3dpf', pocket_center=pocket_center,
-                               flexible=flexible)
+                               flexible=flexible, lm_embeddings=lm)
 
 
 # --------------------------------------------------------------------------------------- npz round trip

@@ -438,6 +438,42 @@ typedef struct {
 } ddp_clash_screen_t;
 int ddp_clash_screen(const ddp_clash_screen_t *args, void *stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * ESM-2 receptor embeddings (DESIGN section 12; diffdock_pocket_b200/esm.py runs the layers, the dense projections are
+ * library GEMMs).  Replaces fair-esm's esm.model.esm2.ESM2.forward as the reference's utils/esm.py calls it (last layer's
+ * representation, no LM / contact head).  Activations are fp32 row-major [rows][cols]; a batch of B padded sequences of
+ * T tokens is [B * T][cols].
+ *
+ * ddp_esm_embed: ESM2.forward's embedding (esm/model/esm2.py): out[b][t] = embed_tokens[tokens[b][t]] * 0.88f / (1 - r_b)
+ *   (token dropout; r_b = #<mask> / #non-pad tokens of sequence b, fp32), rows of <mask> and pad tokens zero.  A token
+ *   outside [0, vocab) gives a NaN row.  tokens int64 [B][T], weight [vocab][D], out [B][T][D]. */
+int ddp_esm_embed(const int64_t *tokens, int32_t B, int32_t T, const float *weight, int32_t vocab, int32_t D, int32_t pad_idx,
+                  int32_t mask_idx, float *out, void *stream);
+
+/* ddp_layer_norm: nn.LayerNorm(cols, eps) of every row (ESM1bLayerNorm, esm/modules.py: self_attn_layer_norm,
+ *   final_layer_norm, emb_layer_norm_after), statistics in fp32: y = (x - mean) / sqrt(var + eps) * gamma + beta.  With
+ *   residual_bias != NULL the row is first updated in place, x += residual_bias (the pending bias of the Linear whose
+ *   output the caller's GEMM added into the residual stream), and y must not alias x; otherwise y may alias x.
+ *   cols % 4 == 0, cols <= 2048, all pointers 16-byte aligned. */
+int ddp_layer_norm(float *x, const float *residual_bias, const float *gamma, const float *beta, int32_t rows, int32_t cols,
+                   float eps, float *y, void *stream);
+
+/* ddp_bias_gelu: x = gelu(x + bias[col]) in place, exact erf GELU 0.5 v (1 + erf(v / sqrt 2)) (esm/modules.py: gelu after
+ *   fc1).  cols % 4 == 0, pointers 16-byte aligned. */
+int ddp_bias_gelu(float *x, const float *bias, int32_t rows, int32_t cols, void *stream);
+
+/* ddp_esm_attention: MultiheadAttention.forward with rotary embeddings (esm/multihead_attention.py,
+ *   esm/rotary_embedding.py) for head_dim 64.  q, k, v: [B * T][ld_in] rows, head h in columns [64 h, 64 h + 64) (the Q / K
+ *   / V projections, Q already scaled by 1/8); out: [B * T][ld_out], heads concatenated (the input of out_proj).  Rotary
+ *   is applied to q and k as they are loaded: angle float(t) * inv_freq[i] in fp32 for position t (0 at BOS), pairs
+ *   (x[i], x[i + 32]) -> (x[i] cos - x[i + 32] sin, x[i + 32] cos + x[i] sin).  Keys t >= lengths[b] are masked; every query
+ *   row t < T is computed.  inv_freq_host: HOST pointer to the 32 inverse frequencies.  fp32 on CUDA cores, online
+ *   softmax, no atomics (bitwise repeatable).  DDP_E_UNSUPPORTED for head_dim != 64, DDP_E_SHAPE for T > 1024; v and out
+ *   16-byte aligned, ld_in and ld_out multiples of 4, lengths[b] >= 1. */
+int ddp_esm_attention(const float *q, const float *k, const float *v, int32_t ld_in, const int32_t *lengths,
+                      const float *inv_freq_host, int32_t B, int32_t T, int32_t H, int32_t head_dim, float *out, int32_t ld_out,
+                      void *stream);
+
 #ifdef __cplusplus
 }
 #endif
